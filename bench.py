@@ -39,8 +39,24 @@ def emit(line):
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree: no __pycache__ next to the sources
 
 import numpy as np  # noqa: E402
+
+DUMP_ENTRIES = 1 << 22   # --dump-outputs: at most 4 Mi float64 values (32 MB) over all ranks
+
+
+def dump_output(out_dir, name, y, world):
+    """Write a result vector as out_dir/name.npy (float64).  A vector longer than this rank's share of DUMP_ENTRIES is
+    sampled at sorted indices drawn with a fixed seed: the same length gives the same indices in every run."""
+    import torch
+    k = DUMP_ENTRIES // world
+    if y.numel() > k:
+        idx = np.sort(np.random.default_rng(0).choice(y.numel(), k, replace=False))
+        y = y[torch.from_numpy(idx).to(y.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), y.detach().to(torch.float64).cpu().numpy())
+
 
 def alg_bytes(problem, p, qextra=0):
     """SURVEY.md 8(d): 8 Q^3 (10 + g) + 4 P^3 + 48 p^3 bytes per element (22 572 for hyperFS p = 4)."""
@@ -331,7 +347,12 @@ def main():
     ap.add_argument("--assemble", default="coo", choices=["coo", "color"], help="p=1 matrix: CeedOperatorLinearAssemble element matrices, or 81 coloured applies (misc.c:151-183)")
     ap.add_argument("--coarse", default="hmg", choices=["hmg", "pcg"], help="coarse solve on the assembled p=1 level: h-multigrid (GAMG stand-in) or Jacobi-PCG")
     ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed MatMults, write the product Y of the last one (this rank's global vector) as "
+                         "DIR/y.npy (DIR/y_rank<r>.npy for N > 1), float64; longer vectors as a fixed seeded sample")
     args = ap.parse_args()
+    if args.dump_outputs and (args.solve or args.impl != "b200"):
+        ap.error("--dump-outputs writes the result of the /gpu/b200 MatMult: not with --solve or --impl reference")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -423,6 +444,8 @@ def main():
     # one call's launches separately (same code path, same count every call)
     ms = timed(pr.matmult, args.steps, args.warmup, world, dist)
     clocks = sampler.result()
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "y" if world == 1 else f"y_rank{rank}", pr.Y, world)
     libceed.launch_count_reset()
     pr.matmult()
     torch.cuda.synchronize()
@@ -436,7 +459,7 @@ def main():
     xl.copy_(torch.from_numpy(np.random.default_rng(7).standard_normal(dm.lsize)))
     xc, yc = data[fine].xceed, data[fine].yceed
     xc.set_array(xl); yc.set_array(yl)
-    nk = max(args.steps, 10)
+    nk = args.steps
     kms = timed(lambda: data[fine].opJacob.apply_add(xc, yc), nk, 3, 1, None) / nk
     # Jacobian cache: rebuilt lazily after every residual evaluation (new linearisation point)
     pr.evaluate_residual()
@@ -494,7 +517,7 @@ def main():
             if world > 1:
                 dist.barrier()
             torch.cuda.synchronize()
-        nrep = max(3, min(args.steps, 10))
+        nrep = args.steps
         for it in range(2 + nrep):
             if it == 2:
                 host_barrier()
@@ -563,7 +586,8 @@ def main():
         xs.normal_()
         xcs, ycs = ps.data[ps.fine].xceed, ps.data[ps.fine].yceed
         xcs.set_array(xs); ycs.set_array(ys)
-        ks = min(timed(lambda: ps.data[ps.fine].opJacob.apply_add(xcs, ycs), 10, 3, world, dist) / 10 for _ in range(2))
+        ks = min(timed(lambda: ps.data[ps.fine].opJacob.apply_add(xcs, ycs), args.steps, 3, world, dist) / args.steps
+                 for _ in range(2))
         xcs.take_array(); ycs.take_array()
         extra["strong_c4"] = {"value": sd * args.steps / (mss * 1e-3) / 1e9, "unit": "GDoF/s", "ms_per_step": mss / args.steps,
                               "scaling": "strong", "dofs": sd, "elements_per_gpu": ps.mesh.nelem, "bricks": "x".join(map(str, ps.grid)),

@@ -10,6 +10,7 @@ cpu_baseline / --impl reference legs.  The product package never imports it.
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -57,14 +58,13 @@ def lib():
 
 def native_lib():
     """TIMING build (-O3 -march=native, FP contraction on), compiled on the box that runs it: bench.py's CPU legs only.
+    Built in a temporary directory that is gone once the library is loaded: the benchmark writes nothing into the tree.
     Parity checks always go through lib()."""
     global _NATIVE
     if _NATIVE is None:
-        so = os.path.join(HERE, "_native", "liboracle_native.so")
-        srcs = [os.path.join(HERE, f) for f in ("ceed_oracle.c", "qf_port.c", "Makefile")]
-        if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-            subprocess.run(["make", "-s", "-C", HERE, "timing"], check=True, stdout=subprocess.DEVNULL)
-        _NATIVE = C.CDLL(so)
+        with tempfile.TemporaryDirectory(prefix="oracle_native_") as d:
+            subprocess.run(["make", "-s", "-C", HERE, "timing", "NATIVE_DIR=" + d], check=True, stdout=subprocess.DEVNULL)
+            _NATIVE = C.CDLL(os.path.join(d, "liboracle_native.so"))
     return _NATIVE
 
 

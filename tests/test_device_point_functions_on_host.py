@@ -102,17 +102,26 @@ def test_closed_form_diagonal_blocks_equal_unit_inputs_through_the_jacobian(host
 @pytest.mark.parametrize("which", ["port", "ref"])
 def test_energy_and_diagnostics_match_the_reference_qfunctions(hostlib, name, which):
     if which == "ref" and not oracle.have_ref():
-        pytest.skip("oracle/_ref not built")
-    Q, J, w, ug, _ = make_golden.rnd_inputs(Q=48, seed=11)
-    phys = oracle.Physics(0.3, 1.0)
-    (qd,) = oracle.call_qf("SetupGeo", which, None, Q, [J.reshape(9, Q), w.reshape(1, Q)], [10])
-    du = np.ascontiguousarray(3.0 * ug.reshape(9, Q))          # strains up to ~0.2: the series branches matter
-    u = np.random.default_rng(1).standard_normal((3, Q))
-    (e_ref,) = oracle.call_qf(name + "Energy", which, phys, Q, [du, qd], [1])
-    (d_ref,) = oracle.call_qf(name + "Diagnostic", which, phys, Q, [u, du, qd], [8])
-    energy, diag5 = np.zeros(Q), np.zeros((5, Q))
-    assert hostlib.qf_host_post(PROBS[name], 0.3, 1.0, Q, _p(du), _p(np.ascontiguousarray(qd)), _p(energy), _p(diag5)) == 0
-    assert _rel(energy, e_ref.reshape(-1)) < 1e-13
-    for k in range(5):
-        assert _rel(diag5[k], d_ref[3 + k]) < 1e-13, (name, k)
-    assert np.array_equal(d_ref[:3], u)
+        # without a live build of the reference's QFunctions: their committed outputs at the committed inputs
+        cases = []
+        for tag in ("katF", "rnd"):
+            Q = GOLD[f"{tag}_qdata"].shape[1]
+            cases.append((Q, GOLD[f"{tag}_ug"].reshape(9, Q), GOLD[f"{tag}_qdata"], GOLD[f"{tag}_J"].reshape(9, Q)[3:6] - 0.1,
+                          GOLD[f"{tag}_{name}Energy"], GOLD[f"{tag}_{name}Diagnostic"]))
+    else:
+        Q, J, w, ug, _ = make_golden.rnd_inputs(Q=48, seed=11)
+        phys = oracle.Physics(0.3, 1.0)
+        (qd,) = oracle.call_qf("SetupGeo", which, None, Q, [J.reshape(9, Q), w.reshape(1, Q)], [10])
+        du = np.ascontiguousarray(3.0 * ug.reshape(9, Q))          # strains up to ~0.2: the series branches matter
+        u = np.random.default_rng(1).standard_normal((3, Q))
+        (e_ref,) = oracle.call_qf(name + "Energy", which, phys, Q, [du, qd], [1])
+        (d_ref,) = oracle.call_qf(name + "Diagnostic", which, phys, Q, [u, du, qd], [8])
+        cases = [(Q, du, qd, u, e_ref, d_ref)]
+    for Q, du, qd, u, e_ref, d_ref in cases:
+        energy, diag5 = np.zeros(Q), np.zeros((5, Q))
+        assert hostlib.qf_host_post(PROBS[name], 0.3, 1.0, Q, _p(np.ascontiguousarray(du)), _p(np.ascontiguousarray(qd)),
+                                    _p(energy), _p(diag5)) == 0
+        assert _rel(energy, e_ref.reshape(-1)) < 1e-13
+        for k in range(5):
+            assert _rel(diag5[k], d_ref[3 + k]) < 1e-13, (name, k)
+        assert np.array_equal(d_ref[:3], u)
