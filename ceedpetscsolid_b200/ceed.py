@@ -164,6 +164,10 @@ _proto("b200_elems_per_block", _i)
 _proto("b200_fused_supported", _i, _i)
 _proto("b200_jcache_ncomp", _i)
 _proto("b200_apply_transfer", _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp)
+_proto("b200_bsr_spmv", _i, _i, _i, _vp, _vp, _vp, _vp, _vp)
+_proto("b200_bsr_pairs_product", _i, _i, _i, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp)
+_proto("b200_bsr_transpose_gather", _i, _i, _sz, _vp, _vp, _vp)
+_proto("b200_bsr_assemble_elem", _sz, _vp, _vp, _vp, _vp)
 
 # sentinels are exported data symbols holding pointers
 def _sentinel(name):

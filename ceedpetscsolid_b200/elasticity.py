@@ -156,10 +156,15 @@ class Elasticity:
     """Builds the whole solver stack for one rank (one GPU)."""
 
     def __init__(self, app, dist=None, rank=0, world=1, device_id=0, gmesh=None, coarse_rtol=1e-2, coarse="hmg",
-                 assemble="coo", masked=True, overlap=True, halo="p2p", deterministic=False):
-        """masked: constrained dofs are masked in L-vector-shaped global vectors (no G2L/L2G copies, see LevelDM);
+                 assemble="coo", masked=True, overlap=True, halo="p2p", deterministic=False, amg_max_coarse=None):
+        """coarse: the solve on the assembled p = 1 level -- "hmg" (geometric h-multigrid on box meshes, Jacobi-PCG on
+        unstructured ones), "pcg" (Jacobi-PCG) or "amg" (one V-cycle of smoothed-aggregation AMG, any mesh, one GPU;
+        amg_max_coarse: rows of its directly solved coarsest level, default amg.MAX_COARSE_DOFS).  masked: constrained dofs are masked in L-vector-shaped global vectors (no G2L/L2G copies, see LevelDM);
         False: compressed PETSc-style global vectors.  deterministic: "/gpu/b200:deterministic" -- every transposed
         restriction sums in the serial /cpu/self order (no FP64 atomics anywhere on the path)."""
+        if coarse == "amg" and world > 1:
+            raise NotImplementedError("coarse='amg': the smoothed-aggregation AMG coarse solve runs on one GPU; "
+                                      "partitioned AMG is not implemented (use coarse='hmg' or 'pcg' with world > 1)")
         self.app, self.dist = app, dist
         halo_mode = halo
         grid = grid_for(world)
@@ -227,7 +232,15 @@ class Elasticity:
             if dm.dot_weight is not None or dm.masked:
                 self.V.consistent[dm.nglobal] = dm.make_consistent
         self.all_dms = self.dms + list(h_dms or [])
-        self.pc = solver.PMultigrid(self.V, self.levels, self.transfers, coarse_rtol=coarse_rtol, h_dms=h_dms)
+        amg_solver = None
+        if coarse == "amg":
+            if self.levels[0].coo is None:
+                raise ValueError("coarse='amg' needs the element matrices of the p = 1 level (assemble='coo', fused operator)")
+            from .amg import MAX_COARSE_DOFS, SmoothedAggregationAMG
+            amg_solver = SmoothedAggregationAMG(self.dms[0], self.mesh,
+                                                max_coarse=MAX_COARSE_DOFS if amg_max_coarse is None else amg_max_coarse)
+        self.pc = solver.PMultigrid(self.V, self.levels, self.transfers, coarse_rtol=coarse_rtol, h_dms=h_dms,
+                                    amg=amg_solver)
         self.U = self.dms[fine].create_global_vector()
 
     @staticmethod

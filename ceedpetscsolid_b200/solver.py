@@ -742,9 +742,11 @@ def _lattice_restrict_cpu(Nc, xf):
 class PMultigrid:
     """PCMG, multiplicative V-cycle, levels[0] = coarsest (p = 1) ... levels[-1] = finest."""
 
-    def __init__(self, V, levels, transfers, coarse_rtol=1e-2, coarse_maxit=500, smooth_its=3, h_dms=None):
+    def __init__(self, V, levels, transfers, coarse_rtol=1e-2, coarse_maxit=500, smooth_its=3, h_dms=None, amg=None):
         """levels: list of objects with .n, .device, .jacobian(X, Y), .diagonal(D), .local_apply(xloc, yloc), .dm
-        transfers[l] (l >= 1): object with .prolong(Xc, Yf), .restrict(Xf, Yc) between l-1 and l."""
+        transfers[l] (l >= 1): object with .prolong(Xc, Yf), .restrict(Xf, Yc) between l-1 and l.
+        amg: an amg.SmoothedAggregationAMG of the p = 1 level -> one AMG V-cycle is the coarse solve (coarse_its
+        then counts V-cycles)."""
         self.V, self.levels, self.transfers = V, levels, transfers
         self.coarse_rtol, self.coarse_maxit = coarse_rtol, coarse_maxit
         L = len(levels)
@@ -757,10 +759,14 @@ class PMultigrid:
         self.t = [mk(l) for l in range(L)]
         self.diag = [mk(l) for l in range(L)]
         CoarseMatrix = ColoredCoarseMatrix if getattr(levels[0].dm.mesh, "structured", True) else SparseCoarseMatrix
-        self.coarse = CoarseMatrix(levels[0].dm, levels[0].local_apply, coo=getattr(levels[0], "coo", None))
+        coo = getattr(levels[0], "coo", None)
+        # the AMG assembles the p = 1 matrix itself (BSR) from the element matrices: no second matrix object then
+        self.coarse = None if (amg is not None and coo is not None) else CoarseMatrix(levels[0].dm, levels[0].local_apply,
+                                                                                      coo=coo)
         # h_dms: LevelDMs of successively halved meshes below the p = 1 level -> geometric multigrid coarse
         # solve (GAMG stand-in); None -> Jacobi-PCG on the assembled p = 1 matrix
         self.hmg = HMultigrid(V, self.coarse, [levels[0].dm] + list(h_dms)) if h_dms else None
+        self.amg = amg
         self.cwork = [mk(0) for _ in range(4)]
         self.cdinv = mk(0)
         self.coarse_its = 0
@@ -773,12 +779,20 @@ class PMultigrid:
             lev.diagonal(self.diag[l])
             if l > 0:
                 self.smoothers[l].setup(self.diag[l])
-        self.coarse.assemble()
+        if self.amg is not None:   # assembles the p = 1 matrix itself, in its own (BSR) layout
+            self.amg.setup(self.coarse if self.coarse is not None else self.levels[0])
+        else:
+            self.coarse.assemble()
         self.cdinv.copy_(1.0 / self.diag[0])
         if self.hmg is not None:
             self.hmg.setup()
 
     def _coarse_solve(self, b, x):
+        if self.amg is not None:
+            self.amg.solve(b, x)
+            self.coarse_solves += 1
+            self.coarse_its += 1
+            return
         if self.hmg is not None:
             self.hmg.solve(b, x)
             self.coarse_solves += 1

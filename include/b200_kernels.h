@@ -289,6 +289,27 @@ int b200_apply_transfer(int transpose, int nelem, int Pc, int Pf, const double *
                         const int *d_offc, const int *d_offf, const double *d_mult, int inject,
                         const double *d_in, double *d_out, double *d_evec);
 
+/* ---- smoothed-aggregation AMG on the assembled p = 1 level (the GAMG coarse solve, elasticity.c:569-585) -------
+ * BSR matrices: block rows rowptr[nbrows+1], block columns colidx[nnzb], values [nnzb][br][bc] (row-major blocks).
+ * Every output is a fixed-order sum of its listed terms (no atomics): results are bit-identical from run to run. */
+/* y = A x; block shapes (br, bc) in {(3,3), (6,6), (3,6), (6,3)} */
+int b200_bsr_spmv(int br, int bc, int nbrows, const int *rowptr, const int *colidx, const double *vals,
+                  const double *x, double *y);
+/* pair-list block product C[k] = sum_{t = ptr[k]}^{ptr[k+1]-1} A[pa[t]] B[pb[t]]  (br x bk times bk x bc blocks);
+ * (br, bk, bc) in {(3,3,6), (6,3,6), (6,6,6), (3,3,3)}.  tmap != NULL selects the smoothed-prolongator epilogue
+ *   C[k] = T[tmap[k]] - omega[0] * dinv[rowof[k]*br + i] * C[k]   (row i of the block; tmap[k] < 0: T block absent)
+ * with omega a DEVICE scalar (no host synchronisation) */
+int b200_bsr_pairs_product(int br, int bk, int bc, size_t nout, const long long *ptr, const int *pa, const int *pb,
+                           const double *A, const double *B, double *C, const int *tmap, const int *rowof,
+                           const double *T, const double *dinv, const double *omega);
+/* dst[k] = src[idx[k]]^T (src blocks br x bc, dst blocks bc x br): the transposed prolongator by a fixed gather;
+ * (br, bc) in {(3,6), (6,6), (3,3)} */
+int b200_bsr_transpose_gather(int br, int bc, size_t nblocks, const int *idx, const double *src, double *dst);
+/* 3x3 blocks from element matrices evals[(e*24 + col)*24 + row] (b200_assemble_p1 layout):
+ *   vals[k][i][j] = sum_{t = ptr[k]}^{ptr[k+1]-1} evals[src[t] + 24 j + i]   (src[t] = (e*24 + 3b)*24 + 3a) */
+int b200_bsr_assemble_elem(size_t nblocks, const long long *ptr, const long long *src, const double *evals,
+                           double *vals);
+
 #ifdef __cplusplus
 }
 #endif
