@@ -283,10 +283,13 @@ class SmoothedAggregationAMG:
     L-vector layout (every node, 3 dofs); constrained (Dirichlet) rows and columns are masked with a unit diagonal and
     no aggregate contains a constrained node."""
 
-    def __init__(self, dm, mesh, smooth_its=2, max_coarse=MAX_COARSE_DOFS, seed=200):
+    def __init__(self, dm, mesh, smooth_its=2, max_coarse=MAX_COARSE_DOFS, seed=200, elem_src=None):
+        """elem_src: optional int array [mesh.nelem], element e -> its position in the element-matrix buffer the
+        numeric set-up reads (default: position e).  RedundantAMG reads a rank-major gathered buffer this way."""
         t0 = time.perf_counter()
         if dm.halo is not None:
-            raise NotImplementedError("smoothed-aggregation AMG runs on one GPU: partitioned AMG is not implemented")
+            raise NotImplementedError("SmoothedAggregationAMG takes the whole p = 1 level of one rank; partitioned runs "
+                                      "use RedundantAMG")
         self.dm, dev = dm, dm.device
         self.device = dev
         en = mesh.offsets(1).reshape(-1, 8).astype(np.int64) // 3
@@ -304,7 +307,8 @@ class SmoothedAggregationAMG:
         a_, b_ = np.meshgrid(np.arange(8), np.arange(8), indexing="ij")
         rn, cn = en[:, a_.reshape(-1)], en[:, b_.reshape(-1)]                     # (E, 64)
         ok = free[rn] & free[cn]
-        src = ((np.arange(E)[:, None] * 24 + 3 * b_.reshape(-1)[None, :]) * 24 + 3 * a_.reshape(-1)[None, :])
+        pos = np.arange(E, dtype=np.int64) if elem_src is None else np.asarray(elem_src, dtype=np.int64)
+        src = ((pos[:, None] * 24 + 3 * b_.reshape(-1)[None, :]) * 24 + 3 * a_.reshape(-1)[None, :])
         keys0 = np.repeat(np.arange(nn, dtype=np.int64), np.diff(A0ptr)) * nn + A0ind
         dest = np.searchsorted(keys0, rn[ok] * nn + cn[ok])
         src = src[ok]
@@ -495,3 +499,83 @@ class SmoothedAggregationAMG:
         """pairs per product per level (A P_tent, A P, P^T A P)"""
         return [{"AP_tent": lev.AP_t.npairs, "AP": lev.AP_p.npairs, "PtAP": lev.Ac_p.npairs}
                 for lev in self.levels[:-1]]
+
+
+class RedundantAMG(SmoothedAggregationAMG):
+    """The AMG coarse solve of a partitioned run (world > 1), as PETSc's PCREDUNDANT / GAMG process agglomeration:
+    every rank builds and holds the whole hierarchy of the GLOBAL p = 1 level and applies it to the gathered
+    right-hand side.
+
+    dm, mesh: this rank's p = 1 LevelDM (masked layout) and part; gmesh: the global mesh, faces: the Dirichlet faces.
+    Symbolic set-up (collective, once): the ranks' global element ids are exchanged and folded into the level-0
+    assembly map, so b200_bsr_assemble_elem reads the gathered buffer directly.  Numeric set-up (once per Newton
+    step): one all-gather of the element matrices into a rank-major buffer padded to the largest part.  Solve: the
+    owned dofs of b are scattered into a zero global vector and summed over ranks (exact: one non-zero contribution
+    per entry), one V-cycle runs on every rank, and each rank gathers its local dofs, shared ones included (the same
+    bits on every holder).  Gathers are copies and the sum is exact, so every rank holds bit-identical levels."""
+
+    def __init__(self, dm, mesh, gmesh, faces, dist, **kw):
+        if not dm.masked:
+            raise NotImplementedError("coarse='amg' with world > 1 needs the masked layout (masked=True)")
+        self.dist, self.world = dist, dist.get_world_size()
+        ids = [None] * self.world
+        dist.all_gather_object(ids, np.asarray(mesh.elem_ids, dtype=np.int64))
+        self.emax = max(v.size for v in ids)
+        pos = np.full(gmesh.nelem, -1, dtype=np.int64)
+        for r, v in enumerate(ids):
+            if (pos[v] >= 0).any():
+                raise ValueError(f"element(s) {v[pos[v] >= 0][:5].tolist()} are held by more than one rank")
+            pos[v] = r * self.emax + np.arange(v.size)
+        if (pos < 0).any():
+            raise ValueError(f"{int((pos < 0).sum())} element(s) of the global mesh are held by no rank")
+        from .matops import LevelDM
+        dev = dm.device
+        gdm = LevelDM(gmesh, 1, bc_faces=faces, device=dev, masked=True)
+        super().__init__(gdm, gmesh, elem_src=pos, **kw)
+        gnode = _global_node_ids(mesh, gmesh)
+        gdof = (gnode[:, None] * 3 + np.arange(3)).reshape(-1)
+        own = np.flatnonzero(np.repeat(dm.halo.owned_node_mask, 3))
+        self.local_dm = dm
+        self.l2g = _t(gdof, np.int32, dev)
+        self.own_l, self.own_g = _t(own, np.int32, dev), _t(gdof[own], np.int32, dev)
+        self.own_vals = torch.zeros(own.size, dtype=torch.float64, device=dev)
+        self.bglob = torch.zeros(gdm.lsize, dtype=torch.float64, device=dev)
+        self.xglob = torch.zeros(gdm.lsize, dtype=torch.float64, device=dev)
+        self.send = torch.zeros(self.emax * 576, dtype=torch.float64, device=dev)
+        self.gathered = torch.zeros(self.world * self.emax * 576, dtype=torch.float64, device=dev)
+        self.coo = self            # setup() hands itself to SmoothedAggregationAMG.setup as the element-matrix source
+
+    def values(self):
+        return self.gathered
+
+    def setup(self, source):
+        """source: the p = 1 level with this rank's element matrices (.coo, CeedOperatorLinearAssemble layout)"""
+        ev = source.coo.values()
+        self.send[:ev.numel()].copy_(ev)
+        if self.send.is_cuda:
+            self.dist.all_gather_into_tensor(self.gathered, self.send)
+        else:
+            self.dist.all_gather(list(self.gathered.view(self.world, -1).unbind(0)), self.send)
+        super().setup(self)
+
+    def solve(self, b, x):
+        """x = one V-cycle of the global hierarchy applied to b (masked local vectors of this rank's p = 1 level)"""
+        self.bglob.zero_()
+        self._gather(self.own_vals, b, self.own_l)
+        if b.is_cuda:
+            b2(lib.b200_scatter_set(self.bglob.data_ptr(), self.own_g.data_ptr(), self.own_vals.data_ptr(),
+                                    self.own_vals.numel()))
+        else:
+            self.bglob[self.own_g.long()] = self.own_vals
+        self.dist.all_reduce(self.bglob)
+        super().solve(self.bglob, self.xglob)
+        self._gather(x, self.xglob, self.l2g)
+
+
+def _global_node_ids(mesh, gmesh):
+    """global p = 1 node id of every local node of a part: HexSubMesh.node_ids, or a brick's lattice position"""
+    if hasattr(mesh, "node_ids"):
+        return mesh.node_ids(1)
+    N, GN = mesh.nodes_per_dim(1), gmesh.nodes_per_dim(1)
+    z, y, x = np.meshgrid(*(np.arange(N[d]) + mesh.origin[d] for d in (2, 1, 0)), indexing="ij")
+    return (x + GN[0] * (y + GN[1] * z)).reshape(-1).astype(np.int64)

@@ -1,5 +1,6 @@
 """The mini-app driver on the `/gpu/b200` backend: what /root/reference/elasticity.c `main` does
-between CeedInit (:110) and the end of the load-increment loop (:676), for synthetic box meshes.
+between CeedInit (:110) and the end of the load-increment loop (:676), for synthetic box meshes and unstructured
+hex8 meshes, on one GPU or partitioned over several.
 
   set-up           elasticity.c:132-281  -> setuplibceed.setup_all, matops.LevelDM per level
   MatShell ctxs    elasticity.c:386-452  -> matops.setup_jacobian_ctx / setup_prolong_restrict_ctx
@@ -158,19 +159,25 @@ class Elasticity:
     def __init__(self, app, dist=None, rank=0, world=1, device_id=0, gmesh=None, coarse_rtol=1e-2, coarse="hmg",
                  assemble="coo", masked=True, overlap=True, halo="p2p", deterministic=False, amg_max_coarse=None):
         """coarse: the solve on the assembled p = 1 level -- "hmg" (geometric h-multigrid on box meshes, Jacobi-PCG on
-        unstructured ones), "pcg" (Jacobi-PCG) or "amg" (one V-cycle of smoothed-aggregation AMG, any mesh, one GPU;
-        amg_max_coarse: rows of its directly solved coarsest level, default amg.MAX_COARSE_DOFS).  masked: constrained dofs are masked in L-vector-shaped global vectors (no G2L/L2G copies, see LevelDM);
+        unstructured ones), "pcg" (Jacobi-PCG) or "amg" (one V-cycle of smoothed-aggregation AMG, any mesh; with
+        world > 1 every rank holds the whole hierarchy, amg.RedundantAMG, masked layout only; amg_max_coarse: rows of
+        its directly solved coarsest level, default amg.MAX_COARSE_DOFS).  Unstructured meshes (app.mesh) are split
+        into world parts by coordinate bisection (exodus.HexMesh.brick), box meshes into bricks.  masked: constrained
+        dofs are masked in L-vector-shaped global vectors (no G2L/L2G copies, see LevelDM);
         False: compressed PETSc-style global vectors.  deterministic: "/gpu/b200:deterministic" -- every transposed
         restriction sums in the serial /cpu/self order (no FP64 atomics anywhere on the path)."""
         if coarse == "amg" and world > 1:
-            raise NotImplementedError("coarse='amg': the smoothed-aggregation AMG coarse solve runs on one GPU; "
-                                      "partitioned AMG is not implemented (use coarse='hmg' or 'pcg' with world > 1)")
+            # checked before any device work: the redundant AMG gathers every rank's element matrices and right-hand
+            # side through the process group, and exists only for the masked layout
+            if not masked:
+                raise NotImplementedError("coarse='amg' with world > 1 needs the masked layout (masked=True)")
+            if dist is None:
+                raise NotImplementedError("coarse='amg' with world > 1 runs the redundant AMG over torch.distributed: "
+                                          "pass the process group (dist); without one the AMG runs on one GPU only")
         self.app, self.dist = app, dist
         halo_mode = halo
         grid = grid_for(world)
         if app.mesh is not None:
-            if world > 1:
-                raise NotImplementedError("partitioned runs need a brick-partitioned box mesh; -mesh files run on one GPU")
             gmesh = app.mesh
         self.gmesh = gmesh if gmesh is not None else BoxMesh(n=app.n, perturb=app.perturb, seed=0)
         self.mesh = self.gmesh.brick(grid, rank, interface_first=masked and overlap) if world > 1 else self.gmesh
@@ -236,9 +243,12 @@ class Elasticity:
         if coarse == "amg":
             if self.levels[0].coo is None:
                 raise ValueError("coarse='amg' needs the element matrices of the p = 1 level (assemble='coo', fused operator)")
-            from .amg import MAX_COARSE_DOFS, SmoothedAggregationAMG
-            amg_solver = SmoothedAggregationAMG(self.dms[0], self.mesh,
-                                                max_coarse=MAX_COARSE_DOFS if amg_max_coarse is None else amg_max_coarse)
+            from .amg import MAX_COARSE_DOFS, RedundantAMG, SmoothedAggregationAMG
+            mc = MAX_COARSE_DOFS if amg_max_coarse is None else amg_max_coarse
+            if world > 1:
+                amg_solver = RedundantAMG(self.dms[0], self.mesh, self.gmesh, faces, dist, max_coarse=mc)
+            else:
+                amg_solver = SmoothedAggregationAMG(self.dms[0], self.mesh, max_coarse=mc)
         self.pc = solver.PMultigrid(self.V, self.levels, self.transfers, coarse_rtol=coarse_rtol, h_dms=h_dms,
                                     amg=amg_solver)
         self.U = self.dms[fine].create_global_vector()

@@ -8,6 +8,8 @@ two side sets that `-bc_clamp 1,2` refers to).
   the set of (vertex id, integer trilinear weight) pairs with non-zero weight, which is the same for every element
   sharing the vertex / edge / face it lies on (GLL points are symmetric, so edge and face orientations cannot
   disagree) -- no coordinate hashing, no tolerance.
+* `HexMesh.brick` / `HexSubMesh`: one part of a recursive coordinate bisection of the elements, for partitioned runs
+  (the DMPlexDistribute step of setupdm.c:58-64); halo.Halo builds the shared-node sets from the parts' node ids.
 * `tube_mesh`: a synthetic quarter/half/full tube of hexes with the two end faces as side sets 1 and 2, used by the
   tests (the reference's own files are read where /root/reference is mounted, never copied).
 """
@@ -85,7 +87,8 @@ def write_exodus(path, coords, connect_tensor, sidesets):
 
 
 class HexMesh:
-    """Conforming hex8 mesh, trilinear geometry; same interface as mesh.BoxMesh for single-rank runs."""
+    """Conforming hex8 mesh, trilinear geometry; same interface as mesh.BoxMesh (brick() gives a part of it for
+    partitioned runs)."""
     structured = False
     elem_order = None
     n_interface = 0
@@ -190,6 +193,113 @@ class HexMesh:
                 loc = self._side_nodes(p, *_SIDE[int(s)])
                 m[ids[np.asarray(el)[sd == s]][:, loc].reshape(-1)] = True
         return m
+
+    # ---------------------------------------------------------------- partition
+    def partition(self, nparts):
+        """list of nparts ascending global element-id arrays: recursive coordinate bisection of the element centroids.
+        Each step splits the longest centroid extent of the current set into nparts//2 and nparts - nparts//2 parts with
+        element counts in proportion; the sort is stable with the element id as tie-break, so every rank computes the
+        same partition without communication."""
+        key = ("parts", nparts)
+        if key in self._cache:
+            return self._cache[key]
+        cen = self.vertices[self.connect].mean(axis=1)
+        parts = []
+
+        def split(ids, k):
+            if k == 1:
+                parts.append(np.sort(ids))
+                return
+            c = cen[ids]
+            axis = int(np.argmax(c.max(axis=0) - c.min(axis=0))) if ids.size else 0
+            ids = ids[np.lexsort((ids, c[:, axis]))]
+            k1 = k // 2
+            n1 = ids.size * k1 // k
+            split(ids[:n1], k1)
+            split(ids[n1:], k - k1)
+
+        split(np.arange(self.nelem, dtype=np.int64), int(nparts))
+        empty = [r for r, p in enumerate(parts) if p.size == 0]
+        if empty:
+            raise ValueError(f"partition of {self.nelem} elements into {nparts} parts leaves part(s) {empty} empty")
+        self._cache[key] = parts
+        return parts
+
+    def part_node_ids(self, nparts, p):
+        """per part: ascending global ids of the degree-p nodes it holds"""
+        key = ("part_nodes", nparts, p)
+        if key not in self._cache:
+            ids = self._level(p)[0]
+            self._cache[key] = [np.unique(ids[e]) for e in self.partition(nparts)]
+        return self._cache[key]
+
+    def brick(self, grid, rank, interface_first=False):
+        """Part `rank` of a prod(grid)-way partition (HexMesh.partition) as a HexSubMesh, the counterpart of
+        BoxMesh.brick.  interface_first: the elements with a vertex held by another part come first (n_interface of
+        them, padded to a multiple of 16), so that an operator application can start the halo exchange before the
+        interior elements; a vertex held by another part is a superset of a shared dof at every degree."""
+        k = int(np.prod(grid))
+        elems = self.partition(k)[rank]
+        order, nif = None, 0
+        if interface_first:
+            held = np.zeros(self.vertices.shape[0], dtype=np.int64)
+            for v in self.part_node_ids(k, 1):
+                held[v] += 1
+            touch = (held[self.connect[elems]] > 1).any(axis=1)
+            order = np.concatenate([np.flatnonzero(touch), np.flatnonzero(~touch)])
+            nif = int(touch.sum())
+            nif = min(order.size, (nif + 15) // 16 * 16) if nif else 0
+        return HexSubMesh(self, elems if order is None else elems[order], order, nif)
+
+
+class HexSubMesh:
+    """One part of a partitioned HexMesh, with the HexMesh interface the DM and set-up code use.  Local node ids of
+    every degree run over the part's nodes in ascending global (parent topological) id; `elem_ids` are the global ids
+    of the rows of offsets(); row i is the part's element elem_order[i] in ascending-id order (None: that order).
+    Dirichlet masks and node coordinates are the parent's, restricted to the part, so a node on a clamped side set
+    is masked on every part that holds it, also where the part touches the node through an edge only."""
+    structured = False
+
+    def __init__(self, parent, elem_ids, elem_order, n_interface):
+        self.parent, self.elem_ids = parent, np.asarray(elem_ids, dtype=np.int64)
+        self.elem_order, self.n_interface = elem_order, int(n_interface)
+        self.nelem = self.elem_ids.size
+        self._cache = {}
+        self.vertices = parent.vertices[self.node_ids(1)]
+
+    def _level(self, p):
+        if p not in self._cache:
+            gids = self.parent._level(p)[0][self.elem_ids]
+            nodes = np.unique(gids)
+            self._cache[p] = (np.searchsorted(nodes, gids), nodes)
+        return self._cache[p]
+
+    def node_ids(self, p):
+        """ascending global ids of the local degree-p nodes (local -> global)"""
+        return self._level(p)[1]
+
+    def num_nodes(self, p):
+        return self.node_ids(p).size
+
+    def lsize(self, p, ncomp=3):
+        return ncomp * self.num_nodes(p)
+
+    def offsets(self, p, ncomp=3, node_perm=None):
+        ids = self._level(p)[0]
+        if node_perm is not None:
+            ids = node_perm[ids]
+        off = ids * ncomp
+        assert off.max() < 2 ** 31
+        return np.ascontiguousarray(off.astype(np.int32))
+
+    def coord_lvector(self):
+        return self.vertices.reshape(-1).copy()
+
+    def node_coords(self, p):
+        return self.parent.node_coords(p)[self.node_ids(p)]
+
+    def boundary_mask(self, p, faces="all"):
+        return self.parent.boundary_mask(p, faces)[self.node_ids(p)]
 
 
 def tube_mesh(nr=2, nt=8, nz=4, r0=0.5, r1=1.0, length=2.0, angle=2 * np.pi):

@@ -1,10 +1,11 @@
-"""Halo exchange for brick-partitioned box meshes: the PetscSF stand-in behind
+"""Halo exchange for partitioned meshes: the PetscSF stand-in behind
 DMGlobalToLocal(INSERT_VALUES) / DMLocalToGlobal(ADD_VALUES) (/root/reference/src/matops.c:33,57).
 
 DMPlexDistribute with overlap 0 (/root/reference/src/setupdm.c:58-64) partitions ELEMENTS; mesh
 nodes on partition interfaces are duplicated in the local vectors and owned by exactly one rank.
-Here the partition is a grid of bricks and an interface node is owned by the LOWEST rank that
-holds it.  Two collective steps, both neighbour point-to-point (<= 26 neighbours, 7 for 2x2x2):
+Here the partition is a grid of bricks of a box mesh (mesh.BoxMesh.brick) or a coordinate bisection of an
+unstructured mesh (exodus.HexMesh.brick), and an interface node is owned by the LOWEST rank that holds it.
+Two collective steps, both neighbour point-to-point (bricks: <= 26 neighbours, 7 for 2x2x2; at most 32):
 
   owner_to_ghost(Xloc)      owners send interface values, ghosts overwrite   (G2L, INSERT)
   ghost_to_owner_add(Yloc)  ghosts send partial sums, owners accumulate       (L2G, ADD)
@@ -31,44 +32,73 @@ def _ranges(mesh_n, grid, p):
     return out
 
 
+MAX_NEIGHBOURS = 32   # B200_HALO_MAX_NEIGHBOURS (include/b200_kernels.h)
+
+
+def _brick_sets(gmesh, grid, rank, p):
+    """Brick partition of a box: (local node count, shared {r: local node ids in global lexicographic order},
+    owner [local node] = lowest rank holding it)."""
+    px, py, pz = grid
+    rng = _ranges(gmesh.n, grid, p)
+    me = (rank % px, (rank // px) % py, rank // (px * py))
+    lo = [rng[d][me[d]][0] for d in range(3)]
+    hi = [rng[d][me[d]][1] for d in range(3)]
+    N = [hi[d] - lo[d] + 1 for d in range(3)]  # local nodes per axis
+    nnodes = N[0] * N[1] * N[2]
+    owner = np.full((N[2], N[1], N[0]), rank, dtype=np.int64)
+    shared = {}
+    lidx = np.arange(nnodes).reshape(N[2], N[1], N[0])
+    for dz in (-1, 0, 1):
+        for dy in (-1, 0, 1):
+            for dx in (-1, 0, 1):
+                if dx == dy == dz == 0:
+                    continue
+                nb = (me[0] + dx, me[1] + dy, me[2] + dz)
+                if not all(0 <= nb[d] < grid[d] for d in range(3)):
+                    continue
+                r = nb[0] + px * (nb[1] + py * nb[2])
+                sl = []
+                for d, dd in enumerate((dx, dy, dz)):
+                    # overlap of my node range with the neighbour's along axis d
+                    a = max(lo[d], rng[d][nb[d]][0]); b = min(hi[d], rng[d][nb[d]][1])
+                    assert a <= b
+                    sl.append(slice(a - lo[d], b - lo[d] + 1))
+                ids = lidx[sl[2], sl[1], sl[0]].reshape(-1)  # z,y,x order == global lexicographic order
+                shared[r] = ids
+                sub = owner[sl[2], sl[1], sl[0]]
+                np.minimum(sub, r, out=sub)
+    return nnodes, shared, owner.reshape(-1)
+
+
+def _part_sets(gmesh, grid, rank, p):
+    """Element partition of an unstructured mesh (exodus.HexMesh.brick): the same triple as _brick_sets, from the
+    parts' global node ids at degree p.  A shared set lists its nodes in ascending global id, the same order on both
+    sides; every rank computes this from the global mesh alone."""
+    nodes = gmesh.part_node_ids(int(np.prod(grid)), p)
+    mine = nodes[rank]
+    owner = np.full(mine.size, rank, dtype=np.int64)
+    shared = {}
+    for r, other in enumerate(nodes):
+        if r == rank:
+            continue
+        _, ids, _ = np.intersect1d(mine, other, assume_unique=True, return_indices=True)
+        if ids.size:
+            shared[r] = ids.astype(np.int64)
+            np.minimum.at(owner, ids, r)
+    return mine.size, shared, owner
+
+
 class Halo:
     def __init__(self, gmesh, grid, rank, p, dist=None, device=None, ncomp=3):
         self.dist, self.rank, self.grid, self.p = dist, rank, grid, p
-        px, py, pz = grid
-        rng = _ranges(gmesh.n, grid, p)
-        me = (rank % px, (rank // px) % py, rank // (px * py))
-        lo = [rng[d][me[d]][0] for d in range(3)]
-        hi = [rng[d][me[d]][1] for d in range(3)]
-        N = [hi[d] - lo[d] + 1 for d in range(3)]  # local nodes per axis
-        self.nnodes = N[0] * N[1] * N[2]
-        owner = np.full((N[2], N[1], N[0]), rank, dtype=np.int64)
+        sets = _brick_sets if getattr(gmesh, "structured", True) else _part_sets
         # shared[r] = local node indices (in a canonical GLOBAL order) shared with neighbour r
-        self.neighbours = []
-        shared = {}
-        lidx = np.arange(self.nnodes).reshape(N[2], N[1], N[0])
-        for dz in (-1, 0, 1):
-            for dy in (-1, 0, 1):
-                for dx in (-1, 0, 1):
-                    if dx == dy == dz == 0:
-                        continue
-                    nb = (me[0] + dx, me[1] + dy, me[2] + dz)
-                    if not all(0 <= nb[d] < grid[d] for d in range(3)):
-                        continue
-                    r = nb[0] + px * (nb[1] + py * nb[2])
-                    sl = []
-                    for d, dd in enumerate((dx, dy, dz)):
-                        # overlap of my node range with the neighbour's along axis d
-                        a = max(lo[d], rng[d][nb[d]][0]); b = min(hi[d], rng[d][nb[d]][1])
-                        assert a <= b
-                        sl.append(slice(a - lo[d], b - lo[d] + 1))
-                    ids = lidx[sl[2], sl[1], sl[0]].reshape(-1)  # z,y,x order == global lexicographic order
-                    shared[r] = ids
-                    sub = owner[sl[2], sl[1], sl[0]]
-                    np.minimum(sub, r, out=sub)
-                    self.neighbours.append(r)
-        self.neighbours.sort()
-        self.owned_node_mask = (owner == rank).reshape(-1)
-        own = owner.reshape(-1)
+        self.nnodes, shared, own = sets(gmesh, grid, rank, p)
+        self.neighbours = sorted(shared)
+        if len(self.neighbours) > MAX_NEIGHBOURS:
+            raise ValueError(f"rank {rank} shares nodes with {len(self.neighbours)} ranks; the halo exchange handles at "
+                             f"most {MAX_NEIGHBOURS} neighbours")
+        self.owned_node_mask = own == rank
         dev = device if device is not None else ("cuda" if torch.cuda.is_available() and dist is not None and dist.get_backend() == "nccl" else "cpu")
         self.device = torch.device(dev)
 

@@ -125,6 +125,13 @@ class BoxMesh:
         assert off.max() < 2 ** 31
         return np.ascontiguousarray(off.astype(np.int32))
 
+    @property
+    def elem_ids(self):
+        """global element ids (lexicographic in the `gn` box) of the rows of offsets()"""
+        ez, ey, ex = np.meshgrid(*(np.arange(self.n[d]) + self.origin[d] for d in (2, 1, 0)), indexing="ij")
+        ids = (ex + self.gn[0] * (ey + self.gn[1] * ez)).reshape(-1).astype(np.int64)
+        return ids if self.elem_order is None else ids[self.elem_order]
+
     def node_coords(self, p):
         """(num_nodes, 3) physical coordinates of the degree-p GLL nodes (trilinear geometry)."""
         P = p + 1
