@@ -60,3 +60,26 @@ class OracleProblem:
 
 def rel_err(a, b):
     return np.linalg.norm(np.asarray(a) - np.asarray(b)) / max(np.linalg.norm(np.asarray(b)), 1e-300)
+
+
+def lattice_ids(N):
+    """(i, j, k) of every node of an (Nx, Ny, Nz) node lattice, x fastest"""
+    k, j, i = np.meshgrid(np.arange(N[2]), np.arange(N[1]), np.arange(N[0]), indexing="ij")
+    return i.reshape(-1), j.reshape(-1), k.reshape(-1)
+
+
+def dense_from_stencil(sv, N):
+    """Dense matrix of a 27-point block stencil in the layout of b200_stencil27_spmv,
+    sv[((dx+1) + 3(dy+1) + 9(dz+1))*3 + b][row]; entries that point outside the lattice are not read."""
+    n = 3 * int(np.prod(N))
+    i, j, k = lattice_ids(N)
+    A = np.zeros((n, n))
+    for o in range(27):
+        dx, dy, dz = o % 3 - 1, (o // 3) % 3 - 1, o // 9 - 1
+        ok = (i + dx >= 0) & (i + dx < N[0]) & (j + dy >= 0) & (j + dy < N[1]) & (k + dz >= 0) & (k + dz < N[2])
+        colnode = (i + dx) + N[0] * ((j + dy) + N[1] * (k + dz))
+        for a in range(3):
+            for b in range(3):
+                r = np.flatnonzero(ok) * 3 + a
+                A[r, colnode[ok] * 3 + b] = sv[o * 3 + b, r]
+    return A

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import OracleProblem, rel_err
+from helpers import OracleProblem, dense_from_stencil, lattice_ids, rel_err
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
@@ -69,25 +69,6 @@ def test_stencil_galerkin_kernel_is_PtAP(Nc):
     Nf = tuple(2 * v - 1 for v in Nc)
     nf, nc = 3 * int(np.prod(Nf)), 3 * int(np.prod(Nc))
     rng = np.random.default_rng(3)
-
-    def lattice_ids(N):
-        k, j, i = np.meshgrid(np.arange(N[2]), np.arange(N[1]), np.arange(N[0]), indexing="ij")
-        return i.reshape(-1), j.reshape(-1), k.reshape(-1)
-
-    def dense_from_stencil(sv, N):
-        n = 3 * int(np.prod(N))
-        i, j, k = lattice_ids(N)
-        A = np.zeros((n, n))
-        for o in range(27):
-            dx, dy, dz = o % 3 - 1, (o // 3) % 3 - 1, o // 9 - 1
-            ok = (i + dx >= 0) & (i + dx < N[0]) & (j + dy >= 0) & (j + dy < N[1]) & (k + dz >= 0) & (k + dz < N[2])
-            colnode = (i + dx) + N[0] * ((j + dy) + N[1] * (k + dz))
-            for a in range(3):
-                for b in range(3):
-                    r = np.flatnonzero(ok) * 3 + a
-                    A[r, colnode[ok] * 3 + b] = sv[o * 3 + b, r]
-        return A
-
     sv = rng.standard_normal((81, nf))
     # entries that point outside the fine lattice are zero by construction of the assembled matrix
     i, j, k = lattice_ids(Nf)
