@@ -848,7 +848,9 @@ k_transfer(const __grid_constant__ XferMats<PC, PF> m, int nelem, const int *__r
       val[it] = smem[el * SE + (fc - el * 3 * NO3)];
       dst[it] = __ldg(oout + node) + (fc - node * 3);
     }
-    if (!TR && inject) {  // every element sharing the node stores the same interpolant
+    // inject: the elements sharing a node store the same interpolant there, bit for bit when they share their local
+    // axes; a differently oriented neighbour contracts in another order and may differ in the last bit
+    if (!TR && inject) {
 #pragma unroll
       for (int it = 0; it < NIT; it++)
         if (tid + it * NT < total) out[dst[it]] = val[it];
@@ -947,7 +949,7 @@ k_transfer(const __grid_constant__ XferMats<PC, PF> m, int nelem, const int *__r
 #pragma unroll
         for (int i = 0; i < NI; i++) s += JM(xx, i) * l[i];
         const int o = __ldg(oout + (b * NO + a) * NO + xx);
-        if (!TR && inject) {  // every element sharing the node stores the same interpolant
+        if (!TR && inject) {  // same interpolant at every holder up to the last bit (see the default form above)
           out[o + c] = s;
           continue;
         }

@@ -699,6 +699,13 @@ int CeedBasisCreateTensorH1Lagrange(Ceed ceed, CeedInt dim, CeedInt ncomp, CeedI
       c1 = c2;
     }
   }
+  /* at a point that is one of the nodes the Lagrange basis is exactly a unit vector; the recurrence can round it
+   * (1 + 2^-52 at the end point of the Pc = 4 -> Pf = 5 Gauss-Lobatto interpolation), and then two elements sharing a
+   * fine node of the p-multigrid prolongation interpolate different values there */
+  for (int i = 0; i < Q; i++)
+    for (int j = 0; j < P; j++)
+      if (qref[i] == nodes[j])
+        for (int k = 0; k < P; k++) B[i * P + k] = k == j ? 1.0 : 0.0;
   return CeedBasisCreateTensorH1(ceed, dim, ncomp, P, Q, B, D, qref, qw, basis);
 }
 

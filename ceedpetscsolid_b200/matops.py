@@ -341,7 +341,7 @@ class UserMultProlongRestr:
     ceed: object
     memType: int = MEM_DEVICE
     fusedScale: object = None   # CeedVector of multVec handed to the fused transfer kernels (None: separate passes)
-    inject: bool = False        # prolongation stores the interpolant (complete on every holder of a node)
+    inject: bool = False        # prolongation stores the interpolant (complete, to rounding, on every holder of a node)
 
 
 def setup_prolong_restrict_ctx(dmC, dmF, ceed, dataC, dataF, userC, userF, memType=MEM_DEVICE, fuse_scaling=True):
@@ -365,8 +365,11 @@ def setup_prolong_restrict_ctx(dmC, dmF, ceed, dataC, dataF, userC, userF, memTy
         # the prolongation stores the interpolant at every fine node (no atomics, no pre-zeroed output)
         fused = ceed.Vector(multVec.numel())
         fused.set_array(multVec, MEM_DEVICE, USE_POINTER)
-        # owner/ghost layouts ADD the ghost copies into the owner afterwards: they need partial sums, not complete values
-        inject = dmF.halo is None or dmF.shared
+        # owner/ghost layouts ADD the ghost copies into the owner afterwards: they need partial sums, not complete values.
+        # The injected value is the same at every holder of a node only to the last bit: elements sharing it with other
+        # local axes contract in another order, and the last store wins.  Deterministic mode therefore sums the scaled
+        # element copies in a fixed order (and, partitioned, exchanges them like every other operator).
+        inject = (dmF.halo is None or dmF.shared) and not ceed.is_deterministic
         dataF.opProlong.set_transfer_scaling(fused, inject=inject)
         dataF.opRestrict.set_transfer_scaling(fused)
     return UserMultProlongRestr(dmC=dmC, dmF=dmF, locVecC=userC.Xloc, locVecF=userF.Xloc, multVec=multVec,

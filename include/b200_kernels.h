@@ -284,7 +284,8 @@ int b200_stencil27_galerkin(int Ncx, int Ncy, int Ncz, const double *d_fine, dou
  * (after prolongation / before restriction, matops.c:149,176).
  * inject (prolongation with d_mult only): out_L[fine node] = interpolant, stored instead of summed and scaled --
  * the elements sharing a fine node all interpolate the same value there (continuous coarse field), so
- * sum x 1/multiplicity is that value; no atomics, no pre-zeroed output, no read of d_mult. */
+ * sum x 1/multiplicity is that value; no atomics, no pre-zeroed output, no read of d_mult.  Bit for bit only
+ * where the sharing elements have the same local axes: a differently oriented one contracts in another order. */
 int b200_apply_transfer(int transpose, int nelem, int Pc, int Pf, const double *h_interpCtoF,
                         const int *d_offc, const int *d_offf, const double *d_mult, int inject,
                         const double *d_in, double *d_out, double *d_evec);

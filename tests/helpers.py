@@ -58,6 +58,52 @@ class OracleProblem:
                                         self.offsets, self.qdata, self.gradu, self.lsize, self.which)
 
 
+def cube_rotations():
+    """The 24 proper rotations of the reference cube as (perm, flip): local axis d of a rotated element runs along
+    old local axis perm[d], reversed where flip[d].  Reflections are left out: they would turn detJ negative."""
+    import itertools
+    out = []
+    for perm in itertools.permutations(range(3)):
+        sign = np.linalg.det(np.eye(3)[list(perm)])
+        for flip in itertools.product((0, 1), repeat=3):
+            if sign * (-1) ** sum(flip) > 0:
+                out.append((perm, flip))
+    assert len(out) == 24
+    return out
+
+
+def reoriented(mesh, seed=0):
+    """exodus.HexMesh with the elements of `mesh` (a HexMesh, or anything with vertices and offsets(1) such as a
+    BoxMesh), each re-listed under a seeded random one of the 24 cube rotations: the same conforming mesh, but
+    neighbouring elements no longer share their local axes.  Side sets are renumbered to the rotated local faces."""
+    from ceedpetscsolid_b200.exodus import _SIDE, HexMesh
+    coords = np.asarray(mesh.vertices, dtype=np.float64).reshape(-1, 3)
+    conn = np.asarray(mesh.connect if hasattr(mesh, "connect") else mesh.offsets(1) // 3, dtype=np.int64)
+    rots = cube_rotations()
+    pick = np.random.default_rng(seed).integers(0, 24, conn.shape[0])
+    # tensor vertex t' = i' + 2 j' + 4 k' of the rotated element is old vertex t with v[perm[d]] = v'[d] ^ flip[d]
+    tables = []
+    for perm, flip in rots:
+        tab = np.empty(8, dtype=np.int64)
+        for t2 in range(8):
+            v2 = [(t2 >> d) & 1 for d in range(3)]
+            v = [0, 0, 0]
+            for d in range(3):
+                v[perm[d]] = v2[d] ^ flip[d]
+            tab[t2] = v[0] + 2 * v[1] + 4 * v[2]
+        tables.append(tab)
+    new = np.stack([conn[e, tables[r]] for e, r in enumerate(pick)])
+    sidesets = {}
+    face = {s: [t for t in range(8) if ((t >> ax) & 1) == side] for s, (ax, side) in _SIDE.items()}
+    for sid, (els, sides) in getattr(mesh, "sidesets", {}).items():
+        ns = []
+        for e, s in zip(np.asarray(els), np.asarray(sides)):
+            target = set(conn[e, face[int(s)]])
+            ns.append(next(s2 for s2 in face if set(new[e, face[s2]]) == target))
+        sidesets[sid] = (np.asarray(els), np.asarray(ns, dtype=np.int64))
+    return HexMesh(coords, new, sidesets)
+
+
 def rel_err(a, b):
     return np.linalg.norm(np.asarray(a) - np.asarray(b)) / max(np.linalg.norm(np.asarray(b)), 1e-300)
 

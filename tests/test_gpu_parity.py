@@ -197,3 +197,40 @@ def test_prolong_restrict_with_scaling_inside_the_kernel(G, masked):
         g.data[level].opRestrict.set_transfer_scaling(None)
         c = rng.standard_normal(lc)
         assert rel_err(g.apply(g.data[level].opProlong, c, lf), oracle.transfer(False, g.mesh.nelem, pc + 1, pf + 1, offc, offf, c, lf)) < TOL
+
+
+def max_rel(got, ref):
+    return np.abs(np.asarray(got) - ref).max() / np.abs(ref).max()
+
+
+@pytest.mark.parametrize("resource", ["/gpu/b200", "/gpu/b200:deterministic"], ids=["default", "deterministic"])
+@pytest.mark.parametrize("problem,p", [("linElas", 4), ("hyperSS", 4), ("hyperFS", 4), ("hyperFS", 3)])
+def test_reoriented_tube_every_level_and_transfer(G, resource, problem, p):
+    """a tube whose elements are listed under random cube rotations (neighbours with different local axes), uniform
+    p-multigrid: every level's Jacobian and diagonal, both transfers between every pair of levels -- at degree 4 the
+    pairs (2,5), (3,5), (4,5), (5,5) and the transfers (2,3), (3,4), (4,5) -- against the oracle, elementwise"""
+    from oracle import oracle
+    from ceedpetscsolid_b200.exodus import tube_mesh
+    from helpers import reoriented
+    mesh = reoriented(tube_mesh(2, 6, 2), seed=5)
+    g = G.GpuProblem(problem, None, p, multigrid="uniform", mesh=mesh, resource=resource)
+    assert g.degrees == list(range(1, p + 1))
+    o = OracleProblem(problem, None, p, mesh=mesh)
+    assert max_rel(g.residual(), o.residual_fine(o.u_fine)) < TOL
+    rng = np.random.default_rng(p)
+    for level, deg in enumerate(g.degrees):
+        ol = OracleProblem(problem, None, p, pl=deg, mesh=mesh)
+        assert g.data[level].opJacob.is_fused
+        x = rng.standard_normal(ol.lsize)
+        assert max_rel(g.jacobian(level, x), ol.jacobian(x)) < TOL, (level, deg)
+        assert max_rel(g.diagonal(level), ol.diagonal()) < TOL, (level, deg)
+        if level == 0:
+            continue
+        pc, pf = g.degrees[level - 1], deg
+        offc, offf = mesh.offsets(pc), mesh.offsets(pf)
+        lc, lf = mesh.lsize(pc), mesh.lsize(pf)
+        c, f = rng.standard_normal(lc), rng.standard_normal(lf)
+        d = g.data[level]
+        assert d.opProlong.is_fused and d.opRestrict.is_fused
+        assert max_rel(g.apply(d.opProlong, c, lf), oracle.transfer(False, mesh.nelem, pc + 1, pf + 1, offc, offf, c, lf)) < TOL
+        assert max_rel(g.apply(d.opRestrict, f, lc), oracle.transfer(True, mesh.nelem, pc + 1, pf + 1, offc, offf, f, lc)) < TOL
