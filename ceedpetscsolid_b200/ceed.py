@@ -168,6 +168,11 @@ _proto("b200_bsr_spmv", _i, _i, _i, _vp, _vp, _vp, _vp, _vp)
 _proto("b200_bsr_pairs_product", _i, _i, _i, _sz, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp)
 _proto("b200_bsr_transpose_gather", _i, _i, _sz, _vp, _vp, _vp)
 _proto("b200_bsr_assemble_elem", _sz, _vp, _vp, _vp, _vp)
+_proto("b200_jit_read_source", C.c_char_p, _pvp, C.c_char_p, _sz)
+_proto("b200_jit_free_source", _vp, restype=None)
+_proto("b200_jit_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, C.POINTER(_i))
+_proto("b200_jit_program", _i, restype=C.c_char_p)
+_proto("b200_jit_compile_count", restype=C.c_ulonglong)
 
 # sentinels are exported data symbols holding pointers
 def _sentinel(name):
@@ -499,6 +504,34 @@ class Operator(_Obj):
         f = C.c_int()
         self._chk(lib.CeedOperatorIsFusedB200(self.h, C.byref(f)))
         return bool(f.value)
+
+
+def jit_compile(path, name, in_sizes, out_sizes):
+    """The compile half of "/gpu/b200:jit" without a device: the QFunction `name` of the source file `path` (quoted
+    includes inlined) with the given field sizes, compiled by NVRTC for sm_100a (cached per process).  Returns the
+    handle; raises CeedError with the reason (unreadable file, NVRTC log)."""
+    text, err = C.c_void_p(), C.create_string_buffer(1024)
+    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
+        raise CeedError(err.value.decode())
+    h = C.c_int(-1)
+    try:
+        rc = lib.b200_jit_compile(text, str(path).encode(), name.encode(), len(in_sizes), (C.c_int * 8)(*in_sizes),
+                                  len(out_sizes), (C.c_int * 8)(*out_sizes), C.byref(h))
+    finally:
+        lib.b200_jit_free_source(text)
+    b2(rc)
+    return h.value
+
+
+def jit_program(handle):
+    """Program text NVRTC compiled for a jit_compile handle (the user source with the generated kernel)."""
+    p = lib.b200_jit_program(int(handle))
+    return p.decode() if p is not None else None
+
+
+def jit_compile_count():
+    """NVRTC compilations run by this process (each distinct program is compiled once)."""
+    return int(lib.b200_jit_compile_count())
 
 
 def launch_count():

@@ -7,7 +7,7 @@
 namespace b200 {
 cudaStream_t g_stream = 0;
 unsigned long long g_launches = 0;
-static char g_err[512] = "";
+static char g_err[8192] = "";  // room for an NVRTC log (b200_jit.cu)
 
 int set_error(cudaError_t e, const char *what) {
   snprintf(g_err, sizeof g_err, "CUDA error %d (%s) in %s", (int)e, cudaGetErrorString(e), what);

@@ -12,7 +12,8 @@
  *   FUSED     residual / Jacobian operators of the three material models -> one kernel
  *             (b200_apply_residual / b200_apply_jacobian); transfer operators -> b200_apply_transfer
  *   GENERIC   everything else: restriction, basis and QFunction kernels chained on the device
- * There is no CPU fallback: a QFunction the backend does not recognise is an error.
+ * There is no CPU fallback: a QFunction the backend does not recognise is an error, unless the resource carries
+ * ":jit" -- then it is compiled from its source file with NVRTC (b200_jit.cu) and runs on the generic path.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -26,6 +27,7 @@
 #define B200_PIPE_CHUNKS 16
 #define B200_PIPE_MIN_ELEMS 8192 /* per chunk: enough CTAs to fill the GPU several times over */
 #define CEED_B200_RESOURCE "/gpu/b200"
+#define CEED_B200_ERRMSG 8192 /* room for an NVRTC log */
 
 /* ------------------------------------------------------------------ objects */
 typedef struct JCacheEntry {
@@ -40,10 +42,12 @@ struct Ceed_private {
   char resource[128];
   int refcount;
   CeedErrorHandler eh;
-  char errmsg[1024];
+  char errmsg[CEED_B200_ERRMSG];
   JCacheEntry *jcaches;
   /* "/gpu/b200:deterministic": transposed restrictions sum their E-vector in the serial /cpu/self order */
   int deterministic;
+  /* "/gpu/b200:jit": QFunctions without a matching built-in body are compiled from their source file (op_setup) */
+  int jit;
   double *det_evec;      /* device scratch E-vector shared by the fused kernels (stream-ordered reuse) */
   size_t det_evec_bytes;
 };
@@ -98,6 +102,8 @@ struct CeedQFunction_private {
   size_t ctxsize;
   int identity_size;
   int guard_done;  /* the caller's host function has been compared with the device body (qf_guard) */
+  int jit_handle;  /* >= 0: runs the NVRTC-compiled kernel b200_jit_apply(jit_handle) instead of a built-in body */
+  size_t jit_ctx_min; /* context bytes copied at least (what the built-in body of the same name reads) */
 };
 
 typedef struct {
@@ -144,7 +150,7 @@ const char *const CeedEvalModes[] = {"none", "interpolation", "gradient", "", "d
                                      "curl", "", "", "", "", "", "", "", "quadrature weights", 0};
 
 /* ------------------------------------------------------------------ errors */
-static char g_last_error[1024];
+static char g_last_error[CEED_B200_ERRMSG];
 static CeedErrorHandler g_default_eh = NULL; /* NULL = CeedErrorAbort (upstream default) */
 
 int CeedErrorAbort(Ceed ceed, const char *file, int line, const char *func, int ecode, const char *format,
@@ -164,9 +170,9 @@ int CeedErrorReturn(Ceed ceed, const char *file, int line, const char *func, int
 int CeedErrorStore(Ceed ceed, const char *file, int line, const char *func, int ecode, const char *format,
                    va_list *args) {
   char *dst = ceed ? ceed->errmsg : g_last_error;
-  int n = snprintf(dst, 1024, "%s:%d in %s(): ", file, line, func);
-  if (n < 1024) vsnprintf(dst + n, 1024 - n, format, *args);
-  if (ceed) memcpy(g_last_error, dst, 1024);
+  int n = snprintf(dst, CEED_B200_ERRMSG, "%s:%d in %s(): ", file, line, func);
+  if (n < CEED_B200_ERRMSG) vsnprintf(dst + n, CEED_B200_ERRMSG - n, format, *args);
+  if (ceed) memcpy(g_last_error, dst, CEED_B200_ERRMSG);
   return ecode;
 }
 static int CeedErrorImpl(Ceed ceed, const char *file, int line, const char *func, int ecode, const char *format, ...) {
@@ -197,6 +203,14 @@ int CeedResetErrorMessage(Ceed ceed, const char **errmsg) {
 }
 
 /* ------------------------------------------------------------------ Ceed */
+/* ":<word>" present as a whole qualifier of the resource */
+static int has_qualifier(const char *resource, const char *word) {
+  const size_t n = strlen(word);
+  for (const char *p = strchr(resource, ':'); p; p = strchr(p + 1, ':'))
+    if (!strncmp(p + 1, word, n) && (p[1 + n] == ':' || p[1 + n] == 0)) return 1;
+  return 0;
+}
+
 int CeedInit(const char *resource, Ceed *ceed) {
   *ceed = NULL;
   if (!resource || strncmp(resource, CEED_B200_RESOURCE, strlen(CEED_B200_RESOURCE)))
@@ -216,6 +230,7 @@ int CeedInit(const char *resource, Ceed *ceed) {
   if (!c) return CeedError(NULL, 3, "out of memory");
   snprintf(c->resource, sizeof c->resource, "%s", resource);
   c->deterministic = strstr(resource, ":deterministic") != NULL;
+  c->jit = has_qualifier(resource, "jit");
   c->refcount = 1;
   c->eh = g_default_eh ? g_default_eh : CeedErrorAbort;
   *ceed = c;
@@ -782,6 +797,7 @@ int CeedQFunctionCreateInterior(Ceed ceed, CeedInt vlength, CeedQFunctionUser f,
   const char *colon = strrchr(q->source, ':');
   snprintf(q->name, sizeof q->name, "%s", colon ? colon + 1 : q->source);
   q->qf_id = qf_lookup(q->name); /* unknown names are reported when an operator tries to run them */
+  q->jit_handle = -1;
   *qf = q;
   return 0;
 }
@@ -880,7 +896,7 @@ static int is_passive(CeedVector v) { return v && v != CEED_VECTOR_ACTIVE && v !
  * the host (b200_qfunction_apply_host: the same __host__ __device__ code).  A mismatch is a loud error.  Covers the
  * hot-path QFunctions (SetupGeo, residual F and Jacobian dF of the three models); skipped when no host pointer was
  * given (bindings without one) or CEED_B200_SKIP_QF_GUARD is set. */
-static int qf_guard(CeedQFunction qf) {
+static int qf_guard(CeedQFunction qf, int *differs) {
   Ceed ceed = qf->ceed;
   if (qf->guard_done || !qf->f || getenv("CEED_B200_SKIP_QF_GUARD")) return 0;
   const int id = qf->qf_id;
@@ -943,15 +959,47 @@ static int qf_guard(CeedQFunction qf) {
       if (fabs(out_user[i][k]) > scale) scale = fabs(out_user[i][k]);
       if (fabs(out_user[i][k] - out_dev[i][k]) > diff) diff = fabs(out_user[i][k] - out_dev[i][k]);
     }
-    if (!(diff <= 1e-10 * (scale > 1e-300 ? scale : 1e-300)))
+    if (!(diff <= 1e-10 * (scale > 1e-300 ? scale : 1e-300))) {
+      if (differs) { /* "/gpu/b200:jit": op_setup compiles the caller's source instead */
+        *differs = 1;
+        return 0;
+      }
       return CeedError(ceed, 1,
                        "%s: the QFunction at %s does not compute what this backend's device body for \"%s\" computes "
                        "(output \"%s\": max difference %.3e at scale %.3e on the known-answer points).  The backend runs its "
                        "own hand-written body for the names it recognises and would silently ignore a modified source; "
-                       "there is no JIT of user headers and no CPU fallback.",
+                       "there is no CPU fallback (the \":jit\" resource qualifier compiles the source instead).",
                        CEED_B200_RESOURCE, qf->source, qf->name, qf->out[i].name, diff, scale);
+    }
   }
   qf->guard_done = 1;
+  return 0;
+}
+
+/* "/gpu/b200:jit": compile the QFunction from the file of its "<file>:<Name>" locator (b200_jit.cu) */
+static int qf_jit_compile(CeedQFunction qf, int guard_differs) {
+  Ceed ceed = qf->ceed;
+  const char *why = guard_differs ? " (the QFunction guard found that the caller's function differs from this backend's "
+                                    "built-in body for this name, so it is compiled from its source)" : "";
+  const char *colon = strrchr(qf->source, ':');
+  if (!colon || colon == qf->source)
+    return CeedError(ceed, 1, "%s: QFunction \"%s\": locator \"%s\" names no source file (\"<file>:<Name>\")%s",
+                     CEED_B200_RESOURCE, qf->name, qf->source, why);
+  char path[sizeof qf->source], err[1024];
+  snprintf(path, sizeof path, "%.*s", (int)(colon - qf->source), qf->source);
+  char *text = NULL;
+  if (b200_jit_read_source(path, &text, err, sizeof err))
+    return CeedError(ceed, 1, "%s: QFunction \"%s\": %s%s", CEED_B200_RESOURCE, qf->name, err, why);
+  int in_sizes[MAXF], out_sizes[MAXF], h = -1;
+  for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
+  for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
+  const int rc = b200_jit_compile(text, path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, &h);
+  b200_jit_free_source(text);
+  if (rc) return CeedError(ceed, rc, "%s: QFunction \"%s\" from %s: %s%s", CEED_B200_RESOURCE, qf->name, path, b200_last_error(), why);
+  qf->jit_handle = h;
+  /* the reference declares the Physics context with sizeof(pointer) (setuplibceed.c:826); the built-in bodies read
+     {nu, E} whatever ctxsize says, so a guard-routed material model gets at least those 16 bytes too */
+  qf->jit_ctx_min = guard_differs && qf->qf_id != B200_QF_SETUPGEO ? sizeof(b200_physics) : 0;
   return 0;
 }
 
@@ -961,11 +1009,24 @@ static int op_setup(CeedOperator op) {
     if (!op->in[i].set) return CeedError(op->ceed, 1, "operator field \"%s\" of QFunction %s not set", qf->in[i].name, qf->name);
   for (int i = 0; i < qf->nout; i++)
     if (!op->out[i].set) return CeedError(op->ceed, 1, "operator field \"%s\" of QFunction %s not set", qf->out[i].name, qf->name);
+  /* "/gpu/b200:jit": an unknown name, or a recognised one whose caller function the guard finds different, is compiled
+     from its source and runs on the generic path; gallery:Identity and a passing (or impossible) guard keep the
+     built-in body */
+  if (op->ceed->jit && qf->jit_handle < 0 && qf->qf_id != B200_QF_IDENTITY) {
+    int differs = 0;
+    if (qf->qf_id != B200_QF_NONE) CeedChk(qf_guard(qf, &differs));
+    if (qf->qf_id == B200_QF_NONE || differs) CeedChk(qf_jit_compile(qf, differs));
+  }
+  if (qf->jit_handle >= 0) {
+    op->kind = OP_GENERIC;
+    return 0;
+  }
   if (qf->qf_id == B200_QF_NONE)
     return CeedError(op->ceed, 1,
-                     "%s: QFunction \"%s\" (%s) is not one this backend has a device body for; there is no CPU fallback",
+                     "%s: QFunction \"%s\" (%s) is not one this backend has a device body for; there is no CPU fallback "
+                     "(the \":jit\" resource qualifier compiles it from its source)",
                      CEED_B200_RESOURCE, qf->name, qf->source);
-  CeedChk(qf_guard(qf));
+  CeedChk(qf_guard(qf, NULL));
   op->kind = OP_GENERIC;
   const int id = qf->qf_id;
   const int is_res = id == B200_QF_LINELAS_F || id == B200_QF_HYPERSS_F || id == B200_QF_HYPERFS_F;
@@ -1143,6 +1204,16 @@ static int op_run_qfunction(CeedOperator op, CeedInt nelem, CeedInt nq, const do
     const size_t qsz = sizeof(double) * (size_t)nelem * qf->out[i].size * nq;
     CeedChk(grow(ceed, &op->qbuf[MAXF + i], &op->qbytes[MAXF + i], qsz));
     qout[i] = op->qbuf[MAXF + i];
+  }
+  if (qf->jit_handle >= 0) {
+    /* the context bytes are copied from the caller's host pointer at every apply, as for the built-in bodies */
+    const size_t bytes = qf->ctxsize > qf->jit_ctx_min ? qf->ctxsize : qf->jit_ctx_min;
+    if (bytes > B200_JIT_MAX_CTX)
+      return CeedError(ceed, 1, "%s: QFunction %s has a context of %zu bytes; a JIT-compiled QFunction takes at most %d",
+                       CEED_B200_RESOURCE, qf->name, bytes, B200_JIT_MAX_CTX);
+    if (bytes && !qf->ctx) return CeedError(ceed, 1, "QFunction %s needs a context (CeedQFunctionSetContext)", qf->name);
+    B2(ceed, b200_jit_apply(qf->jit_handle, qf->ctx, bytes, nelem, nq, qf->nin, qin, qf->nout, qout));
+    return 0;
   }
   /* context: read through the caller's host pointer at apply time, whatever ctxsize says
      (Physics {nu, E}: 2 doubles; constant forcing vector: 3 doubles, declared as sizeof(double),

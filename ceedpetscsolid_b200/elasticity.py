@@ -157,7 +157,8 @@ class Elasticity:
     """Builds the whole solver stack for one rank (one GPU)."""
 
     def __init__(self, app, dist=None, rank=0, world=1, device_id=0, gmesh=None, coarse_rtol=1e-2, coarse="hmg",
-                 assemble="coo", masked=True, overlap=True, halo="p2p", deterministic=False, amg_max_coarse=None):
+                 assemble="coo", masked=True, overlap=True, halo="p2p", deterministic=False, amg_max_coarse=None,
+                 qf_locators=None):
         """coarse: the solve on the assembled p = 1 level -- "hmg" (geometric h-multigrid on box meshes, Jacobi-PCG on
         unstructured ones), "pcg" (Jacobi-PCG) or "amg" (one V-cycle of smoothed-aggregation AMG, any mesh; with
         world > 1 every rank holds the whole hierarchy, amg.RedundantAMG, masked layout only; amg_max_coarse: rows of
@@ -165,7 +166,11 @@ class Elasticity:
         into world parts by coordinate bisection (exodus.HexMesh.brick), box meshes into bricks.  masked: constrained
         dofs are masked in L-vector-shaped global vectors (no G2L/L2G copies, see LevelDM);
         False: compressed PETSc-style global vectors.  deterministic: "/gpu/b200:deterministic" -- every transposed
-        restriction sums in the serial /cpu/self order (no FP64 atomics anywhere on the path)."""
+        restriction sums in the serial /cpu/self order (no FP64 atomics anywhere on the path).  qf_locators:
+        {"apply": "<file>:<Name>", "jacob": "<file>:<Name>"} replaces the residual / Jacobian QFunctions of app.problem
+        (same fields) by user QFunctions, compiled at set-up on the "/gpu/b200:jit" resource.  Their operators run on
+        the generic path, so the p = 1 level is not fused: box meshes assemble it by colouring, unstructured meshes by
+        column probing, and coarse="amg" is refused.  Strain energy and diagnostics keep the problem's stock model."""
         if coarse == "amg" and world > 1:
             # checked before any device work: the redundant AMG gathers every rank's element matrices and right-hand
             # side through the process group, and exists only for the masked layout
@@ -181,9 +186,11 @@ class Elasticity:
             gmesh = app.mesh
         self.gmesh = gmesh if gmesh is not None else BoxMesh(n=app.n, perturb=app.perturb, seed=0)
         self.mesh = self.gmesh.brick(grid, rank, interface_first=masked and overlap) if world > 1 else self.gmesh
-        self.ceed = libceed.Ceed(f"/gpu/b200:device_id={device_id}" + (":deterministic" if deterministic else ""))
+        self.ceed = libceed.Ceed(f"/gpu/b200:device_id={device_id}" + (":deterministic" if deterministic else "")
+                                 + (":jit" if qf_locators else ""))
         self.degrees, self.data, self.phys = setuplibceed.setup_all(self.ceed, self.mesh, app.problem, app.degree, app.nu,
-                                                                    app.E, app.qextra, app.multigrid)
+                                                                    app.E, app.qextra, app.multigrid,
+                                                                    qf_locators=qf_locators)
         if app.test_mode:
             app.forcing = "mms"
         faces = "all" if app.test_mode else list(app.clamp.keys())

@@ -85,9 +85,22 @@ def create_restriction(ceed, mesh, P, ncomp, node_perm=None):
     return ceed.ElemRestriction(mesh.nelem, P ** 3, ncomp, 1, ncomp * mesh.num_nodes(P - 1), off)
 
 
-def setup_fine_level(ceed, mesh, problem, degree, phys, data, qextra=0, node_perm=None):
+def problem_options(problem, qf_locators=None):
+    """PROBLEM_OPTIONS[problem] with the residual ("apply") and Jacobian ("jacob") QFunction locators replaced by those
+    of qf_locators.  The problem still decides the field layout; a locator the backend has no built-in body for needs
+    the "/gpu/b200:jit" resource, which compiles it from its "<file>:<Name>" source."""
+    opt = dict(PROBLEM_OPTIONS[problem])
+    if qf_locators:
+        unknown = set(qf_locators) - {"apply", "jacob"}
+        if unknown:
+            raise ValueError(f"qf_locators: only 'apply' and 'jacob' can be replaced (got {sorted(unknown)})")
+        opt.update(qf_locators)
+    return opt
+
+
+def setup_fine_level(ceed, mesh, problem, degree, phys, data, qextra=0, node_perm=None, qf_locators=None):
     """SetupLibceedFineLevel (setuplibceed.c:243-545, the parts on the hot path)."""
-    opt = PROBLEM_OPTIONS[problem]
+    opt = problem_options(problem, qf_locators)
     P, Q = degree + 1, degree + 1 + qextra
     dim = ncompx = ncompu = 3
     qdatasize = opt["qdatasize"]
@@ -250,9 +263,10 @@ def setup_true_solution(ceed, mesh, data, P):
     return out
 
 
-def setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra=0, node_perm=None, multigrid=True):
+def setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra=0, node_perm=None, multigrid=True,
+                qf_locators=None):
     """SetupLibceedLevel (setuplibceed.c:748-863): data = list of CeedData, fine level last."""
-    opt = PROBLEM_OPTIONS[problem]
+    opt = problem_options(problem, qf_locators)
     fine = len(degrees) - 1
     P = degrees[level] + 1
     Q = degrees[fine] + 1 + qextra
@@ -274,8 +288,9 @@ def setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra=0, node_
     if opt["nonlinear"]:
         d.qfJacob.add_input("gradu", ncompu * dim, EVAL_NONE)
     d.qfJacob.add_output("deltadv", ncompu * dim, EVAL_GRAD)
-    # the reference passes sizeof(phys) == sizeof(pointer) here (:826); tolerated by the backend
-    d.qfJacob.set_context(phys, size=8)
+    # the reference passes sizeof(phys) == sizeof(pointer) here (:826); tolerated by the backend for its built-in
+    # bodies.  A user Jacobian (qf_locators) is compiled at run time and given exactly ctxsize bytes: pass the struct.
+    d.qfJacob.set_context(phys, size=None if qf_locators and "jacob" in qf_locators else 8)
     d.opJacob = ceed.Operator(d.qfJacob)
     d.opJacob.set_field("deltadu", d.Erestrictu, d.basisu, VECTOR_ACTIVE)
     d.opJacob.set_field("qdata", df.Erestrictqdi, BASIS_COLLOCATED, df.qdata)
@@ -296,13 +311,18 @@ def setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra=0, node_
     return d
 
 
-def setup_all(ceed, mesh, problem, degree, nu=0.3, E=1.0, qextra=0, multigrid="logarithmic", node_perm=None):
+def setup_all(ceed, mesh, problem, degree, nu=0.3, E=1.0, qextra=0, multigrid="logarithmic", node_perm=None,
+              qf_locators=None):
     """The reference's set-up sequence (elasticity.c:255-281): fine level first, then every level
-    coarse to fine.  Returns (degrees, [CeedData per level], phys)."""
+    coarse to fine.  Returns (degrees, [CeedData per level], phys).  qf_locators: {"apply": ..., "jacob": ...}
+    overriding the problem's residual / Jacobian QFunction locators (problem_options); energy and diagnostic
+    operators keep the problem's own."""
+    problem_options(problem, qf_locators)  # reject bad keys before any device work
     degrees = level_degrees(degree, multigrid)
     phys = Physics(nu, E)
     data = [CeedData() for _ in degrees]
-    setup_fine_level(ceed, mesh, problem, degree, phys, data[-1], qextra, node_perm)
+    setup_fine_level(ceed, mesh, problem, degree, phys, data[-1], qextra, node_perm, qf_locators)
     for level in range(len(degrees)):
-        setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra, node_perm, multigrid != "none")
+        setup_level(ceed, mesh, problem, degrees, level, phys, data, qextra, node_perm, multigrid != "none",
+                    qf_locators)
     return degrees, data, phys

@@ -311,6 +311,28 @@ int b200_bsr_transpose_gather(int br, int bc, size_t nblocks, const int *idx, co
 int b200_bsr_assemble_elem(size_t nblocks, const long long *ptr, const long long *src, const double *evals,
                            double *vals);
 
+/* ---- K11: user QFunctions compiled at run time with NVRTC ("/gpu/b200:jit", csrc/b200_jit.cu) ---------------------
+ * b200_jit_read_source (host only): the program text of the QFunction source file `path` (used as given), every quoted
+ *   #include "..." that exists next to its includer inlined recursively between #line directives.  *text: free with
+ *   b200_jit_free_source.  On failure returns != 0 with the reason (naming the path) in err.
+ * b200_jit_compile (no device needed): text + the generated kernel for QFunction `name` with the given field sizes
+ *   (Q-vectors [elem][size][nq]), compiled by NVRTC for sm_100a unless the same program was compiled before in this
+ *   process; *handle names it.  Errors carry the NVRTC log (about 4 KB at most) in b200_last_error().
+ * b200_jit_apply: one launch on the backend stream; the context (at most B200_JIT_MAX_CTX bytes) is copied from the
+ *   host pointer at every call.  The user function's return code is ignored.
+ * b200_jit_compile_count: NVRTC compilations run by this process.  b200_jit_program: the compiled program text. */
+#define B200_JIT_MAX_CTX 2048
+#define B200_JIT_MAX_FIELD 64
+#define B200_JIT_MAXF 8
+int b200_jit_read_source(const char *path, char **text, char *err, size_t errlen);
+void b200_jit_free_source(char *text);
+int b200_jit_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes, int nout,
+                     const int *out_sizes, int *handle);
+int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, int nq, int nin, const double *const *d_in,
+                   int nout, double *const *d_out);
+unsigned long long b200_jit_compile_count(void);
+const char *b200_jit_program(int handle);
+
 #ifdef __cplusplus
 }
 #endif
