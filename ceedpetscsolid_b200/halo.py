@@ -306,7 +306,9 @@ class Halo:
             lib.b200_free(buf)
         self._p2p, self._p2p_buf = None, None
 
-    def _map_neighbours(self, infos, total, timeout_s):
+    def _map_neighbours(self, infos, total, timeout_s, bases=None):
+        """bases: {neighbour rank: device address of its window} to use as they are, instead of opening the IPC
+        handles of `infos` (windows that live in this process, e.g. several virtual ranks on one device)."""
         import ctypes as C
         from .ceed import b2, lib
         buf = self._p2p_buf
@@ -321,12 +323,16 @@ class Halo:
             info = infos[r]
             ra, rb = info["views"][self.rank]
             assert rb - ra == b - a, "shared sets of a rank pair must have the same size on both sides"
-            base = C.c_void_p()
-            b2(lib.b200_ipc_open((C.c_ubyte * 64).from_buffer_copy(info["handle"]), C.byref(base)))
-            self._p2p_open.append(base)
+            if bases is None:
+                opened = C.c_void_p()
+                b2(lib.b200_ipc_open((C.c_ubyte * 64).from_buffer_copy(info["handle"]), C.byref(opened)))
+                self._p2p_open.append(opened)
+                base = opened.value
+            else:
+                base = int(bases[r])
             for par in (0, 1):
-                remote[par][s] = base.value + (par * info["total"] + ra) * 8
-            rflag[s] = base.value + 2 * info["total"] * 8 + info["neighbours"].index(self.rank) * 8
+                remote[par][s] = base + (par * info["total"] + ra) * 8
+            rflag[s] = base + 2 * info["total"] * 8 + info["neighbours"].index(self.rank) * 8
         h = C.c_void_p()
         b2(lib.b200_halo_create(nn, seg_start, remote[0], remote[1], rflag, self.share_cat.data_ptr(), total, buf,
                                 self.udof.numel(), self.udof.data_ptr(), self.uptr.data_ptr(), self.uent.data_ptr(),
