@@ -105,6 +105,7 @@ _proto("CeedOperatorLinearAssembleSymbolic", _vp, C.POINTER(_i), C.POINTER(C.POI
 _proto("CeedOperatorLinearAssemble", _vp, _vp)
 _proto("CeedOperatorDestroy", _pvp)
 _proto("CeedOperatorIsFusedB200", _vp, C.POINTER(_i))
+_proto("CeedOperatorIsJitFusedB200", _vp, C.POINTER(_i))
 _proto("CeedOperatorApplyAddRangeB200", _vp, _vp, _vp, _i, _i)
 _proto("CeedOperatorSetTransferScalingB200", _vp, _vp, _i)
 _proto("CeedOperatorApplyPartitionedB200", _vp, _vp, _vp, _i, _vp, _vp, _i)
@@ -172,6 +173,7 @@ _proto("b200_jit_read_source", C.c_char_p, _pvp, C.c_char_p, _sz)
 _proto("b200_jit_free_source", _vp, restype=None)
 _proto("b200_jit_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, C.POINTER(_i))
 _proto("b200_jit_program", _i, restype=C.c_char_p)
+_proto("b200_jit_fused_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, _i, _i, _i, _i, C.POINTER(_i))
 _proto("b200_jit_compile_count", restype=C.c_ulonglong)
 
 # sentinels are exported data symbols holding pointers
@@ -505,6 +507,13 @@ class Operator(_Obj):
         self._chk(lib.CeedOperatorIsFusedB200(self.h, C.byref(f)))
         return bool(f.value)
 
+    @property
+    def is_jit_fused(self):
+        """True if Apply runs the fused operator kernel generated around a JIT-compiled user QFunction (K12)"""
+        f = C.c_int()
+        self._chk(lib.CeedOperatorIsJitFusedB200(self.h, C.byref(f)))
+        return bool(f.value)
+
 
 def jit_compile(path, name, in_sizes, out_sizes):
     """The compile half of "/gpu/b200:jit" without a device: the QFunction `name` of the source file `path` (quoted
@@ -517,6 +526,24 @@ def jit_compile(path, name, in_sizes, out_sizes):
     try:
         rc = lib.b200_jit_compile(text, str(path).encode(), name.encode(), len(in_sizes), (C.c_int * 8)(*in_sizes),
                                   len(out_sizes), (C.c_int * 8)(*out_sizes), C.byref(h))
+    finally:
+        lib.b200_jit_free_source(text)
+    b2(rc)
+    return h.value
+
+
+def jit_fused_compile(path, name, in_sizes, out_sizes, active_in, active_out, P, Q):
+    """The compile half of K12 without a device: the fused operator kernel around QFunction `name` of `path` for the
+    basis (P, Q), with field active_in / active_out as the active gradient and every other field passive (q-blocked).
+    Returns the handle (cached per process, as jit_compile)."""
+    text, err = C.c_void_p(), C.create_string_buffer(1024)
+    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
+        raise CeedError(err.value.decode())
+    h = C.c_int(-1)
+    try:
+        rc = lib.b200_jit_fused_compile(text, str(path).encode(), name.encode(), len(in_sizes),
+                                        (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
+                                        int(active_in), int(active_out), int(P), int(Q), C.byref(h))
     finally:
         lib.b200_jit_free_source(text)
     b2(rc)

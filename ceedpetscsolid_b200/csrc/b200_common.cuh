@@ -12,6 +12,8 @@ extern cudaStream_t g_stream;
 extern unsigned long long g_launches;
 int set_error(cudaError_t e, const char *what);
 int set_error_msg(const char *msg);
+// Gc = D pinv(B), Gc B = D: the collocated derivative of a tensor basis (b200_fused.cu); != 0 if B is rank-deficient
+int collocated_grad_1d(int P, int Q, const double *B, const double *D, double *Gc);
 
 #define B200_CHECK(call)                                   \
   do {                                                     \

@@ -1021,6 +1021,9 @@ static int collocated_grad(int P, int Q, const double *B, const double *D, doubl
   return err <= 1e-12 * nrm ? 0 : 2;
 }
 
+// the same for the generated fused kernels of user QFunctions (b200_jit.cu)
+int collocated_grad_1d(int P, int Q, const double *B, const double *D, double *Gc) { return collocated_grad(P, Q, B, D, Gc); }
+
 template <typename K> static int opt_in_smem(K kern, size_t bytes) {
   if (bytes > 48 * 1024) B200_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   return 0;

@@ -10,8 +10,15 @@
 // no link-time dependency on it.  Each distinct program (text plus options) is compiled once per process.
 // Load half (b200_jit_apply): the cubin is loaded once with cudaLibraryLoadData.  A cudaLibrary_t is
 // context-independent: the runtime loads its kernel into each device's context on first use there.
+//
+// K12 (b200_jit_fused_compile / b200_jit_fused_apply): the same user program with the fused operator kernel of
+// b200_jit_fused.cuh around it, for one (P, Q) of B200_FOR_PQ and one assignment of the fields to the active gradient
+// and the passive q-blocked vectors.  The template is embedded at build time (b200_jit_fused.inc, a raw string made
+// from the header by the Makefile); the lattice constants come from b200_apply_smem_layout, so the built-in and the
+// generated kernels cannot disagree on the layout.
 #include <dlfcn.h>
 #include <nvrtc.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <mutex>
@@ -54,13 +61,31 @@ struct Nvrtc {
   const char *(*errstr)(nvrtcResult);
 };
 
+// the K12 template (b200_jit_fused.cuh) as a string
+const char *const kFusedTemplate =
+#include "b200_jit_fused.inc"
+    ;
+
+// K12 blocks per SM asked of ptxas for the full-group kernel (__launch_bounds__ min blocks): 128 threads x 3 blocks
+// leave 168 registers a thread.  Measured at P = Q = 5, C3 (profiles/jit_fused_ctas_ab.txt): the fastest setting at
+// which port_HyperFSdF neither spills nor has a stack frame; 4 blocks (128 registers) ran 7 % faster with 112 bytes of
+// spills.  B200_JIT_FUSED_CTAS overrides it (tuning runs).
+const int kFusedCtas = 3;
+
 struct Entry {
   std::string key;     // options + program text
-  std::string kernel;  // b200_jit_<Name>
+  std::string kernel;  // b200_jit_<Name>, or b200_jit_fused_<Name> (K12: full element groups)
   std::vector<char> cubin;
   int nin = 0, nout = 0, in_size[B200_JIT_MAXF] = {}, out_size[B200_JIT_MAXF] = {};
   cudaLibrary_t lib = nullptr;
   cudaKernel_t fn = nullptr;
+  // K12 only
+  bool fused = false;
+  int P = 0, Q = 0, ai = -1, ao = -1, lay[6] = {};  // lay: b200_apply_smem_layout {SY, SZ, SC, SE, EB, NT}
+  size_t smem = 0;
+  std::string kernel_tail;  // b200_jit_fused_tail_<Name>: the partial group at the end of a range
+  cudaKernel_t fn_tail = nullptr;
+  unsigned long long smem_set = 0;  // devices on which the dynamic shared-memory limit was raised
 };
 
 std::mutex g_mu;
@@ -179,53 +204,159 @@ int compile_locked(Entry &en, const char *src_name) {
   return 0;
 }
 
+// text + generated kernel(s) -> entry; compiles unless the same program was compiled before in this process
+int find_or_compile(Entry *proto, const char *src_name, int *handle) {
+  std::lock_guard<std::mutex> lock(g_mu);
+  for (size_t i = 0; i < g_entries.size(); i++)
+    if (g_entries[i]->key == proto->key) {
+      *handle = (int)i;
+      delete proto;
+      return 0;
+    }
+  if (int rc = compile_locked(*proto, src_name && src_name[0] ? src_name : "qfunction")) {
+    delete proto;
+    return rc;
+  }
+  g_entries.push_back(proto);
+  *handle = (int)g_entries.size() - 1;
+  return 0;
+}
+
+int check_fields(const char *fn, const char *name, int nin, const int *in_sizes, int nout, const int *out_sizes) {
+  char msg[256];
+  if (!is_identifier(name)) {
+    snprintf(msg, sizeof msg, "%s: QFunction name \"%.128s\" is not a C identifier", fn, name);
+    return b200::set_error_msg(msg);
+  }
+  if (nin < 0 || nout < 1 || nin > B200_JIT_MAXF || nout > B200_JIT_MAXF) {
+    snprintf(msg, sizeof msg, "%s: need 0..8 input and 1..8 output fields", fn);
+    return b200::set_error_msg(msg);
+  }
+  for (int i = 0; i < nin + nout; i++) {
+    const int s = i < nin ? in_sizes[i] : out_sizes[i - nin];
+    if (s < 1 || s > B200_JIT_MAX_FIELD) {
+      snprintf(msg, sizeof msg, "%s: %s field %d of QFunction %.128s has %d components; a JIT QFunction "
+               "field holds 1 to %d", fn, i < nin ? "input" : "output", i < nin ? i : i - nin, name, s, B200_JIT_MAX_FIELD);
+      return b200::set_error_msg(msg);
+    }
+  }
+  return 0;
+}
+
+std::string options_line() {
+  std::string key;
+  for (int i = 0; i < kNumOptions; i++) key += std::string(kOptions[i]) + " ";
+  return key + "\n";
+}
+
+// K12: the prefix the template expects (constants, parameter structs, the point adapter), the template, the kernels
+std::string generated_fused(const char *name, int nin, const int *in_size, int nout, const int *out_size, int ai, int ao,
+                            int P, int Q, const int *lay, int ctas) {
+  std::string k;
+  char line[512];
+  auto add = [&](const char *fmt, auto... a) {
+    snprintf(line, sizeof line, fmt, a...);
+    k += line;
+  };
+  k += "\n#line 1 \"b200_jit_fused_prefix\"\n";
+  add("#define B200_K12_P %d\n#define B200_K12_Q %d\n", P, Q);
+  add("#define B200_K12_SY %d\n#define B200_K12_SZ %d\n#define B200_K12_SC %d\n#define B200_K12_SE %d\n"
+      "#define B200_K12_EB %d\n#define B200_K12_NT %d\n", lay[0], lay[1], lay[2], lay[3], lay[4], lay[5]);
+  add("struct alignas(16) b200_jit_ctx_t { unsigned char b[%d]; };\n", B200_JIT_MAX_CTX);
+  add("struct b200_k12_fields_t { const double *in[%d]; double *out[%d]; };\n", B200_JIT_MAXF, B200_JIT_MAXF);
+  k += "__device__ __forceinline__ void b200_k12_point(const b200_jit_ctx_t &ctx, const b200_k12_fields_t &f,\n"
+       "    const size_t grp, const size_t pos, const size_t cs, const double H[3][3], double W[3][3], const int padd) {\n";
+  for (int i = 0; i < nin; i++) {
+    add("  double in%d[%d];\n", i, in_size[i]);
+    if (i == ai)
+      add("#pragma unroll\n  for (int d = 0; d < 3; d++)\n#pragma unroll\n"
+          "    for (int c = 0; c < 3; c++) in%d[d * 3 + c] = H[c][d];\n", i);
+    else
+      add("  { const double *p = f.in[%d] + grp * %d + pos;\n#pragma unroll\n"
+          "    for (int c = 0; c < %d; c++) in%d[c] = __ldcs(p + c * cs); }\n", i, in_size[i], in_size[i], i);
+  }
+  for (int i = 0; i < nout; i++) add("  double out%d[%d] = {};\n", i, out_size[i]);
+  k += "  const double *ins[] = {";
+  for (int i = 0; i < nin; i++) add("%sin%d", i ? ", " : "", i);
+  k += "};\n  double *outs[] = {";
+  for (int i = 0; i < nout; i++) add("%sout%d", i ? ", " : "", i);
+  k += "};\n";
+  add("  (void)%s((void *)ctx.b, 1, ins, outs);\n", name);
+  for (int i = 0; i < nout; i++) {
+    if (i == ao)
+      add("#pragma unroll\n  for (int kk = 0; kk < 3; kk++)\n#pragma unroll\n"
+          "    for (int c = 0; c < 3; c++) W[c][kk] = out%d[kk * 3 + c];\n", i);
+    else
+      add("  { double *p = f.out[%d] + grp * %d + pos;\n"
+          "    if (padd) {\n#pragma unroll\n      for (int c = 0; c < %d; c++) p[c * cs] += out%d[c];\n"
+          "    } else {\n#pragma unroll\n      for (int c = 0; c < %d; c++) __stcs(p + c * cs, out%d[c]);\n    } }\n",
+          i, out_size[i], out_size[i], i, out_size[i], i);
+  }
+  k += "}\n#line 1 \"b200_jit_fused.cuh\"\n";
+  k += kFusedTemplate;
+  k += "\n#line 1 \"b200_jit_fused_kernels\"\n";
+  // the tail kernel runs as one CTA: occupancy is moot, so it gets every register it wants
+  const char *variant[2] = {"", "tail_"};
+  for (int v = 0; v < 2; v++)
+    add("extern \"C\" __global__ void __launch_bounds__(%d, %d) b200_jit_fused_%s%s(\n"
+        "    const __grid_constant__ b200_k12_mats_t m, const __grid_constant__ b200_jit_ctx_t ctx,\n"
+        "    const __grid_constant__ b200_k12_fields_t f, const int nelem, const int *__restrict__ offsets,\n"
+        "    const double *__restrict__ x, double *__restrict__ y, double *__restrict__ evec, const int padd) {\n"
+        "  b200_k12_body<%s>(m, ctx, f, nelem, offsets, x, y, evec, padd);\n}\n",
+        lay[5], v ? 1 : ctas, variant[v], name, v ? "false" : "true");
+  return k;
+}
+
 }  // namespace
 
 extern "C" int b200_jit_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
                                 int nout, const int *out_sizes, int *handle) {
   *handle = -1;
   if (!text || !name) return b200::set_error_msg("b200_jit_compile: NULL program text or name");
-  if (!is_identifier(name)) {
-    char msg[256];
-    snprintf(msg, sizeof msg, "b200_jit_compile: QFunction name \"%.128s\" is not a C identifier", name);
-    return b200::set_error_msg(msg);
-  }
-  if (nin < 0 || nout < 1 || nin > B200_JIT_MAXF || nout > B200_JIT_MAXF)
-    return b200::set_error_msg("b200_jit_compile: need 0..8 input and 1..8 output fields");
-  for (int i = 0; i < nin + nout; i++) {
-    const int s = i < nin ? in_sizes[i] : out_sizes[i - nin];
-    if (s < 1 || s > B200_JIT_MAX_FIELD) {
-      char msg[256];
-      snprintf(msg, sizeof msg, "b200_jit_compile: %s field %d of QFunction %.128s has %d components; a JIT QFunction "
-               "field holds 1 to %d", i < nin ? "input" : "output", i < nin ? i : i - nin, name, s, B200_JIT_MAX_FIELD);
-      return b200::set_error_msg(msg);
-    }
-  }
-  std::string key;
-  for (int i = 0; i < kNumOptions; i++) key += std::string(kOptions[i]) + " ";
-  key += "\n";
-  key += text;
-  key += generated_kernel(name, nin, in_sizes, nout, out_sizes);
-  std::lock_guard<std::mutex> lock(g_mu);
-  for (size_t i = 0; i < g_entries.size(); i++)
-    if (g_entries[i]->key == key) {
-      *handle = (int)i;
-      return 0;
-    }
+  if (int rc = check_fields("b200_jit_compile", name, nin, in_sizes, nout, out_sizes)) return rc;
   Entry *en = new Entry;
-  en->key = std::move(key);
+  en->key = options_line() + text + generated_kernel(name, nin, in_sizes, nout, out_sizes);
   en->kernel = std::string("b200_jit_") + name;
   en->nin = nin;
   en->nout = nout;
   for (int i = 0; i < nin; i++) en->in_size[i] = in_sizes[i];
   for (int i = 0; i < nout; i++) en->out_size[i] = out_sizes[i];
-  if (int rc = compile_locked(*en, src_name && src_name[0] ? src_name : "qfunction")) {
-    delete en;
-    return rc;
+  return find_or_compile(en, src_name, handle);
+}
+
+extern "C" int b200_jit_fused_compile(const char *text, const char *src_name, const char *name, int nin,
+                                      const int *in_sizes, int nout, const int *out_sizes, int active_in,
+                                      int active_out, int P, int Q, int *handle) {
+  *handle = -1;
+  if (!text || !name) return b200::set_error_msg("b200_jit_fused_compile: NULL program text or name");
+  if (int rc = check_fields("b200_jit_fused_compile", name, nin, in_sizes, nout, out_sizes)) return rc;
+  if (active_in < 0 || active_in >= nin || active_out < 0 || active_out >= nout || in_sizes[active_in] != 9 ||
+      out_sizes[active_out] != 9)
+    return b200::set_error_msg("b200_jit_fused_compile: the active input and output must be fields of 9 components");
+  int lay[6];
+  if (b200_apply_smem_layout(P, Q, lay)) {
+    char msg[160];
+    snprintf(msg, sizeof msg, "b200_jit_fused_compile: (P, Q) = (%d, %d) has no fused lattice layout", P, Q);
+    return b200::set_error_msg(msg);
   }
-  g_entries.push_back(en);
-  *handle = (int)g_entries.size() - 1;
-  return 0;
+  const char *env = getenv("B200_JIT_FUSED_CTAS");  // read at every compile: part of the program text and its key
+  const int ctas = env && atoi(env) > 0 ? atoi(env) : kFusedCtas;
+  Entry *en = new Entry;
+  en->key = options_line() + text + generated_fused(name, nin, in_sizes, nout, out_sizes, active_in, active_out, P, Q, lay, ctas);
+  en->kernel = std::string("b200_jit_fused_") + name;
+  en->kernel_tail = std::string("b200_jit_fused_tail_") + name;
+  en->nin = nin;
+  en->nout = nout;
+  for (int i = 0; i < nin; i++) en->in_size[i] = in_sizes[i];
+  for (int i = 0; i < nout; i++) en->out_size[i] = out_sizes[i];
+  en->fused = true;
+  en->P = P;
+  en->Q = Q;
+  en->ai = active_in;
+  en->ao = active_out;
+  memcpy(en->lay, lay, sizeof lay);
+  en->smem = sizeof(double) * (size_t)lay[4] * lay[3] + sizeof(int) * (size_t)lay[4] * P * P * P;
+  return find_or_compile(en, src_name, handle);
 }
 
 extern "C" unsigned long long b200_jit_compile_count(void) {
@@ -247,6 +378,7 @@ extern "C" int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, i
     std::lock_guard<std::mutex> lock(g_mu);
     if (handle < 0 || handle >= (int)g_entries.size()) return b200::set_error_msg("b200_jit_apply: bad handle");
     en = g_entries[handle];
+    if (en->fused) return b200::set_error_msg("b200_jit_apply: the handle names a fused operator program (b200_jit_fused_apply)");
     if (!en->lib) {
       B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
       B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
@@ -275,5 +407,76 @@ extern "C" int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, i
   B200_CHECK(cudaLaunchKernel((const void *)en->fn, dim3((unsigned)(nb < cap ? nb : cap)), dim3(nt), args, 0,
                               b200::g_stream));
   B200_LAUNCH_CHECK("b200_jit_apply");
+  return 0;
+}
+
+extern "C" int b200_jit_fused_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
+                                    const double *h_grad1d, const int *d_offsets, const double *d_x, double *d_y,
+                                    double *d_evec, int nin, const double *const *d_in, int nout, double *const *d_out,
+                                    int passive_add) {
+  Entry *en;
+  int dev;
+  B200_CHECK(cudaGetDevice(&dev));
+  {
+    std::lock_guard<std::mutex> lock(g_mu);
+    if (handle < 0 || handle >= (int)g_entries.size() || !g_entries[handle]->fused)
+      return b200::set_error_msg("b200_jit_fused_apply: bad handle");
+    en = g_entries[handle];
+    if (!en->lib) {
+      B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn_tail, en->lib, en->kernel_tail.c_str()));
+    }
+    // no (P, Q) of the table needs more than 48 KB today; a larger layout raises the limit once per device
+    if (en->smem > 48 * 1024 && dev >= 0 && dev < 64 && !(en->smem_set >> dev & 1)) {
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      en->smem_set |= 1ull << dev;
+    }
+  }
+  if (nin != en->nin || nout != en->nout)
+    return b200::set_error_msg("b200_jit_fused_apply: field count differs from the compiled one");
+  if (ctx_bytes > B200_JIT_MAX_CTX) {
+    char msg[160];
+    snprintf(msg, sizeof msg, "b200_jit_fused_apply: context of %zu bytes; a JIT QFunction takes at most %d", ctx_bytes,
+             B200_JIT_MAX_CTX);
+    return b200::set_error_msg(msg);
+  }
+  if (ctx_bytes && !h_ctx) return b200::set_error_msg("b200_jit_fused_apply: NULL context");
+  if (nelem <= 0) return 0;
+  const int P = en->P, Q = en->Q, P3 = P * P * P, Q3 = Q * Q * Q, EB = en->lay[4], NT = en->lay[5];
+  // B and Gc as the kernel parameter b200_k12_mats_t (sized for this (P, Q))
+  double mats[8 * 8 + 8 * 8];
+  for (int i = 0; i < Q * P; i++) mats[i] = h_interp1d[i];
+  if (b200::collocated_grad_1d(P, Q, h_interp1d, h_grad1d, mats + Q * P))
+    return b200::set_error_msg("basis: no collocated gradient with Gc*B = D (rank-deficient interp1d)");
+  JitCtx ctx;
+  memset(&ctx, 0, sizeof ctx);
+  if (ctx_bytes) memcpy(ctx.b, h_ctx, ctx_bytes);
+  JitFields f;
+  memset(&f, 0, sizeof f);
+  for (int i = 0; i < nin; i++) f.in[i] = i == en->ai ? nullptr : d_in[i];
+  for (int i = 0; i < nout; i++) f.out[i] = i == en->ao ? nullptr : d_out[i];
+  const int nfull = nelem / EB, ntail = nelem - nfull * EB;
+  if (nfull) {
+    int n = nfull * EB;
+    void *args[] = {mats, &ctx, &f, &n, &d_offsets, &d_x, &d_y, &d_evec, &passive_add};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn, dim3(nfull), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_fused_apply");
+  }
+  if (ntail) {  // the partial group at the end: the same stages with a run-time group extent, one CTA
+    const size_t e0 = (size_t)nfull * EB;
+    JitFields ft = f;
+    for (int i = 0; i < nin; i++)
+      if (ft.in[i]) ft.in[i] += e0 * en->in_size[i] * Q3;
+    for (int i = 0; i < nout; i++)
+      if (ft.out[i]) ft.out[i] += e0 * en->out_size[i] * Q3;
+    const int *off = d_offsets + e0 * P3;
+    double *ev = d_evec ? d_evec + e0 * 3 * P3 : nullptr;
+    int n = ntail;
+    void *args[] = {mats, &ctx, &ft, &n, &off, &d_x, &d_y, &ev, &passive_add};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn_tail, dim3(1), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_fused_apply(tail)");
+  }
   return 0;
 }

@@ -11,9 +11,11 @@
  * Operator execution:
  *   FUSED     residual / Jacobian operators of the three material models -> one kernel
  *             (b200_apply_residual / b200_apply_jacobian); transfer operators -> b200_apply_transfer
+ *   JIT_FUSED residual / Jacobian-shaped operators of a JIT-compiled user QFunction -> one generated kernel (K12,
+ *             b200_jit_fused_apply), compiled at the operator's first apply
  *   GENERIC   everything else: restriction, basis and QFunction kernels chained on the device
  * There is no CPU fallback: a QFunction the backend does not recognise is an error, unless the resource carries
- * ":jit" -- then it is compiled from its source file with NVRTC (b200_jit.cu) and runs on the generic path.
+ * ":jit" -- then it is compiled from its source file with NVRTC (b200_jit.cu) and runs on K12 or the generic path.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -104,6 +106,8 @@ struct CeedQFunction_private {
   int guard_done;  /* the caller's host function has been compared with the device body (qf_guard) */
   int jit_handle;  /* >= 0: runs the NVRTC-compiled kernel b200_jit_apply(jit_handle) instead of a built-in body */
   size_t jit_ctx_min; /* context bytes copied at least (what the built-in body of the same name reads) */
+  char *jit_text;     /* the program text jit_handle was compiled from: K12 compiles it again around the fused kernel */
+  char jit_path[512];
 };
 
 typedef struct {
@@ -113,7 +117,7 @@ typedef struct {
   CeedVector v;
 } OpField;
 
-enum { OP_UNSET = 0, OP_GENERIC, OP_FUSED_RESIDUAL, OP_FUSED_JACOBIAN, OP_FUSED_TRANSFER };
+enum { OP_UNSET = 0, OP_GENERIC, OP_FUSED_RESIDUAL, OP_FUSED_JACOBIAN, OP_FUSED_TRANSFER, OP_JIT_FUSED };
 
 struct CeedOperator_private {
   Ceed ceed;
@@ -126,6 +130,8 @@ struct CeedOperator_private {
   /* fused transfer operators: optional fine-side pointwise scaling (CeedOperatorSetTransferScalingB200) */
   CeedVector xfer_scale;
   int xfer_inject;
+  /* OP_JIT_FUSED: the active input / output fields; jit_fused = K12 program handle + 1 (0: not compiled yet) */
+  int jit_ai, jit_ao, jit_fused;
   /* generic-path work buffers (device), grown on demand */
   double *ebuf[2 * MAXF], *qbuf[2 * MAXF];
   size_t ebytes[2 * MAXF], qbytes[2 * MAXF];
@@ -835,6 +841,7 @@ int CeedQFunctionDestroy(CeedQFunction *qf) {
   if (q == CEED_QFUNCTION_NONE) return 0;
   if (--q->refcount > 0) return 0;
   Ceed c = q->ceed;
+  b200_jit_free_source(q->jit_text);
   free(q);
   return CeedDestroy(&c);
 }
@@ -994,13 +1001,53 @@ static int qf_jit_compile(CeedQFunction qf, int guard_differs) {
   for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
   for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
   const int rc = b200_jit_compile(text, path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, &h);
-  b200_jit_free_source(text);
-  if (rc) return CeedError(ceed, rc, "%s: QFunction \"%s\" from %s: %s%s", CEED_B200_RESOURCE, qf->name, path, b200_last_error(), why);
+  if (rc) {
+    b200_jit_free_source(text);
+    return CeedError(ceed, rc, "%s: QFunction \"%s\" from %s: %s%s", CEED_B200_RESOURCE, qf->name, path, b200_last_error(), why);
+  }
   qf->jit_handle = h;
+  b200_jit_free_source(qf->jit_text);
+  qf->jit_text = text;
+  snprintf(qf->jit_path, sizeof qf->jit_path, "%s", path);
   /* the reference declares the Physics context with sizeof(pointer) (setuplibceed.c:826); the built-in bodies read
      {nu, E} whatever ctxsize says, so a guard-routed material model gets at least those 16 bytes too */
   qf->jit_ctx_min = guard_differs && qf->qf_id != B200_QF_SETUPGEO ? sizeof(b200_physics) : 0;
   return 0;
+}
+
+/* K12 (OP_JIT_FUSED): one active EVAL_GRAD input of 9 on a 3-component offsets restriction (compstride 1, P^3 nodes)
+ * with a tensor basis whose (P, Q) has a fused layout, one active EVAL_GRAD output on the same restriction and basis
+ * matrices, and every other field EVAL_NONE on a passive vector with a q-blocked restriction of the same nelem */
+static int jit_fused_eligible(CeedOperator op) {
+  CeedQFunction qf = op->qf;
+  int ai = -1, ao = -1;
+  for (int i = 0; i < qf->nin; i++)
+    if (op->in[i].v == CEED_VECTOR_ACTIVE) { if (ai >= 0) return 0; ai = i; }
+  for (int i = 0; i < qf->nout; i++)
+    if (op->out[i].v == CEED_VECTOR_ACTIVE) { if (ao >= 0) return 0; ao = i; }
+  if (ai < 0 || ao < 0) return 0;
+  OpField *u = &op->in[ai], *vv = &op->out[ao];
+  if (!(qf->in[ai].emode == CEED_EVAL_GRAD && qf->in[ai].size == 9 && is_tensor3(u->b) && u->b->ncomp == 3 && u->r &&
+        u->r != CEED_ELEMRESTRICTION_NONE && u->r->strided == 0 && u->r->ncomp == 3 && u->r->compstride == 1 &&
+        u->r->elemsize == u->b->P * u->b->P * u->b->P && b200_fused_supported(u->b->P, u->b->Q)))
+    return 0;
+  const int Q = u->b->Q;
+  if (!(qf->out[ao].emode == CEED_EVAL_GRAD && qf->out[ao].size == 9 && vv->r == u->r &&
+        (vv->b == u->b || (is_tensor3(vv->b) && vv->b->P == u->b->P && vv->b->Q == Q &&
+                           !memcmp(vv->b->interp1d, u->b->interp1d, sizeof(double) * Q * u->b->P) &&
+                           !memcmp(vv->b->grad1d, u->b->grad1d, sizeof(double) * Q * u->b->P)))))
+    return 0;
+  for (int i = 0; i < qf->nin + qf->nout; i++) {
+    if (i == ai || i == qf->nin + ao) continue;
+    const QFField *qff = i < qf->nin ? &qf->in[i] : &qf->out[i - qf->nin];
+    OpField *f = i < qf->nin ? &op->in[i] : &op->out[i - qf->nin];
+    if (!(qff->emode == CEED_EVAL_NONE && is_passive(f->v) && is_qstrided(f->r, qff->size, Q) &&
+          f->r->nelem == u->r->nelem && (size_t)f->v->length >= (size_t)f->r->nelem * qff->size * Q * Q * Q))
+      return 0;
+  }
+  op->jit_ai = ai;
+  op->jit_ao = ao;
+  return 1;
 }
 
 static int op_setup(CeedOperator op) {
@@ -1017,8 +1064,9 @@ static int op_setup(CeedOperator op) {
     if (qf->qf_id != B200_QF_NONE) CeedChk(qf_guard(qf, &differs));
     if (qf->qf_id == B200_QF_NONE || differs) CeedChk(qf_jit_compile(qf, differs));
   }
+  op->jit_fused = 0;
   if (qf->jit_handle >= 0) {
-    op->kind = OP_GENERIC;
+    op->kind = qf->jit_text && jit_fused_eligible(op) ? OP_JIT_FUSED : OP_GENERIC;
     return 0;
   }
   if (qf->qf_id == B200_QF_NONE)
@@ -1084,7 +1132,14 @@ static int op_setup(CeedOperator op) {
 int CeedOperatorIsFusedB200(CeedOperator op, int *isFused) {
   if (op->composite) { *isFused = 0; return 0; }
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  *isFused = op->kind != OP_GENERIC;
+  *isFused = op->kind != OP_GENERIC && op->kind != OP_JIT_FUSED;
+  return 0;
+}
+
+int CeedOperatorIsJitFusedB200(CeedOperator op, int *isJitFused) {
+  if (op->composite) { *isJitFused = 0; return 0; }
+  if (op->kind == OP_UNSET) CeedChk(op_setup(op));
+  *isJitFused = op->kind == OP_JIT_FUSED;
   return 0;
 }
 
@@ -1197,6 +1252,18 @@ static int op_input_qvec(CeedOperator op, int i, CeedVector in, CeedInt nelem, C
   return 0;
 }
 
+/* context bytes of a JIT-compiled QFunction: copied from the caller's host pointer at every apply, as for the built-in
+   bodies */
+static int jit_ctx_bytes(CeedQFunction qf, size_t *bytes) {
+  Ceed ceed = qf->ceed;
+  *bytes = qf->ctxsize > qf->jit_ctx_min ? qf->ctxsize : qf->jit_ctx_min;
+  if (*bytes > B200_JIT_MAX_CTX)
+    return CeedError(ceed, 1, "%s: QFunction %s has a context of %zu bytes; a JIT-compiled QFunction takes at most %d",
+                     CEED_B200_RESOURCE, qf->name, *bytes, B200_JIT_MAX_CTX);
+  if (*bytes && !qf->ctx) return CeedError(ceed, 1, "QFunction %s needs a context (CeedQFunctionSetContext)", qf->name);
+  return 0;
+}
+
 static int op_run_qfunction(CeedOperator op, CeedInt nelem, CeedInt nq, const double **qin, double **qout) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
@@ -1206,12 +1273,8 @@ static int op_run_qfunction(CeedOperator op, CeedInt nelem, CeedInt nq, const do
     qout[i] = op->qbuf[MAXF + i];
   }
   if (qf->jit_handle >= 0) {
-    /* the context bytes are copied from the caller's host pointer at every apply, as for the built-in bodies */
-    const size_t bytes = qf->ctxsize > qf->jit_ctx_min ? qf->ctxsize : qf->jit_ctx_min;
-    if (bytes > B200_JIT_MAX_CTX)
-      return CeedError(ceed, 1, "%s: QFunction %s has a context of %zu bytes; a JIT-compiled QFunction takes at most %d",
-                       CEED_B200_RESOURCE, qf->name, bytes, B200_JIT_MAX_CTX);
-    if (bytes && !qf->ctx) return CeedError(ceed, 1, "QFunction %s needs a context (CeedQFunctionSetContext)", qf->name);
+    size_t bytes;
+    CeedChk(jit_ctx_bytes(qf, &bytes));
     B2(ceed, b200_jit_apply(qf->jit_handle, qf->ctx, bytes, nelem, nq, qf->nin, qin, qf->nout, qout));
     return 0;
   }
@@ -1431,6 +1494,72 @@ static int op_apply_fused_range(CeedOperator op, CeedVector in, CeedVector out, 
   return 0;
 }
 
+/* K12: compile the fused program at the first apply (the point program of op_setup stays for the generic diagonal) */
+static int jit_fused_handle(CeedOperator op, int *h) {
+  Ceed ceed = op->ceed;
+  CeedQFunction qf = op->qf;
+  if (!op->jit_fused) {
+    int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
+    for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
+    for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
+    CeedBasis b = op->in[op->jit_ai].b;
+    if (b200_jit_fused_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai,
+                               op->jit_ao, b->P, b->Q, &hh))
+      return CeedError(ceed, 1, "%s: fused kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
+                       qf->jit_path, b200_last_error());
+    op->jit_fused = hh + 1;
+  }
+  *h = op->jit_fused - 1;
+  return 0;
+}
+
+/* K12 on the element range [e0, e1), e0 a multiple of the q-blocked group size: the active output is added to, the
+ * passive outputs are stored (passive_add = 0, Apply) or added to (ApplyAdd) */
+static int op_apply_jit_range(CeedOperator op, CeedVector in, CeedVector out, int e0, int e1, int passive_add) {
+  Ceed ceed = op->ceed;
+  CeedQFunction qf = op->qf;
+  OpField *u = &op->in[op->jit_ai];
+  const int P = u->b->P, Q = u->b->Q, P3 = P * P * P, Q3 = Q * Q * Q, nelem = u->r->nelem;
+  if (in->length < u->r->lsize || out->length < u->r->lsize)
+    return CeedError(ceed, 1, "operator %s: active vectors shorter than the restriction's L-vector size %d", qf->name, u->r->lsize);
+  int h;
+  size_t bytes;
+  CeedChk(jit_fused_handle(op, &h));
+  CeedChk(jit_ctx_bytes(qf, &bytes));
+  double *evec = NULL;
+  if (ceed->deterministic) {
+    if (e0 != 0 || e1 != nelem)
+      return CeedError(ceed, 1, "deterministic mode: element-range applies are not supported (the ordered sum runs over the whole restriction)");
+    CeedChk(det_scratch(ceed, (size_t)nelem * 3 * P3 * sizeof(double), &evec));
+  }
+  const double *din[MAXF] = {NULL}, *x;
+  double *dout[MAXF] = {NULL}, *y;
+  for (int i = 0; i < qf->nin; i++)
+    if (i != op->jit_ai) {
+      CeedChk(vec_dev_read(op->in[i].v, &din[i]));
+      din[i] += (size_t)e0 * qf->in[i].size * Q3;
+    }
+  for (int i = 0; i < qf->nout; i++)
+    if (i != op->jit_ao) {
+      /* a store over the whole range overwrites every entry; anything else keeps the rest valid */
+      if (!passive_add && e0 == 0 && e1 == nelem) CeedChk(vec_dev_write(op->out[i].v, &dout[i]));
+      else CeedChk(vec_dev_rw(op->out[i].v, &dout[i]));
+      dout[i] += (size_t)e0 * qf->out[i].size * Q3;
+    }
+  CeedChk(vec_dev_read(in, &x));
+  CeedChk(vec_dev_rw(out, &y));
+  B2(ceed, b200_jit_fused_apply(h, qf->ctx, bytes, e1 - e0, u->b->interp1d, u->b->grad1d, u->r->d_offsets + (size_t)e0 * P3,
+                                x, y, evec, qf->nin, din, qf->nout, dout, passive_add));
+  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, y));
+  return 0;
+}
+
+/* the fused kernels on [e0, e1): built-in (passive gradu always stored) or K12 */
+static int op_apply_range(CeedOperator op, CeedVector in, CeedVector out, int e0, int e1, int passive_add) {
+  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, e0, e1, passive_add);
+  return op_apply_fused_range(op, in, out, e0, e1);
+}
+
 static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
   Ceed ceed = op->ceed;
   if (op->composite) {
@@ -1439,6 +1568,7 @@ static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
   }
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
   if (op->kind == OP_GENERIC) return op_apply_generic(op, in, out);
+  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, 0, op->in[op->jit_ai].r->nelem, 1);
   if (op->kind == OP_FUSED_TRANSFER) {
     const double *x;
     double *y;
@@ -1472,14 +1602,15 @@ int CeedOperatorApplyAddRangeB200(CeedOperator op, CeedVector in, CeedVector out
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: composite operators are not supported");
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL)
+  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL && op->kind != OP_JIT_FUSED)
     return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: operator %s does not run on the fused kernels", op->qf->name);
-  const int nelem = op->in[0].r->nelem, EB = b200_elems_per_block(op->in[0].b->Q);
+  const int ia = op->kind == OP_JIT_FUSED ? op->jit_ai : 0;
+  const int nelem = op->in[ia].r->nelem, EB = b200_elems_per_block(op->in[ia].b->Q);
   if (start < 0 || stop > nelem || start > stop || start % EB)
     return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: bad element range [%d, %d) (nelem %d, start must be a multiple of %d)",
                      start, stop, nelem, EB);
   if (start == stop) return 0;
-  return op_apply_fused_range(op, in, out, start, stop);
+  return op_apply_range(op, in, out, start, stop, 1);
 }
 
 /* /gpu/b200 extension for the p-multigrid transfer operators (Prolong_Ceed / Restrict_Ceed, matops.c:115-203): the
@@ -1514,15 +1645,16 @@ int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in, CeedVector 
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: composite operators are not supported");
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL)
+  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL && op->kind != OP_JIT_FUSED)
     return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: operator %s does not run on the fused kernels", op->qf->name);
-  const int nelem = op->in[0].r->nelem, EB = b200_elems_per_block(op->in[0].b->Q);
+  const int ia = op->kind == OP_JIT_FUSED ? op->jit_ai : 0;
+  const int nelem = op->in[ia].r->nelem, EB = b200_elems_per_block(op->in[ia].b->Q);
   if (n_interface < 0 || n_interface > nelem || (n_interface % EB && n_interface != nelem))
     return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: n_interface %d must be a multiple of %d within [0, %d]", n_interface, EB, nelem);
   double *y;
   CeedChk(CeedVectorSetValue(out, 0.0));
   if (!halo || ceed->deterministic || n_interface == 0 || n_interface == nelem) {
-    CeedChk(op_apply_fused_range(op, in, out, 0, nelem));
+    CeedChk(op_apply_range(op, in, out, 0, nelem, 0));
     CeedChk(vec_dev_rw(out, &y));
     if (halo) { B2(ceed, b200_halo_begin((b200_halo *)halo, y)); B2(ceed, b200_halo_end((b200_halo *)halo, y)); }
   } else {
@@ -1533,14 +1665,24 @@ int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in, CeedVector 
     CeedChk(vec_dev_read(in, &x));
     CeedChk(vec_dev_rw(out, &y));
     if (op->kind == OP_FUSED_JACOBIAN) CeedChk(jcache_get(op, &jc));
+    if (op->kind == OP_JIT_FUSED) {  /* compiled, and the passive vectors current on the device, before the fork */
+      int h;
+      CeedChk(jit_fused_handle(op, &h));
+      for (int i = 0; i < op->qf->nin; i++)
+        if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &x));
+      for (int i = 0; i < op->qf->nout; i++)
+        if (i != op->jit_ao) CeedChk(vec_dev_rw(op->out[i].v, &y));
+      CeedChk(vec_dev_rw(out, &y));
+      CeedChk(vec_dev_read(in, &x));
+    }
     void *side = NULL, *mainstream = b200_get_stream();
     B2(ceed, b200_halo_fork((b200_halo *)halo, &side));
     B2(ceed, b200_set_stream(side));
-    int rc = op_apply_fused_range(op, in, out, 0, n_interface);
+    int rc = op_apply_range(op, in, out, 0, n_interface, 0);
     b200_set_stream(mainstream);
     if (rc) return rc;
     B2(ceed, b200_halo_begin_forked((b200_halo *)halo, y));
-    CeedChk(op_apply_fused_range(op, in, out, n_interface, nelem));
+    CeedChk(op_apply_range(op, in, out, n_interface, nelem, 0));
     B2(ceed, b200_halo_end((b200_halo *)halo, y));
   }
   if (nmask > 0) B2(ceed, b200_mask_zero(y, d_mask, (size_t)nmask));
@@ -1570,8 +1712,10 @@ static int op_apply(CeedOperator op, CeedVector in, CeedVector out) {
     if (!v || v == CEED_VECTOR_NONE) continue;
     /* the fused residual kernel overwrites every entry of its passive output (gradu) itself */
     if (op->kind == OP_FUSED_RESIDUAL && i == 1) continue;
+    if (op->kind == OP_JIT_FUSED && i != op->jit_ao) continue;  /* K12 stores them (passive_add = 0 below) */
     CeedChk(CeedVectorSetValue(v, 0.0));
   }
+  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, 0, op->in[op->jit_ai].r->nelem, 0);
   return op_apply_add(op, in, out);
 }
 int CeedOperatorApply(CeedOperator op, CeedVector in, CeedVector out, CeedRequest *request) {

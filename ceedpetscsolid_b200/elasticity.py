@@ -169,8 +169,9 @@ class Elasticity:
         restriction sums in the serial /cpu/self order (no FP64 atomics anywhere on the path).  qf_locators:
         {"apply": "<file>:<Name>", "jacob": "<file>:<Name>"} replaces the residual / Jacobian QFunctions of app.problem
         (same fields) by user QFunctions, compiled at set-up on the "/gpu/b200:jit" resource.  Their operators run on
-        the generic path, so the p = 1 level is not fused: box meshes assemble it by colouring, unstructured meshes by
-        column probing, and coarse="amg" is refused.  Strain energy and diagnostics keep the problem's stock model."""
+        K12, the fused kernel generated around the user function (compiled at the first apply), and their diagonal on
+        the generic path.  The p = 1 level has no built-in Jacobian, so box meshes assemble it by colouring,
+        unstructured meshes by column probing, and coarse="amg" is refused.  Strain energy and diagnostics keep the problem's stock model."""
         if coarse == "amg" and world > 1:
             # checked before any device work: the redundant AMG gathers every rank's element matrices and right-hand
             # side through the process group, and exists only for the masked layout

@@ -203,7 +203,9 @@ def ApplyLocalCeedOp(X, Y, user, zero_xloc=False):
         user.Xceed.set_array(X, user.memType, USE_POINTER)
         user.Yceed.set_array(Y, user.memType, USE_POINTER)
         if user.fused is None:
-            user.fused = bool(user.op.is_fused)
+            # built-in fused kernels and K12 (the fused kernel around a JIT-compiled user QFunction) both take the
+            # one-call partitioned apply
+            user.fused = bool(user.op.is_fused or user.op.is_jit_fused)
         if X.is_cuda and user.fused and (dm.halo is None or dm.halo.handle is not None):
             # the whole MatMult in one C call: zero Y, interface elements, peer-memory halo exchange overlapped with
             # the interior elements, ordered sum of the holders' partial sums, zero the Dirichlet rows

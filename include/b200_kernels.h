@@ -333,6 +333,26 @@ int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, i
 unsigned long long b200_jit_compile_count(void);
 const char *b200_jit_program(int handle);
 
+/* ---- K12: the fused operator kernel around a JIT-compiled user QFunction (csrc/b200_jit_fused.cuh) ----------------
+ * b200_jit_fused_compile (no device needed): text + the kernel of b200_jit_fused.cuh around QFunction `name` for the
+ *   basis (P, Q) (one of b200_fused_supported; the lattice constants are those of b200_apply_smem_layout).  Field
+ *   active_in is the 9-component gradient of the 3-component offsets-restricted active vector, in[d*3 + c] = du_c/dX_d;
+ *   field active_out is its 9-component test-function gradient, out[k*3 + c].  Every other field is a passive vector
+ *   in the q-blocked CEED_STRIDES_BACKEND layout, read (inputs) or written (outputs) in place.  Compiled unless the
+ *   same program (text, name, sizes, active fields, P, Q) was compiled before; counted by b200_jit_compile_count and
+ *   shown by b200_jit_program.
+ * b200_jit_fused_apply: y_L += E^T G^T f(G E x_L, passive fields) G E on nelem elements, one launch for the full
+ *   element groups and one for a partial last group, on the backend stream.  d_offsets, d_in / d_out of the passive
+ *   fields and d_evec point at the first element of the range (a multiple of b200_elems_per_block(Q)); entries of the
+ *   active fields are ignored.  passive_add = 0 stores the passive outputs, != 0 adds to them.  d_evec as for the
+ *   built-in fused kernels (NULL: FP64 atomics; else E-vector [e][node][comp] for b200_transpose_gather_add).  The
+ *   context is copied from the host pointer at every call (at most B200_JIT_MAX_CTX bytes). */
+int b200_jit_fused_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
+                           int nout, const int *out_sizes, int active_in, int active_out, int P, int Q, int *handle);
+int b200_jit_fused_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
+                         const double *h_grad1d, const int *d_offsets, const double *d_x, double *d_y, double *d_evec,
+                         int nin, const double *const *d_in, int nout, double *const *d_out, int passive_add);
+
 #ifdef __cplusplus
 }
 #endif

@@ -190,6 +190,9 @@ CEED_EXTERN int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in,
  * Restrict_Ceed (matops.c:149,176) inside the kernel; inject != 0: the prolongation stores the interpolant */
 CEED_EXTERN int CeedOperatorSetTransferScalingB200(CeedOperator op, CeedVector scale, int inject);
 CEED_EXTERN int CeedOperatorIsFusedB200(CeedOperator op, int *isFused);
+/* 1 if the operator's Apply runs as ONE kernel generated around its JIT-compiled user QFunction ("/gpu/b200:jit", K12);
+ * such operators report 0 from CeedOperatorIsFusedB200, which means "runs on a built-in fused kernel" */
+CEED_EXTERN int CeedOperatorIsJitFusedB200(CeedOperator op, int *isJitFused);
 /* kernels launched by this library since the last reset (bench.py "gpu_launches") */
 CEED_EXTERN unsigned long long CeedB200LaunchCount(void);
 CEED_EXTERN void CeedB200LaunchCountReset(void);

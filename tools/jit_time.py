@@ -1,15 +1,18 @@
 #!/usr/bin/env python
-"""Cost of running the Jacobian QFunction through "/gpu/b200:jit" at C3 (hyperFS, p = 4, 64^3 box), in one run:
+"""Cost of user QFunctions through "/gpu/b200:jit" at C3 (hyperFS, p = 4, 64^3 box), in one run on one card:
 
-  * the built-in fused Jacobian apply (CeedOperatorApply on device L-vectors) against the same operator with
-    oracle/qf_port.c:port_HyperFSdF compiled by NVRTC, which runs on the generic path (restriction, basis, K11 point
-    kernel, transposed basis, transposed restriction); both products are checked against each other;
-  * the K11 point kernel alone on the operator's own Q-vectors, with its bytes from the shapes and its share of the
-    HBM bound (7.7 TB/s, the HGX B200 data sheet figure for one GPU);
-  * the NVRTC compile time, cold (a program this process has not compiled) and cached.
+  * the Jacobian apply (CeedOperatorApply on device L-vectors) of the built-in fused kernel against the same operator
+    with oracle/qf_port.c:port_HyperFSdF compiled by NVRTC, which runs on K12, the fused kernel generated around the
+    user function; the residual apply (gradu written) with port_HyperFSF likewise.  K12 is built with 2, 3 and 4
+    blocks per SM asked of ptxas (B200_JIT_FUSED_CTAS), and all variants are timed in alternating batches;
+  * the products checked against the built-in ones;
+  * K12's bytes from the shapes and its share of the HBM bound (7.7 TB/s, the HGX B200 data sheet figure for one GPU);
+  * the NVRTC compile time of the point program (K11) and of the fused programs, cold (programs this process has not
+    compiled) and cached.
 
-Prints the card name and power limit and one JSON line; --out also writes that line to a file.
-  python tools/jit_time.py [--n 64] [--reps 10] [--out profiles/jit_time_c3.jsonl]"""
+The generic path (restriction, basis, K11 point kernel, transposes) that JIT operators took before K12 is recorded
+in profiles/jit_time_c3.jsonl.  Prints the card name and power limit and one JSON line; --out appends it to a file.
+  python tools/jit_time.py [--n 64] [--reps 10] [--out profiles/jit_fused_time_c3.jsonl]"""
 import argparse
 import json
 import os
@@ -19,7 +22,6 @@ import sys
 import tempfile
 import time
 
-import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,6 +33,7 @@ from ceedpetscsolid_b200.mesh import BoxMesh, smooth_displacement  # noqa: E402
 QF_PORT = os.path.join(ROOT, "oracle", "qf_port.c")
 HBM_BYTES_PER_S = 7.7e12
 DP = 8
+CTAS = (2, 3, 4)
 
 
 def timeit(fn, reps, warm=2):
@@ -63,11 +66,17 @@ def compile_times():
             t0 = time.perf_counter()
             libceed.jit_compile(src, "port_HyperFSdF", [9, 10, 9], [9])
             out[f"compile_cold_{tag}_s"] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            libceed.jit_fused_compile(src, "port_HyperFSdF", [9, 10, 9], [9], 0, 0, 5, 5)
+            out[f"fused_jacobian_compile_cold_{tag}_s"] = time.perf_counter() - t0
+            t0 = time.perf_counter()
+            libceed.jit_fused_compile(src, "port_HyperFSF", [9, 10], [9, 9], 0, 0, 5, 5)
+            out[f"fused_residual_compile_cold_{tag}_s"] = time.perf_counter() - t0
         n0 = libceed.jit_compile_count()
         t0 = time.perf_counter()
         for _ in range(100):
-            libceed.jit_compile(src, "port_HyperFSdF", [9, 10, 9], [9])
-        out["compile_cached_s"] = (time.perf_counter() - t0) / 100
+            libceed.jit_fused_compile(src, "port_HyperFSdF", [9, 10, 9], [9], 0, 0, 5, 5)
+        out["fused_compile_cached_s"] = (time.perf_counter() - t0) / 100
         assert libceed.jit_compile_count() == n0
         return out
     finally:
@@ -88,69 +97,71 @@ def main():
 
     mesh = BoxMesh(n=(a.n,) * 3, perturb=0.08, seed=0)
     u = torch.from_numpy(smooth_displacement(mesh.node_coords(4)).reshape(-1)).cuda()
-    ops = {}
-    for tag, resource, locs in (("builtin", "/gpu/b200", None),
-                                ("jit", "/gpu/b200:jit", {"jacob": f"{QF_PORT}:port_HyperFSdF"})):
-        ceed = libceed.Ceed(resource)
-        degrees, data, phys = setuplibceed.setup_all(ceed, mesh, "hyperFS", 4, multigrid="none", qf_locators=locs)
-        d = data[-1]
-        uc, rc = ceed.Vector(u.numel()), ceed.Vector(u.numel())
-        r = torch.zeros_like(u)
-        uc.set_array(u); rc.set_array(r)
-        d.opApply.apply(uc, rc)          # gradu of the linearisation point
-        uc.take_array(); rc.take_array()
-        ops[tag] = (ceed, d, phys)
-        torch.cuda.synchronize()
-    assert ops["builtin"][1].opJacob.is_fused and not ops["jit"][1].opJacob.is_fused
-
     x = torch.randn_like(u)
-    ys = {}
-    for tag, (ceed, d, _) in ops.items():
-        y = torch.zeros_like(u)
-        xc, yc = ceed.Vector(u.numel()), ceed.Vector(u.numel())
-        xc.set_array(x); yc.set_array(y)
-        ys[tag] = (y, xc, yc, d)
-    t = {"builtin": [], "jit": []}
-    for _ in range(3):                   # alternate the two, several rounds
-        for tag, (y, xc, yc, d) in ys.items():
-            t[tag].append(timeit(lambda: d.opJacob.apply(xc, yc), a.reps))
-    yb, yj = ys["builtin"][0], ys["jit"][0]
-    rel = (torch.linalg.norm(yj - yb) / torch.linalg.norm(yb)).item()
-    res.update({"fused_jacobian_ms": min(t["builtin"]), "jit_jacobian_ms": min(t["jit"]),
-                "fused_jacobian_ms_all": t["builtin"], "jit_jacobian_ms_all": t["jit"],
-                "jit_over_fused": min(t["jit"]) / min(t["builtin"]), "rel_diff_jit_vs_fused": rel})
+    locs = {"apply": f"{QF_PORT}:port_HyperFSF", "jacob": f"{QF_PORT}:port_HyperFSdF"}
+    runs = {}
+    env0 = os.environ.get("B200_JIT_FUSED_CTAS")
+    for tag in ["builtin"] + [f"k12_ctas{c}" for c in CTAS]:
+        jit = tag != "builtin"
+        if jit:   # read by the fused compile at the operators' first apply, below
+            os.environ["B200_JIT_FUSED_CTAS"] = tag[len("k12_ctas"):]
+        ceed = libceed.Ceed("/gpu/b200:jit" if jit else "/gpu/b200")
+        _, data, _ = setuplibceed.setup_all(ceed, mesh, "hyperFS", 4, multigrid="none", qf_locators=locs if jit else None)
+        d = data[-1]
+        assert (d.opJacob.is_jit_fused and d.opApply.is_jit_fused) if jit else (d.opJacob.is_fused and d.opApply.is_fused)
+        r, y = torch.zeros_like(u), torch.zeros_like(u)
+        uc, rc, xc, yc = (ceed.Vector(u.numel()) for _ in range(4))
+        uc.set_array(u); rc.set_array(r); xc.set_array(x); yc.set_array(y)
+        d.opApply.apply(uc, rc)          # gradu of the linearisation point; compiles K12's residual program
+        d.opJacob.apply(xc, yc)          # compiles K12's Jacobian program
+        torch.cuda.synchronize()
+        runs[tag] = dict(ceed=ceed, d=d, r=r, y=y, uc=uc, rc=rc, xc=xc, yc=yc)
+    if env0 is None:
+        os.environ.pop("B200_JIT_FUSED_CTAS", None)
+    else:
+        os.environ["B200_JIT_FUSED_CTAS"] = env0
 
-    # K11 alone on the operator's own Q-vectors: deltadu (9), qdata (10), gradu (9) -> deltadv (9)
-    ceed, d, phys = ops["jit"]
-    nelem, nq = mesh.nelem, 5 ** 3
-    def evec(rstr, vec, ncomp):
-        ev = ceed.Vector(nelem * ncomp * nq)
-        rstr.apply(vec, ev)
-        return ev
-    qd_e, gu_e = evec(d.Erestrictqdi, d.qdata, 10), evec(d.ErestrictGradui, d.gradu, 9)
-    ddu = (torch.randn(nelem * 9 * nq, dtype=torch.float64, device="cuda") * 1e-2)
-    out = torch.empty_like(ddu)
-    h = libceed.jit_compile(QF_PORT, "port_HyperFSdF", [9, 10, 9], [9])   # the operator's program: cached
-    import ctypes as C
-    pin = (C.c_void_p * 3)(ddu.data_ptr(), qd_e.device_ptr(), gu_e.device_ptr())
-    pout = (C.c_void_p * 1)(out.data_ptr())
-    lib = libceed.lib
-    lib.b200_jit_apply.argtypes = [C.c_int, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
-                                   C.c_void_p]
-    def k11():
-        libceed.b2(lib.b200_jit_apply(h, C.addressof(phys), C.sizeof(phys), nelem, nq, 3, pin, 1, pout))
-    kt = min(timeit(k11, a.reps * 3) for _ in range(3))
-    kbytes = nelem * nq * (9 + 10 + 9 + 9) * DP
-    res.update({"k11_ms": kt, "k11_bytes": kbytes, "k11_tb_per_s": kbytes / (kt * 1e-3) / 1e12,
-                "k11_share_of_hbm_bound": kbytes / HBM_BYTES_PER_S / (kt * 1e-3),
-                "qvector_gb": nelem * nq * 9 * DP / 1e9})
+    t = {("jacobian", tag): [] for tag in runs}
+    t.update({("residual", tag): [] for tag in runs})
+    for _ in range(3):                   # alternate every variant, several rounds
+        for tag, R in runs.items():
+            t[("jacobian", tag)].append(timeit(lambda: R["d"].opJacob.apply(R["xc"], R["yc"]), a.reps))
+            t[("residual", tag)].append(timeit(lambda: R["d"].opApply.apply(R["uc"], R["rc"]), a.reps))
+    torch.cuda.synchronize()
+    for kind in ("jacobian", "residual"):
+        res[f"{kind}_ms"] = {tag: min(t[(kind, tag)]) for tag in runs}
+        res[f"{kind}_ms_all"] = {tag: t[(kind, tag)] for tag in runs}
+    rb = runs["builtin"]
+    gb = rb["d"].gradu.to_numpy()
+    for tag, R in runs.items():
+        if tag == "builtin":
+            continue
+        res[f"rel_diff_jacobian_{tag}"] = (torch.linalg.norm(R["y"] - rb["y"]) / torch.linalg.norm(rb["y"])).item()
+        res[f"rel_diff_residual_{tag}"] = (torch.linalg.norm(R["r"] - rb["r"]) / torch.linalg.norm(rb["r"])).item()
+        g = R["d"].gradu.to_numpy()
+        res[f"max_abs_diff_gradu_{tag}"] = float(abs(g - gb).max())
+    best = min((f"k12_ctas{c}" for c in CTAS), key=lambda k: res["jacobian_ms"][k] + res["residual_ms"][k])
+    res["k12_best"] = best
+    res["k12_jacobian_over_builtin"] = res["jacobian_ms"][best] / res["jacobian_ms"]["builtin"]
+    res["k12_residual_over_builtin"] = res["residual_ms"][best] / res["residual_ms"]["builtin"]
+    # K12 bytes from the shapes: offsets (4 B per node of every element), the passive per-point fields (Jacobian:
+    # qdata 10 + gradu 9 read; residual: qdata 10 read, gradu 9 written), x read once, y read and written once
+    nelem, P3, Q3, lsize = mesh.nelem, 5 ** 3, 5 ** 3, u.numel()
+    for kind, npt in (("jacobian", 19), ("residual", 19)):
+        b = nelem * (P3 * 4 + npt * Q3 * DP) + 3 * lsize * DP
+        ms = res[f"{kind}_ms"][best]
+        res[f"k12_{kind}_bytes"] = b
+        res[f"k12_{kind}_tb_per_s"] = b / (ms * 1e-3) / 1e12
+        res[f"k12_{kind}_share_of_hbm_bound"] = b / HBM_BYTES_PER_S / (ms * 1e-3)
     line = json.dumps(res)
     print(line, flush=True)
     if a.out:
         os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
         with open(a.out, "a") as f:
             f.write(line + "\n")
-    assert rel <= 1e-12, rel
+    for tag in runs:
+        if tag != "builtin":
+            assert res[f"rel_diff_jacobian_{tag}"] <= 1e-12 and res[f"rel_diff_residual_{tag}"] <= 1e-12, tag
 
 
 if __name__ == "__main__":
