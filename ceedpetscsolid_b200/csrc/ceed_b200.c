@@ -1597,7 +1597,9 @@ static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
 /* /gpu/b200 extension: ApplyAdd restricted to the elements [start, stop) of a fused residual / Jacobian operator
  * (creation order of the restriction).  Lets a partitioned caller run the elements that touch partition
  * interfaces first and overlap its halo exchange with the interior ones.  start must be a multiple of the
- * backend's element-group size (16 always is). */
+ * backend's element-group size (16 always is), and so must stop unless it is nelem: the kernels take the extent
+ * of the range's last group from the range, while the q-blocked per-point vectors (qdata, Jacobian cache, gradu,
+ * passive fields) lay out a group cut short by stop with the extent it has in the whole restriction. */
 int CeedOperatorApplyAddRangeB200(CeedOperator op, CeedVector in, CeedVector out, CeedInt start, CeedInt stop) {
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: composite operators are not supported");
@@ -1606,9 +1608,9 @@ int CeedOperatorApplyAddRangeB200(CeedOperator op, CeedVector in, CeedVector out
     return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: operator %s does not run on the fused kernels", op->qf->name);
   const int ia = op->kind == OP_JIT_FUSED ? op->jit_ai : 0;
   const int nelem = op->in[ia].r->nelem, EB = b200_elems_per_block(op->in[ia].b->Q);
-  if (start < 0 || stop > nelem || start > stop || start % EB)
-    return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: bad element range [%d, %d) (nelem %d, start must be a multiple of %d)",
-                     start, stop, nelem, EB);
+  if (start < 0 || stop > nelem || start > stop || start % EB || (stop % EB && stop != nelem))
+    return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: bad element range [%d, %d) (nelem %d; start, and stop "
+                     "unless it is nelem, must be multiples of %d)", start, stop, nelem, EB);
   if (start == stop) return 0;
   return op_apply_range(op, in, out, start, stop, 1);
 }

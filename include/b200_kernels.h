@@ -187,7 +187,11 @@ int b200_apply_smem_layout(int P, int Q, int *out);
 /* d_evec (all fused kernels): NULL = scatter-add with FP64 atomics straight into the L-vector.  Non-NULL selects
  * the DETERMINISTIC scatter: the kernel stores its element outputs to d_evec[(e*P^3 + node)*3 + comp] instead
  * (plain coalesced stores, d_y untouched) and the caller sums them into the L-vector in a fixed order with
- * b200_transpose_gather_add (layout 1). */
+ * b200_transpose_gather_add (layout 1).
+ * Sub-ranges (residual, Jacobian, diagonal): d_offsets, d_qdata / d_gradu / d_jcache and d_evec may point at the
+ * first element of a range that starts at a multiple of EB = b200_elems_per_block(Q).  nelem must then be a multiple
+ * of EB unless the range runs to the end of the q-blocked vectors: the last group's extent is taken from nelem, and
+ * the q-blocked layout of a group cut short would be that of the whole vector's group. */
 int b200_apply_residual(int problem, const b200_physics *phys, int nelem, int P, int Q,
                         const double *h_interp1d, const double *h_grad1d, const int *d_offsets,
                         const double *d_qdata, double *d_gradu, const double *d_x, double *d_y, double *d_evec);
@@ -343,8 +347,9 @@ const char *b200_jit_program(int handle);
  *   shown by b200_jit_program.
  * b200_jit_fused_apply: y_L += E^T G^T f(G E x_L, passive fields) G E on nelem elements, one launch for the full
  *   element groups and one for a partial last group, on the backend stream.  d_offsets, d_in / d_out of the passive
- *   fields and d_evec point at the first element of the range (a multiple of b200_elems_per_block(Q)); entries of the
- *   active fields are ignored.  passive_add = 0 stores the passive outputs, != 0 adds to them.  d_evec as for the
+ *   fields and d_evec point at the first element of the range (a multiple of b200_elems_per_block(Q)); nelem is a
+ *   multiple of it too unless the range runs to the end of the q-blocked passive vectors (as for the built-in fused
+ *   kernels above); entries of the active fields are ignored.  passive_add = 0 stores the passive outputs, != 0 adds to them.  d_evec as for the
  *   built-in fused kernels (NULL: FP64 atomics; else E-vector [e][node][comp] for b200_transpose_gather_add).  The
  *   context is copied from the host pointer at every call (at most B200_JIT_MAX_CTX bytes). */
 int b200_jit_fused_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,

@@ -180,7 +180,8 @@ CEED_EXTERN int CeedOperatorDestroy(CeedOperator *op);
 
 /* ---- /gpu/b200 extensions (not part of upstream; used by the harness and the tests) -- */
 /* 1 if the operator's Apply runs as ONE fused kernel (gather..scatter), 0 if generic */
-/* ApplyAdd on the element range [start, stop) of a fused operator (halo-exchange overlap in partitioned runs) */
+/* ApplyAdd on the element range [start, stop) of a fused operator (halo-exchange overlap in partitioned runs); start,
+ * and stop unless it is the element count, must be multiples of the backend's element-group size (16 always is) */
 CEED_EXTERN int CeedOperatorApplyAddRangeB200(CeedOperator op, CeedVector in, CeedVector out, CeedInt start, CeedInt stop);
 /* the partitioned MatMult of ApplyLocalCeedOp (matops.c:26-60) in one call: interface elements, halo exchange
  * (b200_halo handle, include/b200_kernels.h; NULL = none) overlapped with the interior elements, Dirichlet rows zeroed */

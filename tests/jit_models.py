@@ -49,3 +49,44 @@ CEED_QFUNCTION(ExtraF)(void *ctx, const CeedInt Q, const CeedScalar *const *in, 
 }
 """
 EXTRA_IN, EXTRA_OUT = [1, 9, 10], [3, 9, 1]
+
+
+# The field-count and width limits of K11 / K12: B200_JIT_MAXF = 8 fields each way, passive widths 1 to
+# B200_JIT_MAX_FIELD = 64.  The active gradient g is the LAST input (7) and a MIDDLE output (3).  The context is 256
+# doubles k (B200_JIT_MAX_CTX = 2048 bytes); k[255], its last 8 bytes, enters every output.  With x the passive input
+# components numbered through the fields in order (92 of them), passive output component m (numbered the same way,
+# 93 of them) is
+#     k[m] x[7m mod 92] + x[(13m + 5) mod 92] (1 + g[m mod 9] / 4) + (m + 1) k[255]
+# (7m mod 92 reaches every x), and active output component j is
+#     sum_d k[100 + 9j + d] g[d] + x[(11j + 3) mod 92] g[(j + 4) mod 9] + k[255] x[40 + j],
+# so a swapped field, component, point or element changes the answer.  Fields are [comp][Q], indexed with Q itself:
+# the same text runs with Q = 1 on the device and Q = nq on the host.
+EDGE_FIELDS = r"""#include <ceed.h>
+
+CEED_QFUNCTION(EdgeF)(void *ctx, const CeedInt Q, const CeedScalar *const *in, CeedScalar *const *out) {
+  const CeedScalar *k = (const CeedScalar *)ctx;
+  const int win[7] = {1, 2, 7, 64, 3, 5, 10}, wout[8] = {2, 64, 1, 9, 7, 3, 5, 11};
+  for (CeedInt i = 0; i < Q; i++) {
+    CeedScalar x[92], g[9];
+    int n = 0;
+    for (int f = 0; f < 7; f++)
+      for (int c = 0; c < win[f]; c++) x[n++] = in[f][c * Q + i];
+    for (int d = 0; d < 9; d++) g[d] = in[7][d * Q + i];
+    int m = 0;
+    for (int f = 0; f < 8; f++) {
+      if (f == 3) {
+        for (int j = 0; j < 9; j++) {
+          CeedScalar s = x[(11 * j + 3) % 92] * g[(j + 4) % 9] + k[255] * x[40 + j];
+          for (int d = 0; d < 9; d++) s += k[100 + 9 * j + d] * g[d];
+          out[3][j * Q + i] = s;
+        }
+        continue;
+      }
+      for (int c = 0; c < wout[f]; c++, m++)
+        out[f][c * Q + i] = k[m] * x[(7 * m) % 92] + x[(13 * m + 5) % 92] * (1 + 0.25 * g[m % 9]) + (m + 1) * k[255];
+    }
+  }
+  return 0;
+}
+"""
+EDGE_IN, EDGE_OUT, EDGE_AI, EDGE_AO, EDGE_CTX = [1, 2, 7, 64, 3, 5, 10, 9], [2, 64, 1, 9, 7, 3, 5, 11], 7, 3, 256

@@ -83,15 +83,16 @@ class PointCtx(C.Structure):
     _fields_ = [("a", C.c_double), ("b", C.c_double), ("c", C.c_double), ("k", C.c_int)]
 
 
-def _host_point_model(tmp_path, ctx, nelem, nq, ins, out_sizes):
-    """the same header built with gcc against oracle/ref_shim.h (CEED_Q_VLA = Q), run element by element"""
+def _host_point_model(tmp_path, ctx, nelem, nq, ins, out_sizes, header="point.h", name="PointModel"):
+    """the same header (tmp_path / header) built with gcc against oracle/ref_shim.h (CEED_Q_VLA = Q), QFunction
+    `name` run element by element"""
     shim = tmp_path / "shim"
-    shim.mkdir()
+    shim.mkdir(exist_ok=True)
     (shim / "ceed.h").write_text('#include "ref_shim.h"\n')
-    drv = tmp_path / "drv.c"
-    drv.write_text('#include "point.h"\n'
-                   "int run(void *ctx, int Q, const double *const *in, double *const *out) { return PointModel(ctx, Q, in, out); }\n")
-    so = tmp_path / "libpoint.so"
+    drv = tmp_path / f"drv_{name}.c"
+    drv.write_text(f'#include "{header}"\n'
+                   f"int run(void *ctx, int Q, const double *const *in, double *const *out) {{ return {name}(ctx, Q, in, out); }}\n")
+    so = tmp_path / f"lib{name}.so"
     subprocess.run(["/usr/bin/gcc", "-std=gnu99", "-O2", "-fPIC", "-shared", "-ffp-contract=off", f"-I{shim}",
                     f"-I{os.path.join(ROOT, 'oracle')}", f"-I{tmp_path}", str(drv), "-o", str(so), "-lm"], check=True)
     lib = C.CDLL(str(so))
