@@ -174,6 +174,8 @@ _proto("b200_jit_free_source", _vp, restype=None)
 _proto("b200_jit_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, C.POINTER(_i))
 _proto("b200_jit_program", _i, restype=C.c_char_p)
 _proto("b200_jit_fused_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, _i, _i, _i, _i, C.POINTER(_i))
+_proto("b200_jit_assemble_compile", _vp, C.c_char_p, C.c_char_p, _i, _vp, _i, _vp, _i, _i, _i, _i, C.POINTER(_i))
+_proto("b200_jit_assemble_apply", _i, _vp, _sz, _i, _vp, _vp, _i, _vp, _vp)
 _proto("b200_jit_compile_count", restype=C.c_ulonglong)
 
 # sentinels are exported data symbols holding pointers
@@ -544,6 +546,24 @@ def jit_fused_compile(path, name, in_sizes, out_sizes, active_in, active_out, P,
         rc = lib.b200_jit_fused_compile(text, str(path).encode(), name.encode(), len(in_sizes),
                                         (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
                                         int(active_in), int(active_out), int(P), int(Q), C.byref(h))
+    finally:
+        lib.b200_jit_free_source(text)
+    b2(rc)
+    return h.value
+
+
+def jit_assemble_compile(path, name, in_sizes, out_sizes, active_in, active_out, P, Q):
+    """The compile half of K13 without a device: the element-matrix kernel of a trilinear level (P = 2) around
+    QFunction `name` of `path`, fields as for jit_fused_compile.  Returns the handle (cached per process, as
+    jit_compile)."""
+    text, err = C.c_void_p(), C.create_string_buffer(1024)
+    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
+        raise CeedError(err.value.decode())
+    h = C.c_int(-1)
+    try:
+        rc = lib.b200_jit_assemble_compile(text, str(path).encode(), name.encode(), len(in_sizes),
+                                           (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
+                                           int(active_in), int(active_out), int(P), int(Q), C.byref(h))
     finally:
         lib.b200_jit_free_source(text)
     b2(rc)

@@ -16,6 +16,10 @@
 // and the passive q-blocked vectors.  The template is embedded at build time (b200_jit_fused.inc, a raw string made
 // from the header by the Makefile); the lattice constants come from b200_apply_smem_layout, so the built-in and the
 // generated kernels cannot disagree on the layout.
+//
+// K13 (b200_jit_assemble_compile / b200_jit_assemble_apply): the same user program with b200_jit_assemble.cuh around
+// it, the element matrices of a trilinear (P = 2) level in the CeedOperatorLinearAssemble layout, from the point
+// tangents the user function gives for the 9 unit active inputs.  Embedded the same way (b200_jit_assemble.inc).
 #include <dlfcn.h>
 #include <nvrtc.h>
 #include <stdlib.h>
@@ -72,6 +76,19 @@ const char *const kFusedTemplate =
 // spills.  B200_JIT_FUSED_CTAS overrides it (tuning runs).
 const int kFusedCtas = 3;
 
+// the K13 template (b200_jit_assemble.cuh) as a string
+const char *const kAssembleTemplate =
+#include "b200_jit_assemble.inc"
+    ;
+
+// K13 blocks per SM asked of ptxas for the full-group kernel, and whether the 9 unit-input calls of the user function
+// are unrolled (NVCC may then share their input-independent part) or kept rolled.  Chosen by measurement at Q = 5,
+// C3 (profiles/jit_assemble_ab.txt); B200_JIT_ASSEMBLE_CTAS and B200_JIT_ASSEMBLE_UNROLL override them (tuning runs).
+const int kAssembleCtas = 2;
+const int kAssembleUnroll = 0;
+// most point tangents a K13 CTA holds in shared memory at once (81 doubles each)
+const int kAssembleMaxChunk = 128;
+
 struct Entry {
   std::string key;     // options + program text
   std::string kernel;  // b200_jit_<Name>, or b200_jit_fused_<Name> (K12: full element groups)
@@ -86,6 +103,8 @@ struct Entry {
   std::string kernel_tail;  // b200_jit_fused_tail_<Name>: the partial group at the end of a range
   cudaKernel_t fn_tail = nullptr;
   unsigned long long smem_set = 0;  // devices on which the dynamic shared-memory limit was raised
+  // K13 only (P, Q, ai, ao, smem, kernel_tail and fn_tail as for K12; lay[4] = EB, lay[5] = threads)
+  bool assemble = false;
 };
 
 std::mutex g_mu;
@@ -307,6 +326,54 @@ std::string generated_fused(const char *name, int nin, const int *in_size, int n
   return k;
 }
 
+// K13: the prefix b200_jit_assemble.cuh expects (constants, parameter structs, the point-tangent adapter), the template,
+// the kernels
+std::string generated_assemble(const char *name, int nin, const int *in_size, int nout, const int *out_size, int ai,
+                               int ao, int Q, int EB, int NT, int CH, int ctas, int unroll) {
+  std::string k;
+  char line[512];
+  auto add = [&](const char *fmt, auto... a) {
+    snprintf(line, sizeof line, fmt, a...);
+    k += line;
+  };
+  k += "\n#line 1 \"b200_jit_assemble_prefix\"\n";
+  add("#define B200_K13_Q %d\n#define B200_K13_EB %d\n#define B200_K13_NT %d\n#define B200_K13_CH %d\n", Q, EB, NT, CH);
+  add("struct alignas(16) b200_jit_ctx_t { unsigned char b[%d]; };\n", B200_JIT_MAX_CTX);
+  add("struct b200_k13_fields_t { const double *in[%d]; };\n", B200_JIT_MAXF);
+  k += "__device__ __forceinline__ void b200_k13_point(const b200_jit_ctx_t &ctx, const b200_k13_fields_t &f,\n"
+       "    const size_t grp, const size_t pos, const size_t cs, double *__restrict__ d) {\n";
+  for (int i = 0; i < nin; i++) {
+    add("  double in%d[%d];\n", i, in_size[i]);
+    if (i != ai)
+      add("  { const double *p = f.in[%d] + grp * %d + pos;\n#pragma unroll\n"
+          "    for (int c = 0; c < %d; c++) in%d[c] = __ldcs(p + c * cs); }\n", i, in_size[i], in_size[i], i);
+  }
+  k += unroll ? "#pragma unroll\n" : "#pragma unroll 1\n";
+  k += "  for (int s = 0; s < 9; s++) {\n";
+  add("#pragma unroll\n    for (int c = 0; c < 9; c++) in%d[c] = c == s ? 1.0 : 0.0;\n", ai);
+  for (int i = 0; i < nout; i++) add("    double out%d[%d] = {};\n", i, out_size[i]);
+  k += "    const double *ins[] = {";
+  for (int i = 0; i < nin; i++) add("%sin%d", i ? ", " : "", i);
+  k += "};\n    double *outs[] = {";
+  for (int i = 0; i < nout; i++) add("%sout%d", i ? ", " : "", i);
+  k += "};\n";
+  add("    (void)%s((void *)ctx.b, 1, ins, outs);\n", name);
+  add("#pragma unroll\n    for (int o = 0; o < 9; o++) d[s * 9 + o] = out%d[o];\n", ao);
+  k += "  }\n}\n#line 1 \"b200_jit_assemble.cuh\"\n";
+  k += kAssembleTemplate;
+  k += "\n#line 1 \"b200_jit_assemble_kernels\"\n";
+  // 384 threads (Q <= 3, EB = 16) leave at most 168 registers a thread whatever is asked: one block per SM, and the
+  // tail kernel runs as one CTA
+  const char *variant[2] = {"", "tail_"};
+  for (int v = 0; v < 2; v++)
+    add("extern \"C\" __global__ void __launch_bounds__(%d, %d) b200_jit_assemble_%s%s(\n"
+        "    const __grid_constant__ b200_k13_mats_t m, const __grid_constant__ b200_jit_ctx_t ctx,\n"
+        "    const __grid_constant__ b200_k13_fields_t f, const int nelem, double *__restrict__ values) {\n"
+        "  b200_k13_body<%s>(m, ctx, f, nelem, values);\n}\n",
+        NT, v || NT > 128 ? 1 : ctas, variant[v], name, v ? "false" : "true");
+  return k;
+}
+
 }  // namespace
 
 extern "C" int b200_jit_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
@@ -378,7 +445,8 @@ extern "C" int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, i
     std::lock_guard<std::mutex> lock(g_mu);
     if (handle < 0 || handle >= (int)g_entries.size()) return b200::set_error_msg("b200_jit_apply: bad handle");
     en = g_entries[handle];
-    if (en->fused) return b200::set_error_msg("b200_jit_apply: the handle names a fused operator program (b200_jit_fused_apply)");
+    if (en->fused || en->assemble)
+      return b200::set_error_msg("b200_jit_apply: the handle names a fused operator or assembly program");
     if (!en->lib) {
       B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
       B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
@@ -477,6 +545,114 @@ extern "C" int b200_jit_fused_apply(int handle, const void *h_ctx, size_t ctx_by
     void *args[] = {mats, &ctx, &ft, &n, &off, &d_x, &d_y, &ev, &passive_add};
     B200_CHECK(cudaLaunchKernel((const void *)en->fn_tail, dim3(1), dim3(NT), args, en->smem, b200::g_stream));
     B200_LAUNCH_CHECK("b200_jit_fused_apply(tail)");
+  }
+  return 0;
+}
+
+extern "C" int b200_jit_assemble_compile(const char *text, const char *src_name, const char *name, int nin,
+                                         const int *in_sizes, int nout, const int *out_sizes, int active_in,
+                                         int active_out, int P, int Q, int *handle) {
+  *handle = -1;
+  if (!text || !name) return b200::set_error_msg("b200_jit_assemble_compile: NULL program text or name");
+  if (int rc = check_fields("b200_jit_assemble_compile", name, nin, in_sizes, nout, out_sizes)) return rc;
+  if (active_in < 0 || active_in >= nin || active_out < 0 || active_out >= nout || in_sizes[active_in] != 9 ||
+      out_sizes[active_out] != 9)
+    return b200::set_error_msg("b200_jit_assemble_compile: the active input and output must be fields of 9 components");
+  char msg[160];
+  if (P != 2) {
+    snprintf(msg, sizeof msg, "b200_jit_assemble_compile: element matrices are assembled on trilinear (P = 2) levels "
+             "only, not P = %d", P);
+    return b200::set_error_msg(msg);
+  }
+  if (!b200_fused_supported(P, Q)) {
+    snprintf(msg, sizeof msg, "b200_jit_assemble_compile: (P, Q) = (%d, %d) is not instantiated", P, Q);
+    return b200::set_error_msg(msg);
+  }
+  const char *env = getenv("B200_JIT_ASSEMBLE_CTAS");  // read at every compile: part of the program text and its key
+  const int ctas = env && atoi(env) > 0 ? atoi(env) : kAssembleCtas;
+  env = getenv("B200_JIT_ASSEMBLE_UNROLL");
+  const int unroll = env && env[0] ? atoi(env) != 0 : kAssembleUnroll;
+  const int EB = b200::elems_per_block(Q), NT = 24 * EB, CH = NT < kAssembleMaxChunk ? NT : kAssembleMaxChunk;
+  Entry *en = new Entry;
+  en->key = options_line() + text +
+            generated_assemble(name, nin, in_sizes, nout, out_sizes, active_in, active_out, Q, EB, NT, CH, ctas, unroll);
+  en->kernel = std::string("b200_jit_assemble_") + name;
+  en->kernel_tail = std::string("b200_jit_assemble_tail_") + name;
+  en->nin = nin;
+  en->nout = nout;
+  for (int i = 0; i < nin; i++) en->in_size[i] = in_sizes[i];
+  for (int i = 0; i < nout; i++) en->out_size[i] = out_sizes[i];
+  en->assemble = true;
+  en->P = P;
+  en->Q = Q;
+  en->ai = active_in;
+  en->ao = active_out;
+  en->lay[4] = EB;
+  en->lay[5] = NT;
+  en->smem = sizeof(double) * 81 * (size_t)CH;
+  return find_or_compile(en, src_name, handle);
+}
+
+extern "C" int b200_jit_assemble_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem,
+                                       const double *h_interp1d, const double *h_grad1d, int nin,
+                                       const double *const *d_in, double *d_values) {
+  Entry *en;
+  int dev;
+  B200_CHECK(cudaGetDevice(&dev));
+  {
+    std::lock_guard<std::mutex> lock(g_mu);
+    if (handle < 0 || handle >= (int)g_entries.size() || !g_entries[handle]->assemble)
+      return b200::set_error_msg("b200_jit_assemble_apply: bad handle");
+    en = g_entries[handle];
+    if (!en->lib) {
+      B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn_tail, en->lib, en->kernel_tail.c_str()));
+    }
+    // the point tangents of a chunk take 62 to 83 KB: the limit is raised once per device
+    if (en->smem > 48 * 1024 && dev >= 0 && dev < 64 && !(en->smem_set >> dev & 1)) {
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      en->smem_set |= 1ull << dev;
+    }
+  }
+  if (nin != en->nin) return b200::set_error_msg("b200_jit_assemble_apply: field count differs from the compiled one");
+  if (ctx_bytes > B200_JIT_MAX_CTX) {
+    char msg[160];
+    snprintf(msg, sizeof msg, "b200_jit_assemble_apply: context of %zu bytes; a JIT QFunction takes at most %d",
+             ctx_bytes, B200_JIT_MAX_CTX);
+    return b200::set_error_msg(msg);
+  }
+  if (ctx_bytes && !h_ctx) return b200::set_error_msg("b200_jit_assemble_apply: NULL context");
+  if (nelem <= 0) return 0;
+  const int Q = en->Q, Q3 = Q * Q * Q, EB = en->lay[4], NT = en->lay[5];
+  double mats[2 * 8 * 2];  // b200_k13_mats_t for this Q: interp1d [Q][2], then grad1d [Q][2]
+  for (int i = 0; i < Q * 2; i++) {
+    mats[i] = h_interp1d[i];
+    mats[Q * 2 + i] = h_grad1d[i];
+  }
+  JitCtx ctx;
+  memset(&ctx, 0, sizeof ctx);
+  if (ctx_bytes) memcpy(ctx.b, h_ctx, ctx_bytes);
+  const double *fin[B200_JIT_MAXF] = {};
+  for (int i = 0; i < nin; i++) fin[i] = i == en->ai ? nullptr : d_in[i];
+  const int nfull = nelem / EB, ntail = nelem - nfull * EB;
+  if (nfull) {
+    int n = nfull * EB;
+    void *args[] = {mats, &ctx, fin, &n, &d_values};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn, dim3(nfull), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_assemble_apply");
+  }
+  if (ntail) {  // the partial group at the end: a run-time group extent, one CTA
+    const size_t e0 = (size_t)nfull * EB;
+    const double *ft[B200_JIT_MAXF] = {};
+    for (int i = 0; i < nin; i++)
+      if (fin[i]) ft[i] = fin[i] + e0 * en->in_size[i] * Q3;
+    double *v = d_values + e0 * 576;
+    int n = ntail;
+    void *args[] = {mats, &ctx, ft, &n, &v};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn_tail, dim3(1), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_assemble_apply(tail)");
   }
   return 0;
 }

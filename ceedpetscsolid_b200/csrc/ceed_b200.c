@@ -130,8 +130,9 @@ struct CeedOperator_private {
   /* fused transfer operators: optional fine-side pointwise scaling (CeedOperatorSetTransferScalingB200) */
   CeedVector xfer_scale;
   int xfer_inject;
-  /* OP_JIT_FUSED: the active input / output fields; jit_fused = K12 program handle + 1 (0: not compiled yet) */
-  int jit_ai, jit_ao, jit_fused;
+  /* OP_JIT_FUSED: the active input / output fields; jit_fused = K12 program handle + 1 (0: not compiled yet);
+     jit_assemble = K13 program handle + 1 (compiled at the first CeedOperatorLinearAssemble) */
+  int jit_ai, jit_ao, jit_fused, jit_assemble;
   /* generic-path work buffers (device), grown on demand */
   double *ebuf[2 * MAXF], *qbuf[2 * MAXF];
   size_t ebytes[2 * MAXF], qbytes[2 * MAXF];
@@ -1065,6 +1066,7 @@ static int op_setup(CeedOperator op) {
     if (qf->qf_id == B200_QF_NONE || differs) CeedChk(qf_jit_compile(qf, differs));
   }
   op->jit_fused = 0;
+  op->jit_assemble = 0;
   if (qf->jit_handle >= 0) {
     op->kind = qf->jit_text && jit_fused_eligible(op) ? OP_JIT_FUSED : OP_GENERIC;
     return 0;
@@ -1755,23 +1757,35 @@ int CeedOperatorLinearAssembleDiagonal(CeedOperator op, CeedVector assembled, Ce
   return CeedOperatorLinearAssembleAddDiagonal(op, assembled, request);
 }
 
-/* COO assembly: entry (e, col, row) of element e sits at (e*24 + col)*24 + row, element dof = node*3 + comp */
+/* COO assembly: entry (e, col, row) of element e sits at (e*24 + col)*24 + row, element dof = node*3 + comp.
+ * Built-in fused Jacobians: K8 from the Jacobian cache.  JIT operators on K12 (OP_JIT_FUSED): K13 around the user
+ * function, which must be linear in its active input (every Jacobian QFunction is). */
 static int op_assemblable(CeedOperator op) {
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorLinearAssemble: composite operators are not supported by /gpu/b200");
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (!(op->kind == OP_FUSED_JACOBIAN || (op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS)) ||
-      op->in[0].b->P != 2)
+  if (op->kind == OP_GENERIC && op->qf->jit_handle >= 0) {
+    CeedBasis b = NULL;
+    for (int i = 0; i < op->qf->nin && !b; i++)
+      if (op->in[i].v == CEED_VECTOR_ACTIVE && op->in[i].b != CEED_BASIS_COLLOCATED) b = op->in[i].b;
+    return CeedError(ceed, 1, "CeedOperatorLinearAssemble: JIT QFunction %s runs on the generic path: its fields are "
+                              "not of the fused shape or its basis (P, Q) = (%d, %d) has no fused kernel, and /gpu/b200 "
+                              "assembles only operators of the fused kernels; there is no CPU fallback",
+                     op->qf->name, b ? b->P : 0, b ? b->Q : 0);
+  }
+  CeedBasis b = op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0].b;
+  if (!(op->kind == OP_FUSED_JACOBIAN || op->kind == OP_JIT_FUSED ||
+        (op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS)) || b->P != 2)
     return CeedError(ceed, 1, "CeedOperatorLinearAssemble: /gpu/b200 assembles fused Jacobian operators on a trilinear "
                               "(P = 2) level only (operator %s, P = %d); there is no CPU fallback",
-                     op->qf->name, op->in[0].b ? op->in[0].b->P : 0);
+                     op->qf->name, b ? b->P : 0);
   return 0;
 }
 
 int CeedOperatorLinearAssembleSymbolic(CeedOperator op, CeedInt *num_entries, CeedInt **rows, CeedInt **cols) {
   Ceed ceed = op->ceed;
   CeedChk(op_assemblable(op));
-  CeedElemRestriction r = op->in[0].r;
+  CeedElemRestriction r = op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0].r;
   const size_t nelem = (size_t)r->nelem, ne = nelem * 576;
   if (ne > 2147483647u) return CeedError(ceed, 1, "CeedOperatorLinearAssembleSymbolic: %zu entries overflow CeedInt", ne);
   int *off = (int *)malloc(sizeof(int) * (nelem * 8 + 1));
@@ -1790,17 +1804,47 @@ int CeedOperatorLinearAssembleSymbolic(CeedOperator op, CeedInt *num_entries, Ce
   return 0;
 }
 
+/* K13: compile the assembly program at the first CeedOperatorLinearAssemble, then assemble; the operator's vectors
+ * are only read (passive outputs are never written) */
+static int op_assemble_jit(CeedOperator op, double *v) {
+  Ceed ceed = op->ceed;
+  CeedQFunction qf = op->qf;
+  OpField *u = &op->in[op->jit_ai];
+  if (!op->jit_assemble) {
+    int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
+    for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
+    for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
+    if (b200_jit_assemble_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes,
+                                  op->jit_ai, op->jit_ao, u->b->P, u->b->Q, &hh))
+      return CeedError(ceed, 1, "%s: assembly kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
+                       qf->jit_path, b200_last_error());
+    op->jit_assemble = hh + 1;
+  }
+  size_t bytes;
+  CeedChk(jit_ctx_bytes(qf, &bytes));
+  const double *din[MAXF] = {NULL};
+  for (int i = 0; i < qf->nin; i++)
+    if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &din[i]));
+  B2(ceed, b200_jit_assemble_apply(op->jit_assemble - 1, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
+                                   qf->nin, din, v));
+  return 0;
+}
+
 int CeedOperatorLinearAssemble(CeedOperator op, CeedVector values) {
   Ceed ceed = op->ceed;
   CeedChk(op_assemblable(op));
-  OpField *u = &op->in[0];
+  OpField *u = &op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0];
   if ((size_t)values->length < (size_t)u->r->nelem * 576)
     return CeedError(ceed, 1, "CeedOperatorLinearAssemble: values vector holds %d entries, %zu needed", values->length,
                      (size_t)u->r->nelem * 576);
+  double *v;
+  if (op->kind == OP_JIT_FUSED) {
+    CeedChk(vec_dev_write(values, &v));
+    return op_assemble_jit(op, v);
+  }
   b200_physics phys;
   CeedChk(qf_physics(op->qf, &phys));
   const double *jc;
-  double *v;
   CeedChk(jcache_get(op, &jc));
   CeedChk(vec_dev_write(values, &v));
   B2(ceed, b200_assemble_p1(op->problem, &phys, u->r->nelem, u->b->Q, u->b->interp1d, u->b->grad1d, jc, v));

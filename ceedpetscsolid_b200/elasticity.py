@@ -170,8 +170,10 @@ class Elasticity:
         {"apply": "<file>:<Name>", "jacob": "<file>:<Name>"} replaces the residual / Jacobian QFunctions of app.problem
         (same fields) by user QFunctions, compiled at set-up on the "/gpu/b200:jit" resource.  Their operators run on
         K12, the fused kernel generated around the user function (compiled at the first apply), and their diagonal on
-        the generic path.  The p = 1 level has no built-in Jacobian, so box meshes assemble it by colouring,
-        unstructured meshes by column probing, and coarse="amg" is refused.  Strain energy and diagnostics keep the problem's stock model."""
+        the generic path.  The p = 1 level has no built-in Jacobian: on unstructured meshes, and with coarse="amg" on
+        any mesh, its element matrices come from K13, CeedOperatorLinearAssemble around the user function (which must
+        be linear in its active input, as every Jacobian QFunction is); box meshes with "hmg" or "pcg" assemble it by
+        colouring.  Strain energy and diagnostics keep the problem's stock model."""
         if coarse == "amg" and world > 1:
             # checked before any device work: the redundant AMG gathers every rank's element matrices and right-hand
             # side through the process group, and exists only for the masked layout
@@ -215,7 +217,10 @@ class Elasticity:
                                         phys=self.phys, memType=fu.memType, bc_values=self._bc_values_fn(self.dms[fine], app))
         self.levels = [GpuLevel(self.dms[l], self.users[l], self.res_user if l == fine else None)
                        for l in range(len(self.degrees))]
-        if assemble == "coo" and self.degrees[0] == 1 and self.users[0].op.is_fused:
+        op0 = self.users[0].op
+        unstructured = not getattr(self.gmesh, "structured", True)
+        if assemble == "coo" and self.degrees[0] == 1 and (
+                op0.is_fused or (op0.is_jit_fused and (unstructured or coarse == "amg"))):
             self.levels[0].enable_coo(self.ceed, self.mesh)
         self.transfers = [None]
         for l in range(1, len(self.degrees)):
@@ -250,7 +255,8 @@ class Elasticity:
         amg_solver = None
         if coarse == "amg":
             if self.levels[0].coo is None:
-                raise ValueError("coarse='amg' needs the element matrices of the p = 1 level (assemble='coo', fused operator)")
+                raise ValueError("coarse='amg' needs the element matrices of the p = 1 level (assemble='coo', and a "
+                                 "built-in fused or K12 operator there)")
             from .amg import MAX_COARSE_DOFS, RedundantAMG, SmoothedAggregationAMG
             mc = MAX_COARSE_DOFS if amg_max_coarse is None else amg_max_coarse
             if world > 1:

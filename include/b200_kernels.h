@@ -358,6 +358,24 @@ int b200_jit_fused_apply(int handle, const void *h_ctx, size_t ctx_bytes, int ne
                          const double *h_grad1d, const int *d_offsets, const double *d_x, double *d_y, double *d_evec,
                          int nin, const double *const *d_in, int nout, double *const *d_out, int passive_add);
 
+/* ---- K13: element matrices of a trilinear level around a JIT-compiled user QFunction (csrc/b200_jit_assemble.cuh) --
+ * b200_jit_assemble_compile (no device needed): text + the kernel of b200_jit_assemble.cuh around QFunction `name`
+ *   for the basis (P, Q) = (2, Q), Q one of B200_FOR_PQ; fields as for b200_jit_fused_compile.  Any other P, or an
+ *   active field that is not 9 wide, is refused.  Compiled unless the same program (text, name, sizes, active fields,
+ *   Q) was compiled before; counted by b200_jit_compile_count and shown by b200_jit_program.
+ * b200_jit_assemble_apply: the CeedOperatorLinearAssemble values of nelem elements, layout of b200_assemble_p1:
+ *   d_values[(e*24 + col)*24 + row] = sum_q G_row(q)^T D_q G_col(q), D_q the point tangent of the user function,
+ *   dout_active / din_active, from its 9 calls with the unit active inputs at point q (passive inputs as given, passive
+ *   outputs discarded; the return code is ignored).  This is the Jacobian only if the function is linear in its
+ *   active input.  One launch for the full element groups and one for a partial last group, on the backend stream;
+ *   no atomics (bit-identical from run to run).  d_in of the passive inputs: q-blocked vectors of nelem elements;
+ *   entries of the active field are ignored.  The context is copied from the host pointer at every call (at most
+ *   B200_JIT_MAX_CTX bytes). */
+int b200_jit_assemble_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
+                              int nout, const int *out_sizes, int active_in, int active_out, int P, int Q, int *handle);
+int b200_jit_assemble_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
+                            const double *h_grad1d, int nin, const double *const *d_in, double *d_values);
+
 #ifdef __cplusplus
 }
 #endif
