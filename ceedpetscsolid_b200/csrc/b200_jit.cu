@@ -20,6 +20,11 @@
 // K13 (b200_jit_assemble_compile / b200_jit_assemble_apply): the same user program with b200_jit_assemble.cuh around
 // it, the element matrices of a trilinear (P = 2) level in the CeedOperatorLinearAssemble layout, from the point
 // tangents the user function gives for the 9 unit active inputs.  Embedded the same way (b200_jit_assemble.inc).
+//
+// K14 (b200_jit_diag_compile / b200_jit_diag_apply): the same user program with b200_jit_diag.cuh around it, the
+// operator diagonal (CeedOperatorLinearAssembleDiagonal) at one (P, Q) of B200_FOR_PQ, from 3 unit-input calls of the
+// user function per point and component, contracted as the built-in diagonal (K3) does.  The lattice constants come
+// from b200_apply_smem_layout, as for K12.  Embedded the same way (b200_jit_diag.inc).
 #include <dlfcn.h>
 #include <nvrtc.h>
 #include <stdlib.h>
@@ -89,6 +94,17 @@ const int kAssembleUnroll = 0;
 // most point tangents a K13 CTA holds in shared memory at once (81 doubles each)
 const int kAssembleMaxChunk = 128;
 
+// the K14 template (b200_jit_diag.cuh) as a string
+const char *const kDiagTemplate =
+#include "b200_jit_diag.inc"
+    ;
+
+// K14 blocks of 128 threads per SM asked of ptxas for the full-group kernel.  Measured on the three levels of C3
+// (profiles/jit_diag_ab.txt): the fastest setting at which port_HyperFSdF neither spills nor has a stack frame
+// (162 registers at P = Q = 5); 4 blocks (128 registers) ran 6 to 7 % faster with 88 bytes of spills.
+// B200_JIT_DIAG_CTAS overrides it (tuning runs).
+const int kDiagCtas = 2;
+
 struct Entry {
   std::string key;     // options + program text
   std::string kernel;  // b200_jit_<Name>, or b200_jit_fused_<Name> (K12: full element groups)
@@ -105,6 +121,8 @@ struct Entry {
   unsigned long long smem_set = 0;  // devices on which the dynamic shared-memory limit was raised
   // K13 only (P, Q, ai, ao, smem, kernel_tail and fn_tail as for K12; lay[4] = EB, lay[5] = threads)
   bool assemble = false;
+  // K14 only (P, Q, ai, ao, lay, smem, kernel_tail and fn_tail as for K12)
+  bool diag = false;
 };
 
 std::mutex g_mu;
@@ -374,6 +392,70 @@ std::string generated_assemble(const char *name, int nin, const int *in_size, in
   return k;
 }
 
+// K14: the prefix b200_jit_diag.cuh expects (constants, parameter structs, the slab prefetch, the adapter that gives
+// one component's point tangent from 3 unit-input calls), the template, the kernels
+std::string generated_diag(const char *name, int nin, const int *in_size, int nout, const int *out_size, int ai, int ao,
+                           int P, int Q, const int *lay, int ctas) {
+  std::string k;
+  char line[512];
+  auto add = [&](const char *fmt, auto... a) {
+    snprintf(line, sizeof line, fmt, a...);
+    k += line;
+  };
+  k += "\n#line 1 \"b200_jit_diag_prefix\"\n";
+  add("#define B200_K14_P %d\n#define B200_K14_Q %d\n", P, Q);
+  add("#define B200_K14_SY %d\n#define B200_K14_SZ %d\n#define B200_K14_SC %d\n#define B200_K14_SE %d\n"
+      "#define B200_K14_EB %d\n#define B200_K14_NT %d\n", lay[0], lay[1], lay[2], lay[3], lay[4], lay[5]);
+  add("struct alignas(16) b200_jit_ctx_t { unsigned char b[%d]; };\n", B200_JIT_MAX_CTX);
+  add("struct b200_k14_fields_t { const double *in[%d]; };\n", B200_JIT_MAXF);
+  // the bulk prefetch wants a 16-byte aligned range: the slab's 16-byte granules that lie inside it
+  k += "__device__ __forceinline__ void b200_k14_l2(const double *p, const size_t n) {\n"
+       "  const unsigned long long a0 = ((unsigned long long)p + 15) & ~15ull, a1 = (unsigned long long)(p + n) & ~15ull;\n"
+       "  if (a1 > a0) asm volatile(\"cp.async.bulk.prefetch.L2.global [%0], %1;\" ::\"l\"(a0), \"r\"((unsigned)(a1 - a0)) : \"memory\");\n"
+       "}\n";
+  k += "__device__ __forceinline__ void b200_k14_prefetch(const b200_k14_fields_t &f, const size_t grp, const size_t npts) {\n";
+  for (int i = 0; i < nin; i++)
+    if (i != ai) add("  b200_k14_l2(f.in[%d] + grp * %d, npts * %d);\n", i, in_size[i], in_size[i]);
+  k += "}\n";
+  k += "template <class Fold>\n"
+       "__device__ __forceinline__ void b200_k14_point(const b200_jit_ctx_t &ctx, const b200_k14_fields_t &f,\n"
+       "    const size_t grp, const size_t pos, const size_t cs, const int comp, Fold &&fold) {\n";
+  k += "#pragma unroll 1\n  for (int m = 0; m < 3; m++) {\n";
+  for (int i = 0; i < nin; i++) {
+    add("    double in%d[%d];\n", i, in_size[i]);
+    if (i != ai)
+      add("    { const double *p = f.in[%d] + grp * %d + pos;\n#pragma unroll\n"
+          "      for (int c = 0; c < %d; c++) in%d[c] = __ldg(p + c * cs); }\n", i, in_size[i], in_size[i], i);
+  }
+  add("#pragma unroll\n    for (int c = 0; c < 9; c++) in%d[c] = c == m * 3 + comp ? 1.0 : 0.0;\n", ai);
+  for (int i = 0; i < nout; i++) add("    double out%d[%d] = {};\n", i, out_size[i]);
+  k += "    const double *ins[] = {";
+  for (int i = 0; i < nin; i++) add("%sin%d", i ? ", " : "", i);
+  k += "};\n    double *outs[] = {";
+  for (int i = 0; i < nout; i++) add("%sout%d", i ? ", " : "", i);
+  k += "};\n";
+  add("    (void)%s((void *)ctx.b, 1, ins, outs);\n", name);
+  // selects, not run-time indices: the outputs stay in registers
+  add("    double v[3];\n#pragma unroll\n    for (int kk = 0; kk < 3; kk++)\n"
+      "      v[kk] = comp == 0 ? out%d[kk * 3] : comp == 1 ? out%d[kk * 3 + 1] : out%d[kk * 3 + 2];\n"
+      "    fold(m, v);\n", ao, ao, ao);
+  k += "  }\n}\n#line 1 \"b200_jit_diag.cuh\"\n";
+  k += kDiagTemplate;
+  k += "\n#line 1 \"b200_jit_diag_kernels\"\n";
+  // ctas blocks of 128 threads' worth per SM: 160-thread CTAs (Q = 3) ask for fewer blocks, as K3 does, so that a
+  // thread keeps the registers the user function needs; the tail kernel runs as one CTA and gets every register
+  const int full = lay[5] > 128 && ctas * 128 / lay[5] >= 1 ? ctas * 128 / lay[5] : ctas;
+  const char *variant[2] = {"", "tail_"};
+  for (int v = 0; v < 2; v++)
+    add("extern \"C\" __global__ void __launch_bounds__(%d, %d) b200_jit_diag_%s%s(\n"
+        "    const __grid_constant__ b200_k14_mats_t m, const __grid_constant__ b200_jit_ctx_t ctx,\n"
+        "    const __grid_constant__ b200_k14_fields_t f, const int nelem, const int *__restrict__ offsets,\n"
+        "    double *__restrict__ diag, double *__restrict__ evec) {\n"
+        "  b200_k14_body<%s>(m, ctx, f, nelem, offsets, diag, evec);\n}\n",
+        lay[5], v ? 1 : full, variant[v], name, v ? "false" : "true");
+  return k;
+}
+
 }  // namespace
 
 extern "C" int b200_jit_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
@@ -445,8 +527,8 @@ extern "C" int b200_jit_apply(int handle, const void *h_ctx, size_t ctx_bytes, i
     std::lock_guard<std::mutex> lock(g_mu);
     if (handle < 0 || handle >= (int)g_entries.size()) return b200::set_error_msg("b200_jit_apply: bad handle");
     en = g_entries[handle];
-    if (en->fused || en->assemble)
-      return b200::set_error_msg("b200_jit_apply: the handle names a fused operator or assembly program");
+    if (en->fused || en->assemble || en->diag)
+      return b200::set_error_msg("b200_jit_apply: the handle names a fused operator, assembly or diagonal program");
     if (!en->lib) {
       B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
       B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
@@ -653,6 +735,107 @@ extern "C" int b200_jit_assemble_apply(int handle, const void *h_ctx, size_t ctx
     void *args[] = {mats, &ctx, ft, &n, &v};
     B200_CHECK(cudaLaunchKernel((const void *)en->fn_tail, dim3(1), dim3(NT), args, en->smem, b200::g_stream));
     B200_LAUNCH_CHECK("b200_jit_assemble_apply(tail)");
+  }
+  return 0;
+}
+
+extern "C" int b200_jit_diag_compile(const char *text, const char *src_name, const char *name, int nin,
+                                     const int *in_sizes, int nout, const int *out_sizes, int active_in, int active_out,
+                                     int P, int Q, int *handle) {
+  *handle = -1;
+  if (!text || !name) return b200::set_error_msg("b200_jit_diag_compile: NULL program text or name");
+  if (int rc = check_fields("b200_jit_diag_compile", name, nin, in_sizes, nout, out_sizes)) return rc;
+  if (active_in < 0 || active_in >= nin || active_out < 0 || active_out >= nout || in_sizes[active_in] != 9 ||
+      out_sizes[active_out] != 9)
+    return b200::set_error_msg("b200_jit_diag_compile: the active input and output must be fields of 9 components");
+  int lay[6];
+  if (!b200_fused_supported(P, Q) || b200_apply_smem_layout(P, Q, lay)) {
+    char msg[160];
+    snprintf(msg, sizeof msg, "b200_jit_diag_compile: (P, Q) = (%d, %d) is not instantiated", P, Q);
+    return b200::set_error_msg(msg);
+  }
+  const char *env = getenv("B200_JIT_DIAG_CTAS");  // read at every compile: part of the program text and its key
+  const int ctas = env && atoi(env) > 0 ? atoi(env) : kDiagCtas;
+  Entry *en = new Entry;
+  en->key = options_line() + text + generated_diag(name, nin, in_sizes, nout, out_sizes, active_in, active_out, P, Q, lay, ctas);
+  en->kernel = std::string("b200_jit_diag_") + name;
+  en->kernel_tail = std::string("b200_jit_diag_tail_") + name;
+  en->nin = nin;
+  en->nout = nout;
+  for (int i = 0; i < nin; i++) en->in_size[i] = in_sizes[i];
+  for (int i = 0; i < nout; i++) en->out_size[i] = out_sizes[i];
+  en->diag = true;
+  en->P = P;
+  en->Q = Q;
+  en->ai = active_in;
+  en->ao = active_out;
+  memcpy(en->lay, lay, sizeof lay);
+  en->smem = sizeof(double) * (size_t)lay[4] * lay[3];
+  return find_or_compile(en, src_name, handle);
+}
+
+extern "C" int b200_jit_diag_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
+                                   const double *h_grad1d, const int *d_offsets, int nin, const double *const *d_in,
+                                   double *d_diag, double *d_evec) {
+  Entry *en;
+  int dev;
+  B200_CHECK(cudaGetDevice(&dev));
+  {
+    std::lock_guard<std::mutex> lock(g_mu);
+    if (handle < 0 || handle >= (int)g_entries.size() || !g_entries[handle]->diag)
+      return b200::set_error_msg("b200_jit_diag_apply: bad handle");
+    en = g_entries[handle];
+    if (!en->lib) {
+      B200_CHECK(cudaLibraryLoadData(&en->lib, en->cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn, en->lib, en->kernel.c_str()));
+      B200_CHECK(cudaLibraryGetKernel(&en->fn_tail, en->lib, en->kernel_tail.c_str()));
+    }
+    // nine lattices per element take 70 KB at Q = 4 (EB = 8): the limit is raised once per device
+    if (en->smem > 48 * 1024 && dev >= 0 && dev < 64 && !(en->smem_set >> dev & 1)) {
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      B200_CHECK(cudaKernelSetAttributeForDevice(en->fn_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)en->smem, dev));
+      en->smem_set |= 1ull << dev;
+    }
+  }
+  if (nin != en->nin) return b200::set_error_msg("b200_jit_diag_apply: field count differs from the compiled one");
+  if (ctx_bytes > B200_JIT_MAX_CTX) {
+    char msg[160];
+    snprintf(msg, sizeof msg, "b200_jit_diag_apply: context of %zu bytes; a JIT QFunction takes at most %d", ctx_bytes,
+             B200_JIT_MAX_CTX);
+    return b200::set_error_msg(msg);
+  }
+  if (ctx_bytes && !h_ctx) return b200::set_error_msg("b200_jit_diag_apply: NULL context");
+  if (nelem <= 0) return 0;
+  const int P = en->P, Q = en->Q, P3 = P * P * P, Q3 = Q * Q * Q, EB = en->lay[4], NT = en->lay[5];
+  double mats[3 * 8 * 8];  // b200_k14_mats_t for this (P, Q): B.B, B.D, D.D element-wise, each [Q][P]
+  for (int i = 0; i < Q * P; i++) {
+    mats[i] = h_interp1d[i] * h_interp1d[i];
+    mats[Q * P + i] = h_interp1d[i] * h_grad1d[i];
+    mats[2 * Q * P + i] = h_grad1d[i] * h_grad1d[i];
+  }
+  JitCtx ctx;
+  memset(&ctx, 0, sizeof ctx);
+  if (ctx_bytes) memcpy(ctx.b, h_ctx, ctx_bytes);
+  const double *fin[B200_JIT_MAXF] = {};
+  for (int i = 0; i < nin; i++) fin[i] = i == en->ai ? nullptr : d_in[i];
+  const int nfull = nelem / EB, ntail = nelem - nfull * EB;
+  if (nfull) {
+    int n = nfull * EB;
+    void *args[] = {mats, &ctx, fin, &n, &d_offsets, &d_diag, &d_evec};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn, dim3(nfull), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_diag_apply");
+  }
+  if (ntail) {  // the partial group at the end: a run-time group extent, one CTA
+    const size_t e0 = (size_t)nfull * EB;
+    const double *ft[B200_JIT_MAXF] = {};
+    for (int i = 0; i < nin; i++)
+      if (fin[i]) ft[i] = fin[i] + e0 * en->in_size[i] * Q3;
+    const int *off = d_offsets + e0 * P3;
+    double *ev = d_evec ? d_evec + e0 * 3 * P3 : nullptr;
+    int n = ntail;
+    void *args[] = {mats, &ctx, ft, &n, &off, &d_diag, &ev};
+    B200_CHECK(cudaLaunchKernel((const void *)en->fn_tail, dim3(1), dim3(NT), args, en->smem, b200::g_stream));
+    B200_LAUNCH_CHECK("b200_jit_diag_apply(tail)");
   }
   return 0;
 }

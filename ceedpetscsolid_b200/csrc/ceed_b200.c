@@ -12,7 +12,8 @@
  *   FUSED     residual / Jacobian operators of the three material models -> one kernel
  *             (b200_apply_residual / b200_apply_jacobian); transfer operators -> b200_apply_transfer
  *   JIT_FUSED residual / Jacobian-shaped operators of a JIT-compiled user QFunction -> one generated kernel (K12,
- *             b200_jit_fused_apply), compiled at the operator's first apply
+ *             b200_jit_fused_apply), compiled at the operator's first apply; their diagonal -> K14
+ *             (b200_jit_diag_apply), compiled at the operator's first diagonal
  *   GENERIC   everything else: restriction, basis and QFunction kernels chained on the device
  * There is no CPU fallback: a QFunction the backend does not recognise is an error, unless the resource carries
  * ":jit" -- then it is compiled from its source file with NVRTC (b200_jit.cu) and runs on K12 or the generic path.
@@ -131,8 +132,9 @@ struct CeedOperator_private {
   CeedVector xfer_scale;
   int xfer_inject;
   /* OP_JIT_FUSED: the active input / output fields; jit_fused = K12 program handle + 1 (0: not compiled yet);
-     jit_assemble = K13 program handle + 1 (compiled at the first CeedOperatorLinearAssemble) */
-  int jit_ai, jit_ao, jit_fused, jit_assemble;
+     jit_assemble = K13 program handle + 1 (compiled at the first CeedOperatorLinearAssemble); jit_diag = K14 program
+     handle + 1 (compiled at the first CeedOperatorLinearAssembleDiagonal) */
+  int jit_ai, jit_ao, jit_fused, jit_assemble, jit_diag;
   /* generic-path work buffers (device), grown on demand */
   double *ebuf[2 * MAXF], *qbuf[2 * MAXF];
   size_t ebytes[2 * MAXF], qbytes[2 * MAXF];
@@ -1067,6 +1069,7 @@ static int op_setup(CeedOperator op) {
   }
   op->jit_fused = 0;
   op->jit_assemble = 0;
+  op->jit_diag = 0;
   if (qf->jit_handle >= 0) {
     op->kind = qf->jit_text && jit_fused_eligible(op) ? OP_JIT_FUSED : OP_GENERIC;
     return 0;
@@ -1496,7 +1499,8 @@ static int op_apply_fused_range(CeedOperator op, CeedVector in, CeedVector out, 
   return 0;
 }
 
-/* K12: compile the fused program at the first apply (the point program of op_setup stays for the generic diagonal) */
+/* K12: compile the fused program at the first apply (the point program of op_setup stays: it reports source errors
+ * at set-up) */
 static int jit_fused_handle(CeedOperator op, int *h) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
@@ -1728,6 +1732,40 @@ int CeedOperatorApply(CeedOperator op, CeedVector in, CeedVector out, CeedReques
   return vec_write_through(out);
 }
 
+/* K14: compile the diagonal program at the operator's first diagonal, then add the diagonal of the user function's
+ * operator (linear in its active input, as every Jacobian QFunction is) to `assembled`.  The passive inputs are read
+ * where K12 reads them; passive outputs are never written.  Same output convention as the built-in diagonal (K3). */
+static int op_diagonal_jit(CeedOperator op, CeedVector assembled) {
+  Ceed ceed = op->ceed;
+  CeedQFunction qf = op->qf;
+  OpField *u = &op->in[op->jit_ai];
+  if (assembled->length < u->r->lsize)
+    return CeedError(ceed, 1, "CeedOperatorLinearAssembleDiagonal: operator %s: vector shorter than the restriction's "
+                              "L-vector size %d", qf->name, u->r->lsize);
+  if (!op->jit_diag) {
+    int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
+    for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
+    for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
+    if (b200_jit_diag_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai,
+                              op->jit_ao, u->b->P, u->b->Q, &hh))
+      return CeedError(ceed, 1, "%s: diagonal kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
+                       qf->jit_path, b200_last_error());
+    op->jit_diag = hh + 1;
+  }
+  size_t bytes;
+  CeedChk(jit_ctx_bytes(qf, &bytes));
+  const double *din[MAXF] = {NULL};
+  for (int i = 0; i < qf->nin; i++)
+    if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &din[i]));
+  double *d, *evec = NULL;
+  CeedChk(vec_dev_rw(assembled, &d));
+  if (ceed->deterministic) CeedChk(det_scratch(ceed, (size_t)u->r->nelem * u->r->elemsize * 3 * sizeof(double), &evec));
+  B2(ceed, b200_jit_diag_apply(op->jit_diag - 1, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
+                               u->r->d_offsets, qf->nin, din, d, evec));
+  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, d));
+  return 0;
+}
+
 int CeedOperatorLinearAssembleAddDiagonal(CeedOperator op, CeedVector assembled, CeedRequest *request) {
   (void)request;
   Ceed ceed = op->ceed;
@@ -1736,6 +1774,7 @@ int CeedOperatorLinearAssembleAddDiagonal(CeedOperator op, CeedVector assembled,
     return 0;
   }
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
+  if (op->kind == OP_JIT_FUSED) return op_diagonal_jit(op, assembled);
   if (op->kind != OP_FUSED_JACOBIAN && !(op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS))
     return op_diagonal_generic(op, assembled);
   OpField *u = &op->in[0];

@@ -376,6 +376,27 @@ int b200_jit_assemble_compile(const char *text, const char *src_name, const char
 int b200_jit_assemble_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
                             const double *h_grad1d, int nin, const double *const *d_in, double *d_values);
 
+/* ---- K14: the operator diagonal around a JIT-compiled user QFunction (csrc/b200_jit_diag.cuh) ----------------------
+ * b200_jit_diag_compile (no device needed): text + the kernel of b200_jit_diag.cuh around QFunction `name` for the
+ *   basis (P, Q) (one of b200_fused_supported; the lattice constants are those of b200_apply_smem_layout); fields as
+ *   for b200_jit_fused_compile.  Any other (P, Q), or an active field that is not 9 wide, is refused.  Compiled unless
+ *   the same program (text, name, sizes, active fields, P, Q) was compiled before; counted by b200_jit_compile_count
+ *   and shown by b200_jit_program.
+ * b200_jit_diag_apply: d_diag += the diagonal of E^T G^T D_q G E on nelem elements, D_q the point tangent of the user
+ *   function, dout_active / din_active, from 3 calls per point and component with the unit active inputs (passive
+ *   inputs as given, passive outputs discarded; the return code is ignored).  The off-diagonal gradient terms enter as
+ *   D[c d][c d'] + D[c d'][c d], so a non-symmetric tangent is handled.  This is the operator's diagonal only if the
+ *   function is linear in its active input.  One launch for the full element groups and one for a partial last group,
+ *   on the backend stream.  d_evec NULL: FP64 atomics into d_diag at d_offsets + c; else d_evec [e][node][comp] is
+ *   stored for b200_transpose_gather_add and d_diag is untouched.  d_in of the passive inputs: q-blocked vectors of
+ *   nelem elements; entries of the active field are ignored.  The context is copied from the host pointer at every
+ *   call (at most B200_JIT_MAX_CTX bytes). */
+int b200_jit_diag_compile(const char *text, const char *src_name, const char *name, int nin, const int *in_sizes,
+                          int nout, const int *out_sizes, int active_in, int active_out, int P, int Q, int *handle);
+int b200_jit_diag_apply(int handle, const void *h_ctx, size_t ctx_bytes, int nelem, const double *h_interp1d,
+                        const double *h_grad1d, const int *d_offsets, int nin, const double *const *d_in,
+                        double *d_diag, double *d_evec);
+
 #ifdef __cplusplus
 }
 #endif
