@@ -170,10 +170,11 @@ class Elasticity:
         {"apply": "<file>:<Name>", "jacob": "<file>:<Name>"} replaces the residual / Jacobian QFunctions of app.problem
         (same fields) by user QFunctions, compiled at set-up on the "/gpu/b200:jit" resource.  Their operators run on
         K12, the fused kernel generated around the user function (compiled at the first apply), and their diagonal on
-        the generic path.  The p = 1 level has no built-in Jacobian: on unstructured meshes, and with coarse="amg" on
-        any mesh, its element matrices come from K13, CeedOperatorLinearAssemble around the user function (which must
-        be linear in its active input, as every Jacobian QFunction is); box meshes with "hmg" or "pcg" assemble it by
-        colouring.  Strain energy and diagnostics keep the problem's stock model."""
+        K14, the diagonal kernel generated around it (compiled at the first diagonal; the Jacobi / Chebyshev smoothers
+        of every level call it).  The p = 1 level has no built-in Jacobian: on unstructured meshes, and with
+        coarse="amg" on any mesh, its element matrices come from K13, CeedOperatorLinearAssemble around the user
+        function (which must be linear in its active input, as every Jacobian QFunction is); box meshes with "hmg" or
+        "pcg" assemble it by colouring.  Strain energy and diagnostics keep the problem's stock model."""
         if coarse == "amg" and world > 1:
             # checked before any device work: the redundant AMG gathers every rank's element matrices and right-hand
             # side through the process group, and exists only for the masked layout

@@ -1,4 +1,4 @@
-"""User QFunction sources for the tests of the fused kernel around JIT-compiled QFunctions (K12)."""
+"""User QFunction sources for the tests of the kernels around JIT-compiled QFunctions (K12, K13, K14)."""
 
 # A linear-elastic model with extra passive fields, its active fields away from index 0 (fields map by declaration
 # order): in = [scale (1), du (9, gradient), qdata (10)], out = [sdiag (3), dv (9, gradient), energy (1)].
@@ -90,3 +90,40 @@ CEED_QFUNCTION(EdgeF)(void *ctx, const CeedInt Q, const CeedScalar *const *in, C
 }
 """
 EDGE_IN, EDGE_OUT, EDGE_AI, EDGE_AO, EDGE_CTX = [1, 2, 7, 64, 3, 5, 10, 9], [2, 64, 1, 9, 7, 3, 5, 11], 7, 3, 256
+
+
+# A non-symmetric linear model: dv = wdetJ dXdx sigma, sigma_i = sum_j K[9 i + j] H_j, H = the physical gradient of du,
+# i = c*3 + k; K (the context, 81 doubles) is not symmetric, so neither is the point tangent.
+# in = [du (9, gradient), qdata (10)], out = [dv (9, gradient)].
+NONSYM = r"""#include <ceed.h>
+CEED_QFUNCTION(NonSymdF)(void *ctx, const CeedInt Q, const CeedScalar *const *in, CeedScalar *const *out) {
+  const CeedScalar *K = (const CeedScalar *)ctx;
+  const CeedScalar(*du)[3][CEED_Q_VLA] = (const CeedScalar(*)[3][CEED_Q_VLA])in[0];
+  const CeedScalar(*qd)[CEED_Q_VLA] = (const CeedScalar(*)[CEED_Q_VLA])in[1];
+  CeedScalar(*dv)[3][CEED_Q_VLA] = (CeedScalar(*)[3][CEED_Q_VLA])out[0];
+  for (CeedInt i = 0; i < Q; i++) {
+    CeedScalar X[3][3], H[9], sig[9];
+    for (int a = 0; a < 3; a++)
+      for (int b = 0; b < 3; b++) X[a][b] = qd[1 + 3 * a + b][i];
+    for (int c = 0; c < 3; c++)
+      for (int k = 0; k < 3; k++) {
+        CeedScalar t = 0;
+        for (int m = 0; m < 3; m++) t += X[m][k] * du[m][c][i];
+        H[c * 3 + k] = t;
+      }
+    for (int r = 0; r < 9; r++) {
+      CeedScalar t = 0;
+      for (int s = 0; s < 9; s++) t += K[9 * r + s] * H[s];
+      sig[r] = t;
+    }
+    for (int k = 0; k < 3; k++)
+      for (int c = 0; c < 3; c++) {
+        CeedScalar t = 0;
+        for (int m = 0; m < 3; m++) t += X[k][m] * sig[c * 3 + m];
+        dv[k][c][i] = t * qd[0][i];
+      }
+  }
+  return 0;
+}
+"""
+NONSYM_IN, NONSYM_OUT, NONSYM_CTX = [9, 10], [9], 81

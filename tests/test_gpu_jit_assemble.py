@@ -125,6 +125,16 @@ def shape_gradients(Q):
     return B, D, G
 
 
+def element_matrices(Dt, Q):
+    """K[e][col = j*3 + b][row = i*3 + a] = sum_q sum_{k,m} G[q,i,k] Dt[e,q,m*3 + b,k*3 + a] G[q,j,m], flattened to
+    [e][576]: the trilinear element matrices of a point tangent Dt[e][q][s][o] (test_gpu_jit_diag.host_tangent's
+    layout)"""
+    nelem, nq = Dt.shape[:2]
+    _, _, Gs = shape_gradients(Q)
+    Dr = Dt.reshape(nelem, nq, 3, 3, 3, 3)                 # [e][q][m][b][k][a]
+    return np.einsum("qik,eqmbka,qjm->ejbia", Gs, Dr, Gs).reshape(nelem, 576)
+
+
 def qblocked(a):
     """[elem][comp][q] -> the q-blocked backend layout"""
     from test_gpu_operator_kernels import to_qb
@@ -151,10 +161,8 @@ def test_edge_model_against_its_host_tangent(tmp_path, Q):
         (sub / "edge.h").write_text(EDGE_FIELDS)
         outs = _host_point_model(sub, ctx, nelem, nq, pin + [act], EDGE_OUT, header="edge.h", name="EdgeF")
         Dt[:, :, s, :] = outs[EDGE_AO].transpose(0, 2, 1)
-    B, D, Gs = shape_gradients(Q)
-    # K[e][col = j*3 + b][row = i*3 + a] = sum_q sum_{k,m} G[q,i,k] Dt[e,q,m*3 + b,k*3 + a] G[q,j,m]
-    Dr = Dt.reshape(nelem, nq, 3, 3, 3, 3)                 # [e][q][m][b][k][a]
-    ref = np.einsum("qik,eqmbka,qjm->ejbia", Gs, Dr, Gs).reshape(nelem, 576)
+    B, D, _ = shape_gradients(Q)
+    ref = element_matrices(Dt, Q)
     h = libceed.jit_assemble_compile(tmp_path / "edge.h", "EdgeF", EDGE_IN, EDGE_OUT, EDGE_AI, EDGE_AO, 2, Q)
     d_in = [torch.from_numpy(qblocked(a)).cuda() for a in pin]
     ptrs = [t.data_ptr() for t in d_in] + [0]

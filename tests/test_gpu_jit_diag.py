@@ -14,7 +14,7 @@ from ceedpetscsolid_b200 import ceed as libceed
 from ceedpetscsolid_b200.ceed import b2, lib
 from ceedpetscsolid_b200.exodus import tube_mesh
 from helpers import OracleProblem, reoriented, rel_err
-from jit_models import EDGE_AI, EDGE_AO, EDGE_CTX, EDGE_FIELDS, EDGE_IN, EDGE_OUT, EXTRA_FIELDS
+from jit_models import EDGE_AI, EDGE_AO, EDGE_CTX, EDGE_FIELDS, EDGE_IN, EDGE_OUT, EXTRA_FIELDS, NONSYM
 from oracle import oracle
 from test_gpu_jit import SVK_HEADER, _host_point_model, port_locators
 from test_gpu_jit_assemble import coo, dense, qblocked
@@ -133,41 +133,7 @@ def test_a_smoother_context_gives_the_diagonal_for_its_constants(pair):
 
 
 # ------------------------------------------------------------------- 3. a non-symmetric linear model, host tangents
-# dv = wdetJ dXdx sigma, sigma_i = sum_j K[9 i + j] H_j, H = the physical gradient of du, i = c*3 + k; K (the context,
-# 81 doubles) is not symmetric, so neither is the point tangent
-NONSYM = r"""#include <ceed.h>
-CEED_QFUNCTION(NonSymdF)(void *ctx, const CeedInt Q, const CeedScalar *const *in, CeedScalar *const *out) {
-  const CeedScalar *K = (const CeedScalar *)ctx;
-  const CeedScalar(*du)[3][CEED_Q_VLA] = (const CeedScalar(*)[3][CEED_Q_VLA])in[0];
-  const CeedScalar(*qd)[CEED_Q_VLA] = (const CeedScalar(*)[CEED_Q_VLA])in[1];
-  CeedScalar(*dv)[3][CEED_Q_VLA] = (CeedScalar(*)[3][CEED_Q_VLA])out[0];
-  for (CeedInt i = 0; i < Q; i++) {
-    CeedScalar X[3][3], H[9], sig[9];
-    for (int a = 0; a < 3; a++)
-      for (int b = 0; b < 3; b++) X[a][b] = qd[1 + 3 * a + b][i];
-    for (int c = 0; c < 3; c++)
-      for (int k = 0; k < 3; k++) {
-        CeedScalar t = 0;
-        for (int m = 0; m < 3; m++) t += X[m][k] * du[m][c][i];
-        H[c * 3 + k] = t;
-      }
-    for (int r = 0; r < 9; r++) {
-      CeedScalar t = 0;
-      for (int s = 0; s < 9; s++) t += K[9 * r + s] * H[s];
-      sig[r] = t;
-    }
-    for (int k = 0; k < 3; k++)
-      for (int c = 0; c < 3; c++) {
-        CeedScalar t = 0;
-        for (int m = 0; m < 3; m++) t += X[k][m] * sig[c * 3 + m];
-        dv[k][c][i] = t * qd[0][i];
-      }
-  }
-  return 0;
-}
-"""
-
-
+# NONSYM (tests/jit_models.py): a linear model whose point tangent is not symmetric
 def shape_gradients(P, Q):
     """G[q][node][k]: reference gradients of the tensor shape functions, q = qx + Q qy + Q^2 qz, node = ix + P iy +
     P^2 iz"""
@@ -181,10 +147,10 @@ def shape_gradients(P, Q):
     return B, D, np.stack([Dx * By * Bz, Bx * Dy * Bz, Bx * By * Dz], axis=-1)
 
 
-def host_element_diagonal(tmp_path, header, name, ctx, nelem, nq, passive, ai, ao, out_sizes, P, Q):
-    """diag_e[e][node][c] = sum_q sum_{k,m} G_k D[c k][c m] G_m from the gcc build of `header` at the 9 unit active
-    inputs (passive inputs [elem][comp][q], inserted around the active input at index ai)"""
-    Dt = np.zeros((nelem, nq, 9, 9))  # [e][q][s = m*3 + b][o = k*3 + a]
+def host_tangent(tmp_path, header, name, ctx, nelem, nq, passive, ai, ao, out_sizes):
+    """Dt[e][q][s = m*3 + b][o = k*3 + a] = dW[a][k] / dH[b][m]: the gcc build of `header` at the 9 unit active inputs
+    (passive inputs [elem][comp][q], inserted around the active input at index ai)"""
+    Dt = np.zeros((nelem, nq, 9, 9))
     for s in range(9):
         act = np.zeros((nelem, 9, nq))
         act[:, s, :] = 1.0
@@ -194,9 +160,19 @@ def host_element_diagonal(tmp_path, header, name, ctx, nelem, nq, passive, ai, a
         outs = _host_point_model(sub, ctx, nelem, nq, passive[:ai] + [act] + passive[ai:], out_sizes, header=header,
                                  name=name)
         Dt[:, :, s, :] = outs[ao].transpose(0, 2, 1)
+    return Dt
+
+
+def element_diagonal(Dt, P, Q):
+    """diag_e[e][node][c] = sum_q sum_{k,m} G_k D[c k][c m] G_m of a host tangent Dt (host_tangent's layout)"""
+    nelem, nq = Dt.shape[:2]
     Dc = np.einsum("eqmckc->eqmkc", Dt.reshape(nelem, nq, 3, 3, 3, 3))   # D[c k][c m] as [e][q][m][k][c]
     _, _, Gs = shape_gradients(P, Q)
     return np.einsum("qnk,eqmkc,qnm->enc", Gs, Dc, Gs)
+
+
+def host_element_diagonal(tmp_path, header, name, ctx, nelem, nq, passive, ai, ao, out_sizes, P, Q):
+    return element_diagonal(host_tangent(tmp_path, header, name, ctx, nelem, nq, passive, ai, ao, out_sizes), P, Q)
 
 
 def test_a_non_symmetric_model_against_its_probed_matrix_and_host_tangent(G, tmp_path):

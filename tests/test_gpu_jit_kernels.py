@@ -46,11 +46,16 @@ def stock_name(problem, jacobian):
 
 
 class PortCase(Case):
-    """Case whose oracle runs the gcc build of oracle/qf_port.c, the functions K12 is compiled around"""
+    """Case whose oracle runs the gcc build of oracle/qf_port.c, the functions K12, K13 and K14 are compiled
+    around"""
 
-    def oracle_apply(self, jacobian, x):
+    def oracle_apply(self, jacobian, x, off=None):
         return oracle.operator_apply(self.problem, jacobian, self.phys, self.nelem, self.P, self.Q, self.B, self.D,
-                                     self.off, self.qdata, self.gradu, x, which="port")
+                                     self.off if off is None else off, self.qdata, self.gradu, x, which="port")
+
+    def oracle_diagonal(self):
+        return oracle.operator_diagonal(self.problem, self.phys, self.nelem, self.P, self.Q, self.B, self.D, self.off,
+                                        self.qdata, self.gradu, self.lsize, which="port")
 
 
 def k12(h, ctx, nelem, c, d_off, d_x, d_y, d_ev, ins, outs, padd):

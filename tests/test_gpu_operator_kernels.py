@@ -95,8 +95,12 @@ def addend(rng, scale, n):
 
 
 def strip(nelem, h=0.5):
-    """a row of nelem perturbed cubes of side h: exact element counts"""
-    return BoxMesh(n=(nelem, 1, 1), perturb=0.1, seed=nelem % 97, lengths=(h * nelem, h, h))
+    """a row of nelem perturbed cubes of side h: exact element counts.  Every vertex of a strip lies on its boundary,
+    which BoxMesh(perturb=...) leaves in place, so the vertices are moved here: with cubes, every element would have
+    the same diagonal dX/dx, and a kernel that swapped x and y nodes, or elements, could still match"""
+    box = BoxMesh(n=(nelem, 1, 1), lengths=(h * nelem, h, h))
+    V = box.vertices + 0.1 * h * (rng_for("strip", nelem).random(box.vertices.shape) - 0.5)
+    return BoxMesh(n=(nelem, 1, 1), lengths=(h * nelem, h, h), vertices=V)
 
 
 def ptr(t):
@@ -124,9 +128,9 @@ class Case:
         self.d_off = dev(self.off.reshape(-1))
         self.d_qd = dev(to_qb(self.qdata), np.nan)
 
-    def oracle_apply(self, jacobian, x):
+    def oracle_apply(self, jacobian, x, off=None):
         return oracle.operator_apply(self.problem, jacobian, self.phys, self.nelem, self.P, self.Q, self.B, self.D,
-                                     self.off, self.qdata, self.gradu, x)
+                                     self.off if off is None else off, self.qdata, self.gradu, x)
 
     def oracle_diagonal(self):
         return oracle.operator_diagonal(self.problem, self.phys, self.nelem, self.P, self.Q, self.B, self.D, self.off,
@@ -156,6 +160,18 @@ class Case:
         b2(lib.b200_jcache_build(self.pid, self.nelem, self.Q, self.d_qd.data_ptr(), ptr(gradu_dev), jc.data_ptr()))
         assert np.isfinite(fetch(jc, nj)).all(), "Jacobian cache entries left unwritten"
         return jc
+
+
+def probed_element_matrices(c):
+    """[e][col][row] = K_e[row, col] of a P = 2 case, element dof node*3 + comp: 24 unit probes of the case's oracle
+    Jacobian on the same elements with every element's nodes its own (offsets = arange(8 nelem) * 3)"""
+    own = (np.arange(c.nelem * 8, dtype=np.int32) * 3).reshape(c.nelem, 8)
+    ref = np.empty((c.nelem, 24, 24))
+    for col in range(24):
+        x = np.zeros(c.nelem * 24)
+        x[col::24] = 1.0
+        ref[:, col, :] = c.oracle_apply(True, x, own).reshape(c.nelem, 24)
+    return ref
 
 
 def ordered_add(lsize, off, elemsize, ev, d_y):
@@ -303,8 +319,7 @@ def test_inject_is_refused_on_the_host_unless_it_is_a_scaled_prolongation():
 @pytest.mark.parametrize("Q", [2, 3, 4, 5])
 @pytest.mark.parametrize("problem", PROBLEMS)
 def test_assemble_p1_element_matrices(problem, Q):
-    """d_values[(e*24 + col)*24 + row] = K_e[row, col], element dof node*3 + comp; reference: 24 unit probes of the
-    oracle Jacobian on the same elements with every element's nodes its own (offsets = arange(8 nelem) * 3)"""
+    """d_values[(e*24 + col)*24 + row] = K_e[row, col], element dof node*3 + comp, against probed_element_matrices"""
     nelem = 2 * eb(Q) + 3
     c = Case(problem, 2, Q, nelem)
     d_gu = dev(to_qb(c.gradu), np.nan) if c.has_gradu else None
@@ -313,13 +328,7 @@ def test_assemble_p1_element_matrices(problem, Q):
     vals = out(n)
     b2(lib.b200_assemble_p1(c.pid, C.addressof(c.cphys), nelem, Q, c.B.ctypes.data, c.D.ctypes.data, jc.data_ptr(),
                             vals.data_ptr()))
-    own = (np.arange(nelem * 8, dtype=np.int32) * 3).reshape(nelem, 8)
-    ref = np.empty((nelem, 24, 24))
-    for col in range(24):
-        x = np.zeros(nelem * 24)
-        x[col::24] = 1.0
-        y = oracle.operator_apply(problem, True, c.phys, nelem, 2, Q, c.B, c.D, own, c.qdata, c.gradu, x)
-        ref[:, col, :] = y.reshape(nelem, 24)
+    ref = probed_element_matrices(c)
     check(fetch(vals, n).reshape(nelem, 24, 24), ref, ref, "element matrices")
 
 
