@@ -519,74 +519,47 @@ class Operator(_Obj):
         return bool(f.value)
 
 
-def jit_compile(path, name, in_sizes, out_sizes):
-    """The compile half of "/gpu/b200:jit" without a device: the QFunction `name` of the source file `path` (quoted
-    includes inlined) with the given field sizes, compiled by NVRTC for sm_100a (cached per process).  Returns the
-    handle; raises CeedError with the reason (unreadable file, NVRTC log)."""
+def _jit_compile(compile_fn, path, name, in_sizes, out_sizes, *ints):
+    """Read the QFunction source `path` (quoted includes inlined) and call compile_fn, one of the b200_jit_*compile
+    entry points, with its field sizes and trailing ints; returns the handle or raises CeedError with the reason."""
     text, err = C.c_void_p(), C.create_string_buffer(1024)
     if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
         raise CeedError(err.value.decode())
     h = C.c_int(-1)
     try:
-        rc = lib.b200_jit_compile(text, str(path).encode(), name.encode(), len(in_sizes), (C.c_int * 8)(*in_sizes),
-                                  len(out_sizes), (C.c_int * 8)(*out_sizes), C.byref(h))
+        rc = compile_fn(text, str(path).encode(), name.encode(), len(in_sizes), (C.c_int * 8)(*in_sizes),
+                        len(out_sizes), (C.c_int * 8)(*out_sizes), *(int(i) for i in ints), C.byref(h))
     finally:
         lib.b200_jit_free_source(text)
     b2(rc)
     return h.value
+
+
+def jit_compile(path, name, in_sizes, out_sizes):
+    """The compile half of "/gpu/b200:jit" without a device: the QFunction `name` of the source file `path` (quoted
+    includes inlined) with the given field sizes, compiled by NVRTC for sm_100a (cached per process).  Returns the
+    handle; raises CeedError with the reason (unreadable file, NVRTC log)."""
+    return _jit_compile(lib.b200_jit_compile, path, name, in_sizes, out_sizes)
 
 
 def jit_fused_compile(path, name, in_sizes, out_sizes, active_in, active_out, P, Q):
     """The compile half of K12 without a device: the fused operator kernel around QFunction `name` of `path` for the
     basis (P, Q), with field active_in / active_out as the active gradient and every other field passive (q-blocked).
     Returns the handle (cached per process, as jit_compile)."""
-    text, err = C.c_void_p(), C.create_string_buffer(1024)
-    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
-        raise CeedError(err.value.decode())
-    h = C.c_int(-1)
-    try:
-        rc = lib.b200_jit_fused_compile(text, str(path).encode(), name.encode(), len(in_sizes),
-                                        (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
-                                        int(active_in), int(active_out), int(P), int(Q), C.byref(h))
-    finally:
-        lib.b200_jit_free_source(text)
-    b2(rc)
-    return h.value
+    return _jit_compile(lib.b200_jit_fused_compile, path, name, in_sizes, out_sizes, active_in, active_out, P, Q)
 
 
 def jit_assemble_compile(path, name, in_sizes, out_sizes, active_in, active_out, P, Q):
     """The compile half of K13 without a device: the element-matrix kernel of a trilinear level (P = 2) around
     QFunction `name` of `path`, fields as for jit_fused_compile.  Returns the handle (cached per process, as
     jit_compile)."""
-    text, err = C.c_void_p(), C.create_string_buffer(1024)
-    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
-        raise CeedError(err.value.decode())
-    h = C.c_int(-1)
-    try:
-        rc = lib.b200_jit_assemble_compile(text, str(path).encode(), name.encode(), len(in_sizes),
-                                           (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
-                                           int(active_in), int(active_out), int(P), int(Q), C.byref(h))
-    finally:
-        lib.b200_jit_free_source(text)
-    b2(rc)
-    return h.value
+    return _jit_compile(lib.b200_jit_assemble_compile, path, name, in_sizes, out_sizes, active_in, active_out, P, Q)
 
 
 def jit_diag_compile(path, name, in_sizes, out_sizes, active_in, active_out, P, Q):
     """The compile half of K14 without a device: the operator-diagonal kernel for the basis (P, Q) around QFunction
     `name` of `path`, fields as for jit_fused_compile.  Returns the handle (cached per process, as jit_compile)."""
-    text, err = C.c_void_p(), C.create_string_buffer(1024)
-    if lib.b200_jit_read_source(str(path).encode(), C.byref(text), err, len(err)):
-        raise CeedError(err.value.decode())
-    h = C.c_int(-1)
-    try:
-        rc = lib.b200_jit_diag_compile(text, str(path).encode(), name.encode(), len(in_sizes),
-                                       (C.c_int * 8)(*in_sizes), len(out_sizes), (C.c_int * 8)(*out_sizes),
-                                       int(active_in), int(active_out), int(P), int(Q), C.byref(h))
-    finally:
-        lib.b200_jit_free_source(text)
-    b2(rc)
-    return h.value
+    return _jit_compile(lib.b200_jit_diag_compile, path, name, in_sizes, out_sizes, active_in, active_out, P, Q)
 
 
 def jit_program(handle):

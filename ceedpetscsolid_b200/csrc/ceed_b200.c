@@ -1499,23 +1499,26 @@ static int op_apply_fused_range(CeedOperator op, CeedVector in, CeedVector out, 
   return 0;
 }
 
-/* K12: compile the fused program at the first apply (the point program of op_setup stays: it reports source errors
- * at set-up) */
-static int jit_fused_handle(CeedOperator op, int *h) {
+/* K12, K13, K14: the operator's program of the given kind, compiled with `compile` at its first use; *slot holds the
+ * handle + 1 (0: not compiled yet).  K12 is compiled at the first apply (the point program of op_setup stays: it
+ * reports source errors at set-up), K13 at the first CeedOperatorLinearAssemble, K14 at the first diagonal. */
+typedef int (*jit_compile_fn)(const char *, const char *, const char *, int, const int *, int, const int *, int, int,
+                              int, int, int *);
+static int jit_op_handle(CeedOperator op, jit_compile_fn compile, int *slot, const char *what, int *h) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
-  if (!op->jit_fused) {
+  if (!*slot) {
     int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
     for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
     for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
     CeedBasis b = op->in[op->jit_ai].b;
-    if (b200_jit_fused_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai,
-                               op->jit_ao, b->P, b->Q, &hh))
-      return CeedError(ceed, 1, "%s: fused kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
+    if (compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai, op->jit_ao,
+                b->P, b->Q, &hh))
+      return CeedError(ceed, 1, "%s: %s of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, what, qf->name,
                        qf->jit_path, b200_last_error());
-    op->jit_fused = hh + 1;
+    *slot = hh + 1;
   }
-  *h = op->jit_fused - 1;
+  *h = *slot - 1;
   return 0;
 }
 
@@ -1530,7 +1533,7 @@ static int op_apply_jit_range(CeedOperator op, CeedVector in, CeedVector out, in
     return CeedError(ceed, 1, "operator %s: active vectors shorter than the restriction's L-vector size %d", qf->name, u->r->lsize);
   int h;
   size_t bytes;
-  CeedChk(jit_fused_handle(op, &h));
+  CeedChk(jit_op_handle(op, b200_jit_fused_compile, &op->jit_fused, "fused kernel", &h));
   CeedChk(jit_ctx_bytes(qf, &bytes));
   double *evec = NULL;
   if (ceed->deterministic) {
@@ -1675,7 +1678,7 @@ int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in, CeedVector 
     if (op->kind == OP_FUSED_JACOBIAN) CeedChk(jcache_get(op, &jc));
     if (op->kind == OP_JIT_FUSED) {  /* compiled, and the passive vectors current on the device, before the fork */
       int h;
-      CeedChk(jit_fused_handle(op, &h));
+      CeedChk(jit_op_handle(op, b200_jit_fused_compile, &op->jit_fused, "fused kernel", &h));
       for (int i = 0; i < op->qf->nin; i++)
         if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &x));
       for (int i = 0; i < op->qf->nout; i++)
@@ -1742,17 +1745,9 @@ static int op_diagonal_jit(CeedOperator op, CeedVector assembled) {
   if (assembled->length < u->r->lsize)
     return CeedError(ceed, 1, "CeedOperatorLinearAssembleDiagonal: operator %s: vector shorter than the restriction's "
                               "L-vector size %d", qf->name, u->r->lsize);
-  if (!op->jit_diag) {
-    int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
-    for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
-    for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
-    if (b200_jit_diag_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai,
-                              op->jit_ao, u->b->P, u->b->Q, &hh))
-      return CeedError(ceed, 1, "%s: diagonal kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
-                       qf->jit_path, b200_last_error());
-    op->jit_diag = hh + 1;
-  }
+  int h;
   size_t bytes;
+  CeedChk(jit_op_handle(op, b200_jit_diag_compile, &op->jit_diag, "diagonal kernel", &h));
   CeedChk(jit_ctx_bytes(qf, &bytes));
   const double *din[MAXF] = {NULL};
   for (int i = 0; i < qf->nin; i++)
@@ -1760,7 +1755,7 @@ static int op_diagonal_jit(CeedOperator op, CeedVector assembled) {
   double *d, *evec = NULL;
   CeedChk(vec_dev_rw(assembled, &d));
   if (ceed->deterministic) CeedChk(det_scratch(ceed, (size_t)u->r->nelem * u->r->elemsize * 3 * sizeof(double), &evec));
-  B2(ceed, b200_jit_diag_apply(op->jit_diag - 1, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
+  B2(ceed, b200_jit_diag_apply(h, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
                                u->r->d_offsets, qf->nin, din, d, evec));
   if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, d));
   return 0;
@@ -1849,22 +1844,14 @@ static int op_assemble_jit(CeedOperator op, double *v) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
   OpField *u = &op->in[op->jit_ai];
-  if (!op->jit_assemble) {
-    int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
-    for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
-    for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
-    if (b200_jit_assemble_compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes,
-                                  op->jit_ai, op->jit_ao, u->b->P, u->b->Q, &hh))
-      return CeedError(ceed, 1, "%s: assembly kernel of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, qf->name,
-                       qf->jit_path, b200_last_error());
-    op->jit_assemble = hh + 1;
-  }
+  int h;
   size_t bytes;
+  CeedChk(jit_op_handle(op, b200_jit_assemble_compile, &op->jit_assemble, "assembly kernel", &h));
   CeedChk(jit_ctx_bytes(qf, &bytes));
   const double *din[MAXF] = {NULL};
   for (int i = 0; i < qf->nin; i++)
     if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &din[i]));
-  B2(ceed, b200_jit_assemble_apply(op->jit_assemble - 1, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
+  B2(ceed, b200_jit_assemble_apply(h, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
                                    qf->nin, din, v));
   return 0;
 }
