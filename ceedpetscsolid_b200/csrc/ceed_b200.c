@@ -131,10 +131,11 @@ struct CeedOperator_private {
   /* fused transfer operators: optional fine-side pointwise scaling (CeedOperatorSetTransferScalingB200) */
   CeedVector xfer_scale;
   int xfer_inject;
-  /* OP_JIT_FUSED: the active input / output fields; jit_fused = K12 program handle + 1 (0: not compiled yet);
-     jit_assemble = K13 program handle + 1 (compiled at the first CeedOperatorLinearAssemble); jit_diag = K14 program
-     handle + 1 (compiled at the first CeedOperatorLinearAssembleDiagonal) */
-  int jit_ai, jit_ao, jit_fused, jit_assemble, jit_diag;
+  /* ai / ao: the active input / output fields of a fused apply (0 / 0 for the built-in residual and Jacobian, whose
+     QFunctions fix the field order; 0 for every other kind).  OP_JIT_FUSED: jit_fused = K12 program handle + 1 (0: not
+     compiled yet); jit_assemble = K13 program handle + 1 (compiled at the first CeedOperatorLinearAssemble); jit_diag =
+     K14 program handle + 1 (compiled at the first CeedOperatorLinearAssembleDiagonal) */
+  int ai, ao, jit_fused, jit_assemble, jit_diag;
   /* generic-path work buffers (device), grown on demand */
   double *ebuf[2 * MAXF], *qbuf[2 * MAXF];
   size_t ebytes[2 * MAXF], qbytes[2 * MAXF];
@@ -556,14 +557,18 @@ static int rstr_ordered_add(CeedElemRestriction r, int layout, const double *eve
   return 0;
 }
 
-/* the Ceed's scratch E-vector (deterministic mode), at least `bytes` long */
-static int det_scratch(Ceed ceed, size_t bytes, double **p) {
+/* deterministic mode: the Ceed's scratch E-vector, grown to a transposed restriction through r, which the caller sums
+   into the L-vector with rstr_ordered_add; NULL otherwise (the kernels add with atomics) */
+static int det_evec(Ceed ceed, CeedElemRestriction r, double **evec) {
+  const size_t bytes = (size_t)r->nelem * r->elemsize * r->ncomp * sizeof(double);
+  *evec = NULL;
+  if (!ceed->deterministic) return 0;
   if (ceed->det_evec_bytes < bytes) {
     if (ceed->det_evec) { B2(ceed, b200_sync()); B2(ceed, b200_free(ceed->det_evec)); ceed->det_evec = NULL; ceed->det_evec_bytes = 0; }
     B2(ceed, b200_malloc((void **)&ceed->det_evec, bytes));
     ceed->det_evec_bytes = bytes;
   }
-  *p = ceed->det_evec;
+  *evec = ceed->det_evec;
   return 0;
 }
 
@@ -1018,9 +1023,25 @@ static int qf_jit_compile(CeedQFunction qf, int guard_differs) {
   return 0;
 }
 
-/* K12 (OP_JIT_FUSED): one active EVAL_GRAD input of 9 on a 3-component offsets restriction (compstride 1, P^3 nodes)
- * with a tensor basis whose (P, Q) has a fused layout, one active EVAL_GRAD output on the same restriction and basis
- * matrices, and every other field EVAL_NONE on a passive vector with a q-blocked restriction of the same nelem */
+/* the active fields of the fused kernels: input ai an active EVAL_GRAD of 9 on a 3-component offsets restriction
+ * (compstride 1, P^3 nodes) with a tensor basis whose (P, Q) has a fused layout, output ao an active EVAL_GRAD of 9 on
+ * the same restriction and the same basis matrices */
+static int fused_active_shape(CeedOperator op, int ai, int ao) {
+  CeedQFunction qf = op->qf;
+  OpField *u = &op->in[ai], *vv = &op->out[ao];
+  if (!(qf->in[ai].emode == CEED_EVAL_GRAD && qf->in[ai].size == 9 && u->v == CEED_VECTOR_ACTIVE && is_tensor3(u->b) &&
+        u->b->ncomp == 3 && u->r && u->r != CEED_ELEMRESTRICTION_NONE && u->r->strided == 0 && u->r->ncomp == 3 &&
+        u->r->compstride == 1 && u->r->elemsize == u->b->P * u->b->P * u->b->P && b200_fused_supported(u->b->P, u->b->Q)))
+    return 0;
+  const int Q = u->b->Q;
+  return qf->out[ao].emode == CEED_EVAL_GRAD && qf->out[ao].size == 9 && vv->v == CEED_VECTOR_ACTIVE && vv->r == u->r &&
+         (vv->b == u->b || (is_tensor3(vv->b) && vv->b->P == u->b->P && vv->b->Q == Q &&
+                            !memcmp(vv->b->interp1d, u->b->interp1d, sizeof(double) * Q * u->b->P) &&
+                            !memcmp(vv->b->grad1d, u->b->grad1d, sizeof(double) * Q * u->b->P)));
+}
+
+/* K12 (OP_JIT_FUSED): one active input and one active output of the fused active shape, and every other field
+ * EVAL_NONE on a passive vector with a q-blocked restriction of the same nelem */
 static int jit_fused_eligible(CeedOperator op) {
   CeedQFunction qf = op->qf;
   int ai = -1, ao = -1;
@@ -1028,18 +1049,9 @@ static int jit_fused_eligible(CeedOperator op) {
     if (op->in[i].v == CEED_VECTOR_ACTIVE) { if (ai >= 0) return 0; ai = i; }
   for (int i = 0; i < qf->nout; i++)
     if (op->out[i].v == CEED_VECTOR_ACTIVE) { if (ao >= 0) return 0; ao = i; }
-  if (ai < 0 || ao < 0) return 0;
-  OpField *u = &op->in[ai], *vv = &op->out[ao];
-  if (!(qf->in[ai].emode == CEED_EVAL_GRAD && qf->in[ai].size == 9 && is_tensor3(u->b) && u->b->ncomp == 3 && u->r &&
-        u->r != CEED_ELEMRESTRICTION_NONE && u->r->strided == 0 && u->r->ncomp == 3 && u->r->compstride == 1 &&
-        u->r->elemsize == u->b->P * u->b->P * u->b->P && b200_fused_supported(u->b->P, u->b->Q)))
-    return 0;
+  if (ai < 0 || ao < 0 || !fused_active_shape(op, ai, ao)) return 0;
+  OpField *u = &op->in[ai];
   const int Q = u->b->Q;
-  if (!(qf->out[ao].emode == CEED_EVAL_GRAD && qf->out[ao].size == 9 && vv->r == u->r &&
-        (vv->b == u->b || (is_tensor3(vv->b) && vv->b->P == u->b->P && vv->b->Q == Q &&
-                           !memcmp(vv->b->interp1d, u->b->interp1d, sizeof(double) * Q * u->b->P) &&
-                           !memcmp(vv->b->grad1d, u->b->grad1d, sizeof(double) * Q * u->b->P)))))
-    return 0;
   for (int i = 0; i < qf->nin + qf->nout; i++) {
     if (i == ai || i == qf->nin + ao) continue;
     const QFField *qff = i < qf->nin ? &qf->in[i] : &qf->out[i - qf->nin];
@@ -1048,8 +1060,8 @@ static int jit_fused_eligible(CeedOperator op) {
           f->r->nelem == u->r->nelem && (size_t)f->v->length >= (size_t)f->r->nelem * qff->size * Q * Q * Q))
       return 0;
   }
-  op->jit_ai = ai;
-  op->jit_ao = ao;
+  op->ai = ai;
+  op->ao = ao;
   return 1;
 }
 
@@ -1067,6 +1079,7 @@ static int op_setup(CeedOperator op) {
     if (qf->qf_id != B200_QF_NONE) CeedChk(qf_guard(qf, &differs));
     if (qf->qf_id == B200_QF_NONE || differs) CeedChk(qf_jit_compile(qf, differs));
   }
+  op->ai = op->ao = 0;
   op->jit_fused = 0;
   op->jit_assemble = 0;
   op->jit_diag = 0;
@@ -1089,20 +1102,12 @@ static int op_setup(CeedOperator op) {
                      : (id == B200_QF_HYPERSS_F || id == B200_QF_HYPERSS_DF) ? B200_PROB_HYPERSS : B200_PROB_HYPERFS;
     const int has_gradu = prob != B200_PROB_LINELAS;
     const int nin = is_jac && has_gradu ? 3 : 2, nout = is_res && has_gradu ? 2 : 1;
-    int ok = qf->nin == nin && qf->nout == nout;
+    int ok = qf->nin == nin && qf->nout == nout && fused_active_shape(op, 0, 0);
     if (ok) {
-      OpField *u = &op->in[0], *qd = &op->in[1], *vv = &op->out[0];
-      ok = qf->in[0].emode == CEED_EVAL_GRAD && qf->in[0].size == 9 && u->v == CEED_VECTOR_ACTIVE && is_tensor3(u->b) &&
-           u->b->ncomp == 3 && u->r && u->r != CEED_ELEMRESTRICTION_NONE && u->r->strided == 0 && u->r->ncomp == 3 &&
-           u->r->compstride == 1 && u->r->elemsize == u->b->P * u->b->P * u->b->P;
-      const int Q = ok ? u->b->Q : 0;
-      ok = ok && b200_fused_supported(u->b->P, Q);
-      ok = ok && qf->in[1].emode == CEED_EVAL_NONE && qf->in[1].size == 10 && is_qstrided(qd->r, 10, Q) &&
-           is_passive(qd->v) && qd->r->nelem == u->r->nelem;
-      ok = ok && qf->out[0].emode == CEED_EVAL_GRAD && qf->out[0].size == 9 && vv->v == CEED_VECTOR_ACTIVE &&
-           vv->r == u->r && (vv->b == u->b || (is_tensor3(vv->b) && vv->b->P == u->b->P && vv->b->Q == Q &&
-                                               !memcmp(vv->b->interp1d, u->b->interp1d, sizeof(double) * Q * u->b->P) &&
-                                               !memcmp(vv->b->grad1d, u->b->grad1d, sizeof(double) * Q * u->b->P)));
+      OpField *u = &op->in[0], *qd = &op->in[1];
+      const int Q = u->b->Q;
+      ok = qf->in[1].emode == CEED_EVAL_NONE && qf->in[1].size == 10 && is_qstrided(qd->r, 10, Q) && is_passive(qd->v) &&
+           qd->r->nelem == u->r->nelem;
       if (ok && has_gradu) {
         OpField *g = is_jac ? &op->in[2] : &op->out[1];
         const QFField *gf = is_jac ? &qf->in[2] : &qf->out[1];
@@ -1132,6 +1137,19 @@ static int op_setup(CeedOperator op) {
     }
   }
   return 0;
+}
+
+/* the operators whose apply runs on the fused kernels, element range by element range: the built-in residual and
+   Jacobian, and K12 */
+static int op_fused_apply(CeedOperator op) {
+  return op->kind == OP_FUSED_JACOBIAN || op->kind == OP_FUSED_RESIDUAL || op->kind == OP_JIT_FUSED;
+}
+
+/* the operators whose diagonal and p = 1 assembly run on fused kernels: the built-in Jacobians (the linear-elastic
+   residual is its own Jacobian), and the JIT operators of K12 */
+static int op_fused_jacobian(CeedOperator op) {
+  return op->kind == OP_FUSED_JACOBIAN || op->kind == OP_JIT_FUSED ||
+         (op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS);
 }
 
 int CeedOperatorIsFusedB200(CeedOperator op, int *isFused) {
@@ -1428,7 +1446,7 @@ static int op_apply_hostpipe(CeedOperator op, CeedVector in, CeedVector out, int
   if (ceed->deterministic) return 0;  /* chunked launches scatter with atomics */
   if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL) return 0;
   if (!in || !out || in == out || !in->h_valid || in->d_valid || !in->h || !out->h) return 0;
-  OpField *u = &op->in[0];
+  OpField *u = &op->in[op->ai];
   if (in->length != u->r->lsize || out->length != u->r->lsize) return 0;
   CeedChk(rstr_pipe_setup(u->r, u->b->Q));
   if (u->r->pipe_n < 2) return 0;
@@ -1455,50 +1473,6 @@ static int op_apply_hostpipe(CeedOperator op, CeedVector in, CeedVector out, int
   return 0;
 }
 
-/* fused residual / Jacobian kernels on the element range [e0, e1): e0 a multiple of the q-blocked group size */
-static int op_apply_fused_range(CeedOperator op, CeedVector in, CeedVector out, int e0, int e1) {
-  Ceed ceed = op->ceed;
-  const double *x;
-  double *y;
-  OpField *u = &op->in[0];
-  b200_physics phys;
-  CeedChk(qf_physics(op->qf, &phys));
-  const int P = u->b->P, Q = u->b->Q, P3 = P * P * P, Q3 = Q * Q * Q;
-  if (in->length < u->r->lsize || out->length < u->r->lsize)
-    return CeedError(ceed, 1, "operator %s: active vectors shorter than the restriction's L-vector size %d", op->qf->name, u->r->lsize);
-  const int *off = u->r->d_offsets + (size_t)e0 * P3;
-  double *evec = NULL;
-  if (ceed->deterministic) {
-    if (e0 != 0 || e1 != u->r->nelem)
-      return CeedError(ceed, 1, "deterministic mode: element-range applies are not supported (the ordered sum runs over the whole restriction)");
-    CeedChk(det_scratch(ceed, (size_t)u->r->nelem * 3 * P3 * sizeof(double), &evec));
-  }
-  if (op->kind == OP_FUSED_JACOBIAN) {
-    const double *jc;
-    CeedChk(jcache_get(op, &jc));
-    CeedChk(vec_dev_read(in, &x));
-    CeedChk(vec_dev_rw(out, &y));
-    B2(ceed, b200_apply_jacobian(op->problem, &phys, e1 - e0, P, Q, u->b->interp1d, u->b->grad1d, off,
-                                 jc + (size_t)e0 * b200_jcache_ncomp(op->problem) * Q3, x, y, evec));
-  } else {
-    const double *qd;
-    double *gu = NULL;
-    CeedChk(vec_dev_read(op->in[1].v, &qd));
-    if (op->problem != B200_PROB_LINELAS) {
-      /* a partial range rewrites only its own slice of gradu: the rest must stay valid */
-      if (e0 == 0 && e1 == u->r->nelem) CeedChk(vec_dev_write(op->out[1].v, &gu));
-      else CeedChk(vec_dev_rw(op->out[1].v, &gu));
-      gu += (size_t)e0 * 9 * Q3;
-    }
-    CeedChk(vec_dev_read(in, &x));
-    CeedChk(vec_dev_rw(out, &y));
-    B2(ceed, b200_apply_residual(op->problem, &phys, e1 - e0, P, Q, u->b->interp1d, u->b->grad1d, off,
-                                 qd + (size_t)e0 * 10 * Q3, gu, x, y, evec));
-  }
-  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, y));
-  return 0;
-}
-
 /* K12, K13, K14: the operator's program of the given kind, compiled with `compile` at its first use; *slot holds the
  * handle + 1 (0: not compiled yet).  K12 is compiled at the first apply (the point program of op_setup stays: it
  * reports source errors at set-up), K13 at the first CeedOperatorLinearAssemble, K14 at the first diagonal. */
@@ -1511,9 +1485,9 @@ static int jit_op_handle(CeedOperator op, jit_compile_fn compile, int *slot, con
     int in_sizes[MAXF], out_sizes[MAXF], hh = -1;
     for (int i = 0; i < qf->nin; i++) in_sizes[i] = qf->in[i].size;
     for (int i = 0; i < qf->nout; i++) out_sizes[i] = qf->out[i].size;
-    CeedBasis b = op->in[op->jit_ai].b;
-    if (compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->jit_ai, op->jit_ao,
-                b->P, b->Q, &hh))
+    CeedBasis b = op->in[op->ai].b;
+    if (compile(qf->jit_text, qf->jit_path, qf->name, qf->nin, in_sizes, qf->nout, out_sizes, op->ai, op->ao, b->P,
+                b->Q, &hh))
       return CeedError(ceed, 1, "%s: %s of QFunction \"%s\" from %s: %s", CEED_B200_RESOURCE, what, qf->name,
                        qf->jit_path, b200_last_error());
     *slot = hh + 1;
@@ -1522,51 +1496,89 @@ static int jit_op_handle(CeedOperator op, jit_compile_fn compile, int *slot, con
   return 0;
 }
 
-/* K12 on the element range [e0, e1), e0 a multiple of the q-blocked group size: the active output is added to, the
- * passive outputs are stored (passive_add = 0, Apply) or added to (ApplyAdd) */
-static int op_apply_jit_range(CeedOperator op, CeedVector in, CeedVector out, int e0, int e1, int passive_add) {
-  Ceed ceed = op->ceed;
+/* the device copies of a JIT operator's passive inputs (K12, K13, K14), from element e0 on; NULL at the active input */
+static int jit_passive_inputs(CeedOperator op, int e0, const double **din) {
   CeedQFunction qf = op->qf;
-  OpField *u = &op->in[op->jit_ai];
-  const int P = u->b->P, Q = u->b->Q, P3 = P * P * P, Q3 = Q * Q * Q, nelem = u->r->nelem;
-  if (in->length < u->r->lsize || out->length < u->r->lsize)
-    return CeedError(ceed, 1, "operator %s: active vectors shorter than the restriction's L-vector size %d", qf->name, u->r->lsize);
-  int h;
-  size_t bytes;
-  CeedChk(jit_op_handle(op, b200_jit_fused_compile, &op->jit_fused, "fused kernel", &h));
-  CeedChk(jit_ctx_bytes(qf, &bytes));
-  double *evec = NULL;
-  if (ceed->deterministic) {
-    if (e0 != 0 || e1 != nelem)
-      return CeedError(ceed, 1, "deterministic mode: element-range applies are not supported (the ordered sum runs over the whole restriction)");
-    CeedChk(det_scratch(ceed, (size_t)nelem * 3 * P3 * sizeof(double), &evec));
+  const int Q = op->in[op->ai].b->Q;
+  for (int i = 0; i < qf->nin; i++) {
+    din[i] = NULL;
+    if (i == op->ai) continue;
+    CeedChk(vec_dev_read(op->in[i].v, &din[i]));
+    din[i] += (size_t)e0 * qf->in[i].size * Q * Q * Q;
   }
-  const double *din[MAXF] = {NULL}, *x;
-  double *dout[MAXF] = {NULL}, *y;
-  for (int i = 0; i < qf->nin; i++)
-    if (i != op->jit_ai) {
-      CeedChk(vec_dev_read(op->in[i].v, &din[i]));
-      din[i] += (size_t)e0 * qf->in[i].size * Q3;
-    }
-  for (int i = 0; i < qf->nout; i++)
-    if (i != op->jit_ao) {
-      /* a store over the whole range overwrites every entry; anything else keeps the rest valid */
-      if (!passive_add && e0 == 0 && e1 == nelem) CeedChk(vec_dev_write(op->out[i].v, &dout[i]));
-      else CeedChk(vec_dev_rw(op->out[i].v, &dout[i]));
-      dout[i] += (size_t)e0 * qf->out[i].size * Q3;
-    }
-  CeedChk(vec_dev_read(in, &x));
-  CeedChk(vec_dev_rw(out, &y));
-  B2(ceed, b200_jit_fused_apply(h, qf->ctx, bytes, e1 - e0, u->b->interp1d, u->b->grad1d, u->r->d_offsets + (size_t)e0 * P3,
-                                x, y, evec, qf->nin, din, qf->nout, dout, passive_add));
-  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, y));
   return 0;
 }
 
-/* the fused kernels on [e0, e1): built-in (passive gradu always stored) or K12 */
+/* makes current what every element range of a fused apply reads, so that ranges can run on two streams at once: the
+ * Jacobian cache of a built-in Jacobian (*jc); K12 of a JIT operator, compiled at its first apply (*h), with the device
+ * copies of its passive vectors from element e0 on (din, dout).  A passive output the apply stores over all of its
+ * entries (overwrite) is not copied in. */
+static int op_fused_state(CeedOperator op, int e0, int overwrite, const double **jc, int *h, const double **din,
+                          double **dout) {
+  CeedQFunction qf = op->qf;
+  if (op->kind == OP_FUSED_JACOBIAN) return jcache_get(op, jc);
+  if (op->kind != OP_JIT_FUSED) return 0;
+  const int Q = op->in[op->ai].b->Q;
+  CeedChk(jit_op_handle(op, b200_jit_fused_compile, &op->jit_fused, "fused kernel", h));
+  CeedChk(jit_passive_inputs(op, e0, din));
+  for (int i = 0; i < qf->nout; i++) {
+    dout[i] = NULL;
+    if (i == op->ao) continue;
+    if (overwrite) CeedChk(vec_dev_write(op->out[i].v, &dout[i]));
+    else CeedChk(vec_dev_rw(op->out[i].v, &dout[i]));
+    dout[i] += (size_t)e0 * qf->out[i].size * Q * Q * Q;
+  }
+  return 0;
+}
+
+/* the fused kernels on the element range [e0, e1), e0 a multiple of the q-blocked group size: the built-in residual or
+ * Jacobian, or K12.  The active output is added to.  K12 stores its passive outputs (passive_add = 0, Apply) or adds to
+ * them (ApplyAdd); the built-in residual always stores gradu. */
 static int op_apply_range(CeedOperator op, CeedVector in, CeedVector out, int e0, int e1, int passive_add) {
-  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, e0, e1, passive_add);
-  return op_apply_fused_range(op, in, out, e0, e1);
+  Ceed ceed = op->ceed;
+  CeedQFunction qf = op->qf;
+  OpField *u = &op->in[op->ai];
+  const int P = u->b->P, Q = u->b->Q, P3 = P * P * P, Q3 = Q * Q * Q, nelem = u->r->nelem;
+  const int whole = e0 == 0 && e1 == nelem;
+  b200_physics phys;
+  size_t bytes = 0;
+  if (op->kind == OP_JIT_FUSED) CeedChk(jit_ctx_bytes(qf, &bytes));
+  else CeedChk(qf_physics(qf, &phys));
+  if (in->length < u->r->lsize || out->length < u->r->lsize)
+    return CeedError(ceed, 1, "operator %s: active vectors shorter than the restriction's L-vector size %d", qf->name, u->r->lsize);
+  if (ceed->deterministic && !whole)
+    return CeedError(ceed, 1, "deterministic mode: element-range applies are not supported (the ordered sum runs over the whole restriction)");
+  double *evec, *dout[MAXF], *y;
+  const double *jc = NULL, *din[MAXF], *x;
+  int h = -1;
+  CeedChk(det_evec(ceed, u->r, &evec));
+  CeedChk(op_fused_state(op, e0, !passive_add && whole, &jc, &h, din, dout));
+  const double *qd = NULL;
+  double *gu = NULL;
+  if (op->kind == OP_FUSED_RESIDUAL) {
+    CeedChk(vec_dev_read(op->in[1].v, &qd));
+    qd += (size_t)e0 * 10 * Q3;
+    if (op->problem != B200_PROB_LINELAS) {
+      /* a partial range rewrites only its own slice of gradu: the rest must stay valid */
+      if (whole) CeedChk(vec_dev_write(op->out[1].v, &gu));
+      else CeedChk(vec_dev_rw(op->out[1].v, &gu));
+      gu += (size_t)e0 * 9 * Q3;
+    }
+  }
+  CeedChk(vec_dev_read(in, &x));
+  CeedChk(vec_dev_rw(out, &y));
+  const int *off = u->r->d_offsets + (size_t)e0 * P3;
+  if (op->kind == OP_FUSED_RESIDUAL)
+    B2(ceed, b200_apply_residual(op->problem, &phys, e1 - e0, P, Q, u->b->interp1d, u->b->grad1d, off, qd, gu, x, y,
+                                 evec));
+  else if (op->kind == OP_FUSED_JACOBIAN)
+    B2(ceed, b200_apply_jacobian(op->problem, &phys, e1 - e0, P, Q, u->b->interp1d, u->b->grad1d, off,
+                                 jc + (size_t)e0 * b200_jcache_ncomp(op->problem) * Q3, x, y, evec));
+  else
+    B2(ceed, b200_jit_fused_apply(h, qf->ctx, bytes, e1 - e0, u->b->interp1d, u->b->grad1d, off, x, y, evec, qf->nin,
+                                  din, qf->nout, dout, passive_add));
+  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, y));
+  return 0;
 }
 
 static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
@@ -1577,7 +1589,6 @@ static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
   }
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
   if (op->kind == OP_GENERIC) return op_apply_generic(op, in, out);
-  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, 0, op->in[op->jit_ai].r->nelem, 1);
   if (op->kind == OP_FUSED_TRANSFER) {
     const double *x;
     double *y;
@@ -1593,14 +1604,13 @@ static int op_apply_add(CeedOperator op, CeedVector in, CeedVector out) {
     const int inject = prolong && mult && op->xfer_inject;
     CeedElemRestriction ro = prolong ? f->r : c->r;
     double *evec = NULL;
-    if (ceed->deterministic && !inject)
-      CeedChk(det_scratch(ceed, (size_t)ro->nelem * ro->elemsize * 3 * sizeof(double), &evec));
+    if (!inject) CeedChk(det_evec(ceed, ro, &evec));
     B2(ceed, b200_apply_transfer(!prolong, c->r->nelem, c->b->P, c->b->Q, c->b->interp1d, c->r->d_offsets, f->r->d_offsets,
                                  mult, inject, x, y, evec));
     if (evec) CeedChk(rstr_ordered_add(ro, 1, evec, y));
     return 0;
   }
-  return op_apply_fused_range(op, in, out, 0, op->in[0].r->nelem);
+  return op_apply_range(op, in, out, 0, op->in[op->ai].r->nelem, 1);
 }
 
 /* /gpu/b200 extension: ApplyAdd restricted to the elements [start, stop) of a fused residual / Jacobian operator
@@ -1613,10 +1623,9 @@ int CeedOperatorApplyAddRangeB200(CeedOperator op, CeedVector in, CeedVector out
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: composite operators are not supported");
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL && op->kind != OP_JIT_FUSED)
+  if (!op_fused_apply(op))
     return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: operator %s does not run on the fused kernels", op->qf->name);
-  const int ia = op->kind == OP_JIT_FUSED ? op->jit_ai : 0;
-  const int nelem = op->in[ia].r->nelem, EB = b200_elems_per_block(op->in[ia].b->Q);
+  const int nelem = op->in[op->ai].r->nelem, EB = b200_elems_per_block(op->in[op->ai].b->Q);
   if (start < 0 || stop > nelem || start > stop || start % EB || (stop % EB && stop != nelem))
     return CeedError(ceed, 1, "CeedOperatorApplyAddRangeB200: bad element range [%d, %d) (nelem %d; start, and stop "
                      "unless it is nelem, must be multiples of %d)", start, stop, nelem, EB);
@@ -1656,10 +1665,9 @@ int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in, CeedVector 
   Ceed ceed = op->ceed;
   if (op->composite) return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: composite operators are not supported");
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (op->kind != OP_FUSED_JACOBIAN && op->kind != OP_FUSED_RESIDUAL && op->kind != OP_JIT_FUSED)
+  if (!op_fused_apply(op))
     return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: operator %s does not run on the fused kernels", op->qf->name);
-  const int ia = op->kind == OP_JIT_FUSED ? op->jit_ai : 0;
-  const int nelem = op->in[ia].r->nelem, EB = b200_elems_per_block(op->in[ia].b->Q);
+  const int nelem = op->in[op->ai].r->nelem, EB = b200_elems_per_block(op->in[op->ai].b->Q);
   if (n_interface < 0 || n_interface > nelem || (n_interface % EB && n_interface != nelem))
     return CeedError(ceed, 1, "CeedOperatorApplyPartitionedB200: n_interface %d must be a multiple of %d within [0, %d]", n_interface, EB, nelem);
   double *y;
@@ -1670,22 +1678,14 @@ int CeedOperatorApplyPartitionedB200(CeedOperator op, CeedVector in, CeedVector 
     if (halo) { B2(ceed, b200_halo_begin((b200_halo *)halo, y)); B2(ceed, b200_halo_end((b200_halo *)halo, y)); }
   } else {
     /* everything the two element ranges share is made current on the compute stream first (device copies of the
-       vectors, the Jacobian cache); then the interface elements + push run on the halo's high-priority side stream
+       vectors, the Jacobian cache, K12); then the interface elements + push run on the halo's high-priority side stream
        CONCURRENTLY with the interior elements on the compute stream (both only add into Y, on disjoint shared dofs) */
-    const double *x, *jc;
+    const double *x, *jc, *din[MAXF];
+    double *dout[MAXF];
+    int h;
     CeedChk(vec_dev_read(in, &x));
     CeedChk(vec_dev_rw(out, &y));
-    if (op->kind == OP_FUSED_JACOBIAN) CeedChk(jcache_get(op, &jc));
-    if (op->kind == OP_JIT_FUSED) {  /* compiled, and the passive vectors current on the device, before the fork */
-      int h;
-      CeedChk(jit_op_handle(op, b200_jit_fused_compile, &op->jit_fused, "fused kernel", &h));
-      for (int i = 0; i < op->qf->nin; i++)
-        if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &x));
-      for (int i = 0; i < op->qf->nout; i++)
-        if (i != op->jit_ao) CeedChk(vec_dev_rw(op->out[i].v, &y));
-      CeedChk(vec_dev_rw(out, &y));
-      CeedChk(vec_dev_read(in, &x));
-    }
+    CeedChk(op_fused_state(op, 0, 0, &jc, &h, din, dout));
     void *side = NULL, *mainstream = b200_get_stream();
     B2(ceed, b200_halo_fork((b200_halo *)halo, &side));
     B2(ceed, b200_set_stream(side));
@@ -1723,10 +1723,10 @@ static int op_apply(CeedOperator op, CeedVector in, CeedVector out) {
     if (!v || v == CEED_VECTOR_NONE) continue;
     /* the fused residual kernel overwrites every entry of its passive output (gradu) itself */
     if (op->kind == OP_FUSED_RESIDUAL && i == 1) continue;
-    if (op->kind == OP_JIT_FUSED && i != op->jit_ao) continue;  /* K12 stores them (passive_add = 0 below) */
+    if (op->kind == OP_JIT_FUSED && i != op->ao) continue;  /* K12 stores them (passive_add = 0 below) */
     CeedChk(CeedVectorSetValue(v, 0.0));
   }
-  if (op->kind == OP_JIT_FUSED) return op_apply_jit_range(op, in, out, 0, op->in[op->jit_ai].r->nelem, 0);
+  if (op_fused_apply(op)) return op_apply_range(op, in, out, 0, op->in[op->ai].r->nelem, 0);
   return op_apply_add(op, in, out);
 }
 int CeedOperatorApply(CeedOperator op, CeedVector in, CeedVector out, CeedRequest *request) {
@@ -1735,56 +1735,51 @@ int CeedOperatorApply(CeedOperator op, CeedVector in, CeedVector out, CeedReques
   return vec_write_through(out);
 }
 
-/* K14: compile the diagonal program at the operator's first diagonal, then add the diagonal of the user function's
- * operator (linear in its active input, as every Jacobian QFunction is) to `assembled`.  The passive inputs are read
- * where K12 reads them; passive outputs are never written.  Same output convention as the built-in diagonal (K3). */
-static int op_diagonal_jit(CeedOperator op, CeedVector assembled) {
+/* the diagonal of a fused Jacobian, added to `assembled`: K3 from the built-in Jacobian cache, or K14 around the user
+ * function (compiled at the operator's first diagonal; linear in its active input, as every Jacobian QFunction is),
+ * which reads the passive inputs where K12 reads them and never writes the passive outputs.  Both add at the
+ * restriction's offsets, so the vector must hold its whole L-vector. */
+static int op_diagonal_fused(CeedOperator op, CeedVector assembled) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
-  OpField *u = &op->in[op->jit_ai];
+  OpField *u = &op->in[op->ai];
   if (assembled->length < u->r->lsize)
     return CeedError(ceed, 1, "CeedOperatorLinearAssembleDiagonal: operator %s: vector shorter than the restriction's "
                               "L-vector size %d", qf->name, u->r->lsize);
-  int h;
+  b200_physics phys;
+  const double *jc, *din[MAXF];
   size_t bytes;
-  CeedChk(jit_op_handle(op, b200_jit_diag_compile, &op->jit_diag, "diagonal kernel", &h));
-  CeedChk(jit_ctx_bytes(qf, &bytes));
-  const double *din[MAXF] = {NULL};
-  for (int i = 0; i < qf->nin; i++)
-    if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &din[i]));
-  double *d, *evec = NULL;
+  int h;
+  if (op->kind == OP_JIT_FUSED) {
+    CeedChk(jit_op_handle(op, b200_jit_diag_compile, &op->jit_diag, "diagonal kernel", &h));
+    CeedChk(jit_ctx_bytes(qf, &bytes));
+    CeedChk(jit_passive_inputs(op, 0, din));
+  } else {
+    CeedChk(qf_physics(qf, &phys));
+    CeedChk(jcache_get(op, &jc));
+  }
+  double *d, *evec;
   CeedChk(vec_dev_rw(assembled, &d));
-  if (ceed->deterministic) CeedChk(det_scratch(ceed, (size_t)u->r->nelem * u->r->elemsize * 3 * sizeof(double), &evec));
-  B2(ceed, b200_jit_diag_apply(h, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
-                               u->r->d_offsets, qf->nin, din, d, evec));
+  CeedChk(det_evec(ceed, u->r, &evec));
+  if (op->kind == OP_JIT_FUSED)
+    B2(ceed, b200_jit_diag_apply(h, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d, u->r->d_offsets, qf->nin,
+                                 din, d, evec));
+  else
+    B2(ceed, b200_apply_diagonal(op->problem, &phys, u->r->nelem, u->b->P, u->b->Q, u->b->interp1d, u->b->grad1d,
+                                 u->r->d_offsets, jc, d, evec));
   if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, d));
   return 0;
 }
 
 int CeedOperatorLinearAssembleAddDiagonal(CeedOperator op, CeedVector assembled, CeedRequest *request) {
   (void)request;
-  Ceed ceed = op->ceed;
   if (op->composite) {
     for (int i = 0; i < op->nsubs; i++) CeedChk(CeedOperatorLinearAssembleAddDiagonal(op->subs[i], assembled, request));
     return 0;
   }
   if (op->kind == OP_UNSET) CeedChk(op_setup(op));
-  if (op->kind == OP_JIT_FUSED) return op_diagonal_jit(op, assembled);
-  if (op->kind != OP_FUSED_JACOBIAN && !(op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS))
-    return op_diagonal_generic(op, assembled);
-  OpField *u = &op->in[0];
-  b200_physics phys;
-  CeedChk(qf_physics(op->qf, &phys));
-  const double *jc;
-  double *d;
-  CeedChk(jcache_get(op, &jc));
-  CeedChk(vec_dev_rw(assembled, &d));
-  double *evec = NULL;
-  if (ceed->deterministic) CeedChk(det_scratch(ceed, (size_t)u->r->nelem * u->r->elemsize * 3 * sizeof(double), &evec));
-  B2(ceed, b200_apply_diagonal(op->problem, &phys, u->r->nelem, u->b->P, u->b->Q, u->b->interp1d, u->b->grad1d,
-                               u->r->d_offsets, jc, d, evec));
-  if (evec) CeedChk(rstr_ordered_add(u->r, 1, evec, d));
-  return 0;
+  if (!op_fused_jacobian(op)) return op_diagonal_generic(op, assembled);
+  return op_diagonal_fused(op, assembled);
 }
 int CeedOperatorLinearAssembleDiagonal(CeedOperator op, CeedVector assembled, CeedRequest *request) {
   CeedChk(CeedVectorSetValue(assembled, 0.0));
@@ -1807,9 +1802,8 @@ static int op_assemblable(CeedOperator op) {
                               "assembles only operators of the fused kernels; there is no CPU fallback",
                      op->qf->name, b ? b->P : 0, b ? b->Q : 0);
   }
-  CeedBasis b = op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0].b;
-  if (!(op->kind == OP_FUSED_JACOBIAN || op->kind == OP_JIT_FUSED ||
-        (op->kind == OP_FUSED_RESIDUAL && op->problem == B200_PROB_LINELAS)) || b->P != 2)
+  CeedBasis b = op->in[op->ai].b;
+  if (!op_fused_jacobian(op) || b->P != 2)
     return CeedError(ceed, 1, "CeedOperatorLinearAssemble: /gpu/b200 assembles fused Jacobian operators on a trilinear "
                               "(P = 2) level only (operator %s, P = %d); there is no CPU fallback",
                      op->qf->name, b ? b->P : 0);
@@ -1819,7 +1813,7 @@ static int op_assemblable(CeedOperator op) {
 int CeedOperatorLinearAssembleSymbolic(CeedOperator op, CeedInt *num_entries, CeedInt **rows, CeedInt **cols) {
   Ceed ceed = op->ceed;
   CeedChk(op_assemblable(op));
-  CeedElemRestriction r = op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0].r;
+  CeedElemRestriction r = op->in[op->ai].r;
   const size_t nelem = (size_t)r->nelem, ne = nelem * 576;
   if (ne > 2147483647u) return CeedError(ceed, 1, "CeedOperatorLinearAssembleSymbolic: %zu entries overflow CeedInt", ne);
   int *off = (int *)malloc(sizeof(int) * (nelem * 8 + 1));
@@ -1843,14 +1837,13 @@ int CeedOperatorLinearAssembleSymbolic(CeedOperator op, CeedInt *num_entries, Ce
 static int op_assemble_jit(CeedOperator op, double *v) {
   Ceed ceed = op->ceed;
   CeedQFunction qf = op->qf;
-  OpField *u = &op->in[op->jit_ai];
+  OpField *u = &op->in[op->ai];
   int h;
   size_t bytes;
   CeedChk(jit_op_handle(op, b200_jit_assemble_compile, &op->jit_assemble, "assembly kernel", &h));
   CeedChk(jit_ctx_bytes(qf, &bytes));
-  const double *din[MAXF] = {NULL};
-  for (int i = 0; i < qf->nin; i++)
-    if (i != op->jit_ai) CeedChk(vec_dev_read(op->in[i].v, &din[i]));
+  const double *din[MAXF];
+  CeedChk(jit_passive_inputs(op, 0, din));
   B2(ceed, b200_jit_assemble_apply(h, qf->ctx, bytes, u->r->nelem, u->b->interp1d, u->b->grad1d,
                                    qf->nin, din, v));
   return 0;
@@ -1859,7 +1852,7 @@ static int op_assemble_jit(CeedOperator op, double *v) {
 int CeedOperatorLinearAssemble(CeedOperator op, CeedVector values) {
   Ceed ceed = op->ceed;
   CeedChk(op_assemblable(op));
-  OpField *u = &op->in[op->kind == OP_JIT_FUSED ? op->jit_ai : 0];
+  OpField *u = &op->in[op->ai];
   if ((size_t)values->length < (size_t)u->r->nelem * 576)
     return CeedError(ceed, 1, "CeedOperatorLinearAssemble: values vector holds %d entries, %zu needed", values->length,
                      (size_t)u->r->nelem * 576);
